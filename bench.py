@@ -115,6 +115,41 @@ def oracle_masks(O, w, l, B, seed):
     return O.dropout_masks(PDROP, seed, l + 1, B, w["E"], w["H2"])
 
 
+DUMP_BUDGET = 64 << 20   # bytes written by --dump-outputs at most
+DUMP_SAMPLE = 1 << 20    # elements kept of a larger array
+
+
+def last_step_outputs(h, B, l):
+    """What the last lrcn_train_step_staged left for its caller: the nine updated weights (weight_k = parameter k of the ABI)
+    and the per-token target log-probs of its forward pass [l+1][B]; `loss` is their negated mean, the value the call returns
+    when asked for it.  Partial sums land in any order, and every step before this one (graph capture, warm-up, timed steps)
+    trains the same weights, so two runs of one build drift apart with the step count.  Measured on a B200 at 1000 W
+    (flickr30k_train_b256), two runs agreed to relative 5e-4 in every weight and 1e-5 in the loss at --steps 10, and to 2e-2
+    and 2e-5 at --steps 100; the gradients are not written, as those of layer 2 drifted by 18 % at --steps 7."""
+    out = {f"weight_{k}": h.get_param(k) for k in range(1, 10)}
+    lp = h.token_logps(l, B)
+    out["token_logps"] = lp
+    out["loss"] = np.float64(-lp.sum(dtype=np.float64) / lp.size)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes out_dir/<name>.npy.  An array of more than DUMP_SAMPLE elements is replaced by DUMP_SAMPLE of its entries at
+    sorted column-major positions drawn with a fixed seed, so that two runs or two builds compare entry for entry."""
+    small = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.size > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.ravel(order="F")[pos]
+        small[name] = a
+    assert sum(a.nbytes for a in small.values()) <= DUMP_BUDGET, f"--dump-outputs would write more than {DUMP_BUDGET} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in small.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def cpu_beam_leg(budget_s=12.0, n_max=64, K=3, nword=30):
     """BASELINE metric "beam-3 captions/s ... vs Knet CPU": the oracle's generate() (lrcn.jl:585-678 restated, host
     sortperm over V per beam per step exactly like lrcn.jl:655,667) on the COCO-shaped model, bounded sample."""
@@ -248,7 +283,14 @@ def main():
     ap.add_argument("--precision", default="bf16x3", choices=["bf16x3", "fp32"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-beam", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (updated weights, token log-probs, loss) "
+                         "as DIR/<name>.npy; arrays of more than 2^20 elements as a fixed seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3)
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -353,6 +395,11 @@ def main():
     # ---- device-resident run at the reference's training setting: `value`
     ms, ntok, launches, t_timed = timed_run(PDROP, 0)
     value = ntok * world / (ms * 1e-3)
+    outputs = None
+    if args.dump_outputs:  # read now: the runs below train the same weights further
+        if rank == 0:
+            outputs = last_step_outputs(h, w["B"], batches[(args.warmup + args.steps - 1) % N_SLOTS][2])
+        barrier()  # no peer starts the next exchange into this rank's buffers while they are read
     # ---- the same with dropout off (what round 1 timed), reported beside it
     ms0, ntok0, _, _ = timed_run(0.0, 5000)
 
@@ -474,6 +521,8 @@ def main():
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if line is not None:
         print(json.dumps(line), flush=True)
 
