@@ -41,7 +41,8 @@ extern "C" {
 #endif
 
 /* 2: lrcn_config gained n_gpus / device_ids (single-process multi-GPU group); sticky errors; lrcn_checkpoint_save / _load;
- *    lrcn_train_epoch / lrcn_loss_epoch (epoch-level calls, batches staged on the device: additive, same version) */
+ *    lrcn_train_epoch / lrcn_loss_epoch (epoch-level calls, batches staged on the device: additive, same version);
+ *    lrcn_set_cnn_param / lrcn_get_cnn_param / lrcn_extract_features (VGG-16 fc7 producer: additive, same version) */
 #define LRCN_ABI_VERSION 2
 #define LRCN_F_CNN 4096 /* lrcn.jl:28  const cnnout = 4096 */
 #define LRCN_NUM_PARAMS 9
@@ -156,6 +157,32 @@ LRCN_API int lrcn_train_step_staged(lrcn_handle* h, int slot, float pdrop, uint6
  * prints tokens[2:] up to the first eos (lrcn.jl:633-640). */
 LRCN_API int lrcn_beam_search(lrcn_handle* h, int split, const int64_t* image_ids, int64_t n, int beam_width, int nword,
                      int64_t* tokens_out, int32_t* len_out, float* prob_out, float* logp_out);
+
+/* ---- fc7 producer (SURVEY 8 row f-4): VGG-16 up to relu7.  Replaces get_params_cnn / get_convnet / extract_features
+ * (lrcn.jl:190-221, 697-773).  layer 1..13 = conv1_1..conv5_3, 14 = fc6, 15 = fc7; which 0 = filter, 1 = bias.
+ * All arrays are column-major Float32 as Julia / MatConvNet hold them; indices below are 0-based.
+ *  - images: 224 x 224 x 3 x n, already resized and mean-subtracted by the host (read_image_data); (y, x, c, i) is at
+ *    y + 224 x + 224^2 c + 3 224^2 i.
+ *  - filter: kh x kw x Cin x Cout, (dy, dx, c, o) at dy + kh dx + kh kw c + kh kw Cin o; dims {kh, kw, Cin, Cout}.
+ *    bias: dims {Cout, 1, 1, 1}.  Shapes (MatConvNet's): conv1_x 3->64, 64->64; conv2_x 64->128, 128->128; conv3_x 128->256,
+ *    256->256 x2; conv4_x 256->512, 512->512 x2; conv5_x 512->512 x3 (all 3x3); fc6 7x7x512x4096; fc7 1x1x4096x4096.
+ *  - layer rule: out(y,x,o) = b(o) + sum_{dy,dx,c} w(dy,dx,c,o) in(y+dy-p, x+dx-p, c) (cross-correlation, zero padding,
+ *    p = 1 for the 3x3 layers, 0 for fc6 / fc7); ReLU after every layer; 2x2 stride-2 max-pool after conv1_2, conv2_2,
+ *    conv3_3, conv4_3 and conv5_3 (fc6 is a 7x7 convolution over the pooled 7x7x512 map).
+ *  - feats_out: relu7 as 4096 x n (image i's 4096 floats contiguous): the layout lrcn_load_features takes.
+ *    LRCN_FEAT_L1: each row divided by its sum; a row whose sum is 0 stays all zero.
+ *  - images and feats_out may be host memory or device memory (unified addressing).
+ *  - get(set(x)) is bit-exact.  LRCN_ERR_ARG: wrong dims, layer / which out of range, null pointers, n <= 0, unknown
+ *    flags.  LRCN_ERR_STATE: extraction before all 30 tensors are set, get of a tensor never set.
+ *  - the weights (fp32 + bf16 hi/lo, ~1.07 GB) and the extraction workspace (~2.7 GB) are allocated on the first
+ *    lrcn_set_cnn_param / lrcn_extract_features and freed by lrcn_destroy.  Group handle: set goes to every GPU,
+ *    extraction splits the images into contiguous slices, one per GPU. */
+#define LRCN_CNN_LAYERS 15
+#define LRCN_CNN_IMAGE 224
+#define LRCN_FEAT_L1 1   /* f /= sum(f) per image, like the featsn files and lrcn.jl:597 */
+LRCN_API int lrcn_set_cnn_param(lrcn_handle* h, int layer, int which, const float* data, const int64_t dims[4]);
+LRCN_API int lrcn_get_cnn_param(lrcn_handle* h, int layer, int which, float* data, const int64_t dims[4]);
+LRCN_API int lrcn_extract_features(lrcn_handle* h, const float* images, int64_t n, int flags, float* feats_out);
 
 /* ---- checkpoint sidecar (SURVEY 8 row f-2).  Replaces save(file,"model",model,"vocab",vocab) lrcn.jl:185,230 and
  * load(file) lrcn.jl:88-93 (JLD/HDF5 is not available to a C library): a raw little-endian file

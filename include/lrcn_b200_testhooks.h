@@ -30,6 +30,10 @@ LRCN_API int lrcn_test_beam_select(lrcn_handle* h, const float* probs, const flo
 /* the PRODUCTION top-K kernel of generation from logits [R][V]: tok_out/score_out/lp_out are [R][K] (ids 1-based) */
 LRCN_API int lrcn_test_beam_topk_logits(lrcn_handle* h, const float* logits, const float* parent_prob, int R, int V, int K,
                                int64_t* tok_out, float* score_out, float* lp_out);
+/* pre-ReLU output of CNN layer `layer` (1..15) for the n images of the last lrcn_extract_features call, as H x W x Cout x n
+ * column-major (H = W = 224, 112, 56, 28, 14 for conv1..conv5, 1 for fc6 / fc7).  LRCN_ERR_STATE if that call ran more than
+ * one internal chunk of images (only the last chunk is kept) or no call ran; LRCN_ERR_ARG if n differs from its n. */
+LRCN_API int lrcn_test_cnn_activation(lrcn_handle* h, int layer, float* out, int64_t n);
 
 #ifdef __cplusplus
 }

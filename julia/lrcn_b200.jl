@@ -197,6 +197,30 @@ function beam_search(net, split, ids, beam_width, nword)
     return [tokens[1:lens[i], i] for i = 1:n], prob, lps
 end
 
+# ---- fc7 producer (SURVEY 8 row f-4): replaces get_params_cnn / get_convnet / extract_features (lrcn.jl:190-221, 697-773).
+# cnn = the 15 (filter, bias) pairs conv1_1..conv5_3, fc6, fc7 as MatConvNet stores them (filter kh x kw x Cin x Cout,
+# bias of Cout values); images = 224 x 224 x 3 x n Float32 from read_image_data (resized, mean subtracted).
+function set_cnn!(net, cnn)
+    for l = 1:15, which = 0:1
+        a = convert(Array{Float32}, cnn[l][which + 1])
+        dims = which == 0 ? Int64[size(a,1), size(a,2), size(a,3), size(a,4)] : Int64[length(a), 1, 1, 1]
+        check(ccall((:lrcn_set_cnn_param, lib), Cint, (Ptr{Void}, Cint, Cint, Ptr{Float32}, Ptr{Int64}), net.handle, l, which, a, dims))
+    end
+end
+function get_cnn_param(net, l, which, dims)
+    a = Array(Float32, dims...)
+    check(ccall((:lrcn_get_cnn_param, lib), Cint, (Ptr{Void}, Cint, Cint, Ptr{Float32}, Ptr{Int64}), net.handle, l, which, a,
+                convert(Vector{Int64}, collect(dims))))
+    return a
+end
+# relu7 of every image, 4096 x n; normalize=true divides each column by its sum like the featsn files (lrcn.jl:597)
+function extract_features(net, images; normalize=true)
+    n = size(images, 4); feats = Array(Float32, 4096, n)
+    check(ccall((:lrcn_extract_features, lib), Cint, (Ptr{Void}, Ptr{Float32}, Int64, Cint, Ptr{Float32}),
+                net.handle, convert(Array{Float32}, images), n, normalize ? 1 : 0, feats))
+    return feats
+end
+
 # ---- checkpoint sidecar (replaces save(file,"model",model,"vocab",vocab) lrcn.jl:185,230 and load(file) lrcn.jl:88-93).
 # Format: include/lrcn_b200.h.  vocab travels as "word\tindex\n" lines.
 vocab_bytes(vocab) = convert(Vector{UInt8}, join(["$(w)\t$(i)\n" for (w, i) in sort(collect(vocab), by=last)]))

@@ -18,6 +18,22 @@ OK, ERR_ARG, ERR_CUDA, ERR_NCCL, ERR_MISSING, ERR_STATE = 0, 1, 2, 3, 4, 5
 COMM_ID_BYTES = 128
 P2P_BLOB_BYTES = 512
 
+# VGG-16 up to fc7 (include/lrcn_b200.h, lrcn_set_cnn_param): filter shapes kh x kw x Cin x Cout of layers 1..15 and the
+# spatial size of each layer's output
+CNN_LAYERS, CNN_IMAGE, FEAT_L1 = 15, 224, 1
+CNN_SHAPES = [(3, 3, 3, 64), (3, 3, 64, 64), (3, 3, 64, 128), (3, 3, 128, 128), (3, 3, 128, 256), (3, 3, 256, 256),
+              (3, 3, 256, 256), (3, 3, 256, 512), (3, 3, 512, 512), (3, 3, 512, 512), (3, 3, 512, 512), (3, 3, 512, 512),
+              (3, 3, 512, 512), (7, 7, 512, 4096), (1, 1, 4096, 4096)]
+CNN_HOUT = [224, 224, 112, 112, 56, 56, 56, 28, 28, 28, 14, 14, 14, 1, 1]
+CNN_POOL_AFTER = (2, 4, 7, 10, 13)  # 2x2 max-pool after conv1_2, conv2_2, conv3_3, conv4_3, conv5_3
+
+
+def cnn_dims(layer, which):
+    if not 1 <= layer <= CNN_LAYERS or which not in (0, 1):
+        raise ValueError(f"CNN layer {layer} / which {which} out of range")
+    s = CNN_SHAPES[layer - 1]
+    return s if which == 0 else (s[3], 1, 1, 1)
+
 
 class LrcnError(RuntimeError):
     def __init__(self, code, msg):
@@ -63,6 +79,9 @@ SIGNATURES = {
     "lrcn_stage_batch": (C.c_int, [_H, C.c_int, C.c_int, _i64p, _i64p, C.c_int, C.c_int]),
     "lrcn_train_step_staged": (C.c_int, [_H, C.c_int, C.c_float, C.c_uint64, _f64p]),
     "lrcn_beam_search": (C.c_int, [_H, C.c_int, _i64p, C.c_int64, C.c_int, C.c_int, _i64p, _i32p, _f32p, _f32p]),
+    "lrcn_set_cnn_param": (C.c_int, [_H, C.c_int, C.c_int, _f32p, _i64p]),
+    "lrcn_get_cnn_param": (C.c_int, [_H, C.c_int, C.c_int, _f32p, _i64p]),
+    "lrcn_extract_features": (C.c_int, [_H, _f32p, C.c_int64, C.c_int, _f32p]),
     "lrcn_checkpoint_save": (C.c_int, [_H, C.c_char_p, C.c_int, C.c_char_p, C.c_int64]),
     "lrcn_checkpoint_load": (C.c_int, [_H, C.c_char_p, _i32p, C.c_char_p, C.c_int64, _i64p]),
     "lrcn_comm_unique_id": (C.c_int, [C.c_char_p]),
@@ -85,6 +104,7 @@ TEST_SIGNATURES = {
     "lrcn_test_gemm": (C.c_int, [_H, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _f32p, _f32p, _f32p, C.c_int, _f32p]),
     "lrcn_test_beam_select": (C.c_int, [_H, _f32p, _f32p, C.c_int, C.c_int, C.c_int, C.c_int, _i64p, _i32p, _f32p]),
     "lrcn_test_beam_topk_logits": (C.c_int, [_H, _f32p, _f32p, C.c_int, C.c_int, C.c_int, _i64p, _f32p, _f32p]),
+    "lrcn_test_cnn_activation": (C.c_int, [_H, C.c_int, _f32p, C.c_int64]),
 }
 
 _lib = None
@@ -341,6 +361,38 @@ class Handle:
         check(self.lib.lrcn_beam_search(self._h, split, _i64(ids), n, beam_width, nword, _i64(toks),
                                         lens.ctypes.data_as(_i32p), _f32(prob), _f32(lps) if want_logps else None))
         return toks, lens, prob, lps
+
+    # ---- fc7 producer (f-4): VGG-16 up to relu7
+    def set_cnn_param(self, layer, which, a):
+        """layer 1..15 (conv1_1..conv5_3, fc6, fc7); which 0: filter kh x kw x Cin x Cout, 1: bias of Cout values."""
+        a = np.asfortranarray(a, dtype=np.float32)
+        dims = cnn_dims(layer, which)
+        if a.size != int(np.prod(dims)) or (which == 0 and a.shape != dims):
+            raise ValueError(f"CNN layer {layer} {'bias' if which else 'filter'}: shape {a.shape}, expected {dims}")
+        check(self.lib.lrcn_set_cnn_param(self._h, layer, which, _f32(a), _i64(np.array(dims, dtype=np.int64))))
+
+    def get_cnn_param(self, layer, which):
+        dims = cnn_dims(layer, which)
+        out = np.empty(dims if which == 0 else (dims[0],), dtype=np.float32, order="F")
+        check(self.lib.lrcn_get_cnn_param(self._h, layer, which, _f32(out), _i64(np.array(dims, dtype=np.int64))))
+        return out
+
+    def extract_features(self, images, flags=0):
+        """images: 224 x 224 x 3 x n (column-major element order) -> relu7 as an n x 4096 array (row i = image i)."""
+        images = np.asfortranarray(images, dtype=np.float32)
+        if images.ndim != 4 or images.shape[:3] != (CNN_IMAGE, CNN_IMAGE, 3):
+            raise ValueError(f"images must be {CNN_IMAGE} x {CNN_IMAGE} x 3 x n, got {images.shape}")
+        n = images.shape[3]
+        out = np.zeros((n, 4096), dtype=np.float32)
+        check(self.lib.lrcn_extract_features(self._h, _f32(images), n, flags, _f32(out)))
+        return out
+
+    def test_cnn_activation(self, layer, n):
+        """Pre-ReLU output of CNN layer `layer` for the n images of the last extraction, H x W x Cout x n."""
+        h = CNN_HOUT[layer - 1]
+        out = np.zeros((h, h, CNN_SHAPES[layer - 1][3], n), dtype=np.float32, order="F")
+        check(self.lib.lrcn_test_cnn_activation(self._h, layer, _f32(out), n))
+        return out
 
     # ---- checkpoint sidecar (f-2)
     def checkpoint_save(self, path: str, with_adam: bool = True, aux: bytes = b""):

@@ -158,6 +158,7 @@ static int s_destroy(lrcn_handle* h) {
   }
   cudaSetDevice(h->cfg.device);
   if (h->stream) cudaStreamSynchronize(h->stream);
+  cnn_free(h);
   for (auto& kv : h->graphs) cudaGraphExecDestroy(kv.second);
   if (h->comm && nccl_api()) nccl_api()->CommDestroy(h->comm);
   if (!h->peers_direct) for (void* q : h->p2p_opened) if (q) cudaIpcCloseMemHandle(q);
@@ -1918,6 +1919,39 @@ extern "C" int lrcn_beam_search(lrcn_handle* h, int split, const int64_t* image_
       rcs[i] = s_beam_search(h->members[i], split, image_ids + lo, hi - lo, K, nword, tokens_out + lo * maxlen, len_out + lo, prob_out + lo,
                              logp_out ? logp_out + lo * (maxlen - 1) : nullptr);
       if (rcs[i]) msgs[i] = g_err;  // thread-local message of the worker
+    });
+  }
+  for (auto& t : th) t.join();
+  for (int i = 0; i < N; i++) if (rcs[i]) return fail(rcs[i], "GPU %d: %s", h->members[i]->cfg.device, msgs[i].c_str());
+  return LRCN_OK;
+}
+
+// ---- VGG-16 fc7 producer (row f-4, cnn_sm100.cu)
+extern "C" int lrcn_set_cnn_param(lrcn_handle* h, int layer, int which, const float* data, const int64_t dims[4]) {
+  ENTER(h);
+  if (is_group(h)) FOR_ALL(h, cnn_set_param(m, layer, which, data, dims));
+  return cnn_set_param(h, layer, which, data, dims);
+}
+extern "C" int lrcn_get_cnn_param(lrcn_handle* h, int layer, int which, float* data, const int64_t dims[4]) {
+  ENTER(h);
+  return cnn_get_param(is_group(h) ? h->members[0] : h, layer, which, data, dims);
+}
+extern "C" int lrcn_extract_features(lrcn_handle* h, const float* images, int64_t n, int flags, float* feats_out) {
+  ENTER(h);
+  if (!is_group(h)) return cnn_extract(h, images, n, flags, feats_out);
+  // images are independent: contiguous slices, one worker thread per GPU, each writing its rows of feats_out
+  if (!images || !feats_out || n <= 0) return fail(LRCN_ERR_ARG, "bad argument to lrcn_extract_features");
+  const int N = (int)h->members.size();
+  const int64_t img = (int64_t)3 * LRCN_CNN_IMAGE * LRCN_CNN_IMAGE;
+  std::vector<int> rcs(N, LRCN_OK);
+  std::vector<std::string> msgs(N);
+  std::vector<std::thread> th;
+  for (int i = 0; i < N; i++) {
+    const int64_t lo = n * i / N, hi = n * (i + 1) / N;
+    if (hi <= lo) continue;
+    th.emplace_back([&, i, lo, hi] {
+      rcs[i] = cnn_extract(h->members[i], images + lo * img, hi - lo, flags, feats_out + lo * LRCN_F_CNN);
+      if (rcs[i]) msgs[i] = g_err;
     });
   }
   for (auto& t : th) t.join();

@@ -128,7 +128,15 @@ struct lrcn_handle {
   int* h_ndone = nullptr;    // pinned: [0] = images done so far, [1..] = done flags of the images in flight
   int *g_keep = nullptr, *g_omap = nullptr, *g_omap_s = nullptr;  // compaction: survivors, compacted -> caller index (+ scratch)
   float* l2_scratch = nullptr; size_t l2_n = 0;
+  struct CnnState* cnn = nullptr;  // VGG-16 fc7 producer (cnn_sm100.cu): allocated by the first CNN call, null until then
 };
+
+// VGG-16 fc7 producer (cnn_sm100.cu), one GPU handle each; argument checks included, group dispatch in lrcn_api.cu
+int cnn_set_param(lrcn_handle* h, int layer, int which, const float* data, const int64_t dims[4]);
+int cnn_get_param(lrcn_handle* h, int layer, int which, float* data, const int64_t dims[4]);
+int cnn_extract(lrcn_handle* h, const float* images, int64_t n, int flags, float* feats_out);
+int cnn_activation(lrcn_handle* h, int layer, float* out, int64_t n);  // test hook lrcn_test_cnn_activation
+void cnn_free(lrcn_handle* h);
 
 static inline float* WS(lrcn_handle* h, size_t off) { return h->ws.f + off; }
 static inline float* Wp(lrcn_handle* h, int idx1) { return h->w + h->off[idx1 - 1]; }

@@ -143,3 +143,9 @@ extern "C" int lrcn_test_beam_topk_logits(lrcn_handle* h, const float* logits, c
   cleanup();
   return LRCN_OK;
 }
+
+extern "C" int lrcn_test_cnn_activation(lrcn_handle* h, int layer, float* out, int64_t n) {
+  if (!h) return fail(LRCN_ERR_ARG, "null handle");
+  if (!h->members.empty()) return fail(LRCN_ERR_ARG, "test hooks take a single-GPU handle");
+  return cnn_activation(h, layer, out, n);
+}

@@ -77,6 +77,25 @@ class LRCN:
     def load_feature_matrix(self, ids, mat, split=0):
         self.h.load_features(split, ids, mat)
 
+    # ---- fc7 producer (lrcn.jl:190-221, 697-773; SURVEY 8 row f-4)
+    def load_cnn(self, params):
+        """get_params_cnn + get_convnet: params = 15 (filter, bias) pairs conv1_1..conv5_3, fc6, fc7 in MatConvNet's layout
+        (filter kh x kw x Cin x Cout, bias of Cout values), uploaded once."""
+        if len(params) != abi.CNN_LAYERS:
+            raise ValueError(f"VGG-16 up to fc7 has {abi.CNN_LAYERS} layers, got {len(params)}")
+        for layer, (w, b) in enumerate(params, start=1):
+            self.h.set_cnn_param(layer, 0, w)
+            self.h.set_cnn_param(layer, 1, b)
+
+    def extract_features(self, images, ids, normalize=True):
+        """extract_features (lrcn.jl:190-221) for preprocessed images (224 x 224 x 3 x n, resized and mean-subtracted on the
+        host like read_image_data): the id -> relu7 Dict it saves, each row divided by its sum when normalize is set."""
+        ids = list(ids)
+        if np.ndim(images) != 4 or np.shape(images)[3] != len(ids):
+            raise ValueError("images must be 224 x 224 x 3 x n with one id per image")
+        feats = self.h.extract_features(images, abi.FEAT_L1 if normalize else 0)
+        return {int(i): feats[k] for k, i in enumerate(ids)}
+
     # ---- one batch (lrcn.jl:553-583)
     @staticmethod
     def _tokens(sequence, rng):
