@@ -212,9 +212,10 @@ LRCN_API int lrcn_sync(lrcn_handle* h);
 LRCN_API int lrcn_timer_start(lrcn_handle* h);
 LRCN_API int lrcn_timer_stop(lrcn_handle* h, float* ms_out);
 LRCN_API int lrcn_kernel_launches(lrcn_handle* h, int64_t* n_out); /* kernels launched (incl. inside graph replays) */
-LRCN_API int lrcn_flush_l2(lrcn_handle* h);
-/* LRCN_SEQ_TRACE=1 at create: [T][8] globaltimer (ns) stamps of CTA (0,0) of the layer-2 forward sequence kernel */
-LRCN_API int lrcn_get_trace(lrcn_handle* h, uint64_t* out, int64_t n);                        /* writes a 256 MiB scratch buffer */
+LRCN_API int lrcn_flush_l2(lrcn_handle* h);                                                   /* writes a 256 MiB scratch buffer */
+/* LRCN_SEQ_TRACE=1 at create: [T][4 chains][8] globaltimer (ns) stamps of CTA (0,0) of the layer-2 forward sequence kernel
+ * (LRCN_TRACE_BWD=1: of the backward one); n counts uint64 values, at most 2048 */
+LRCN_API int lrcn_get_trace(lrcn_handle* h, uint64_t* out, int64_t n);
 /* time `reps` launches of one named kernel family on the current buffers: "adam", "vocab_gemm", "gather" ... */
 LRCN_API int lrcn_time_kernel(lrcn_handle* h, const char* name, int reps, float* avg_ms_out, double* algo_bytes_out,
                      double* algo_flops_out);

@@ -445,7 +445,7 @@ class Handle:
         return int(n.value)
 
     def get_trace(self, steps):
-        out = np.zeros((steps, 8), dtype=np.uint64)
+        out = np.zeros((steps, 4, 8), dtype=np.uint64)  # [step][chain][stamp]
         check(self.lib.lrcn_get_trace(self._h, out.ctypes.data_as(_p(C.c_uint64)), out.size))
         return out
 

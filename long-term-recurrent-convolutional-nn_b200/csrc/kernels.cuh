@@ -265,12 +265,12 @@ bool lstm_bwd_step(cudaStream_t s, int B, int H, bool has_rec, const __nv_bfloat
                    const __nv_bfloat16* gnext_hi, const __nv_bfloat16* gnext_lo, float* gates, __nv_bfloat16* g_hi, __nv_bfloat16* g_lo,
                    const float* c_prev, const float* c_cur, const float* dh_in, float* dc);
 
-// persistent whole-sequence variants (weights resident in smem, grid barrier per step).  *launched = false (and nothing
-// enqueued) when they do not apply (H too large for residency, T < 2, grid not co-resident): use the per-step kernels then.
+// persistent whole-sequence variants (weights resident in tensor and shared memory, grid barrier per step).  *launched = false
+// (and nothing enqueued) when they do not apply (H > 512, B > 2048, T < 2, grid not co-resident): use the per-step kernels then.
 // counters: 64 uint32 in device memory, ZERO on entry (the caller zeroes them once per step; one region per launch).  hs/cs: [(T+1)*B][H] slot buffers; acts: [T*B][4H].
 bool lstm_fwd_seq(cudaStream_t s, int B, int H, int T, const __nv_bfloat16* wperm_hi, const __nv_bfloat16* wperm_lo, float* acts, float* hs,
                   float* cs, __nv_bfloat16* hs_hi, __nv_bfloat16* hs_lo, unsigned int* counters, bool* launched,
-                  unsigned long long* trace = nullptr /* optional [T][8] globaltimer stamps of CTA (0,0) */);
+                  unsigned long long* trace = nullptr /* optional [T][4 chains][8] globaltimer stamps of CTA (0,0) */);
 bool lstm_bwd_seq(cudaStream_t s, int B, int H, int T, const __nv_bfloat16* wt_hi, const __nv_bfloat16* wt_lo, float* acts,
                   __nv_bfloat16* acts_hi, __nv_bfloat16* acts_lo, float* cs, const float* dh_all, float* dc, unsigned int* counters,
                   bool* launched, float* dbias = nullptr /* optional [4H], zero on entry: receives the bias gradient (column sums of dG) */,

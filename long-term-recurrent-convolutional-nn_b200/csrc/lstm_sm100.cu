@@ -108,7 +108,7 @@ __device__ __forceinline__ StepSmem step_smem(uint8_t* smem_raw) {
 // MMA issue loop shared by both directions.  Called by the WHOLE (converged) warp: the loop runs on warp-uniform values and one
 // elected lane issues, so the descriptors stay in uniform registers (see elect_one(); inside `if (lane == 0)` every
 // tcgen05.mma was wrapped in an ELECT / R2UR / branch waterfall: ~125 clk per MMA instead of ~80).
-// STACKED SPLIT MMA (as in the sequence kernels): the stage holds {A_hi 64 rows; A_lo 64 rows} and {B_hi 64; B_lo 64} back to
+// STACKED SPLIT MMA: the stage holds {A_hi 64 rows; A_lo 64 rows} and {B_hi 64; B_lo 64} back to
 // back, each a valid 128-row K-major SWIZZLE_128B tile, so ONE 128x128x16 tcgen05.mma per k-step yields all split products:
 //   lanes 0-63 x cols 0-63: A_hi*B_hi | lanes 0-63 x cols 64-127: A_hi*B_lo | lanes 64-127 x cols 0-63: A_lo*B_hi | (lo*lo ignored)
 // -- a third of the instructions of three M=64 MMAs (the step is bound by MMA instructions and operand delivery, not flops).
@@ -449,28 +449,13 @@ lstm_bwd_step_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_co
 
 // ============================================================================================================
 // Persistent sequence kernels: ONE launch runs all T timesteps of a layer.  The CTA's slice of the recurrent weights
-// (bf16 hi/lo) is loaded once and stays resident in shared memory; per step only the activation tile streams through a
-// small TMA ring.  Steps are separated by a per-m-tile grid barrier (release/acquire counter in global memory): the
+// (bf16 hi/lo) is loaded once and stays resident in tensor and shared memory; per step only the activation chunk streams in
+// by TMA.  Steps are separated by a grid barrier per (m-tile, chain) (release/acquire counter in global memory): the
 // h_t (or dG_t) rows a step produces are read by the TMA engines of the other CTAs in the next step, so the releasing
 // thread fences generic->async proxy before the release and the reading producer fences after the acquire.
-//
-// STACKED SPLIT MMA.  The ring stage holds {A_hi (64 rows), A_lo (64 rows)} back to back and the resident block holds
-// {B_hi (64 rows), B_lo (64 rows)} back to back; both are therefore valid 128-row K-major SWIZZLE_128B tiles, and ONE
-// full-rate 128x128x16 tcgen05.mma per k-step produces all split products at once:
-//     lanes 0-63   x cols 0-63  : A_hi*B_hi      lanes 0-63   x cols 64-127 : A_hi*B_lo
-//     lanes 64-127 x cols 0-63  : A_lo*B_hi      lanes 64-127 x cols 64-127 : A_lo*B_lo (ignored)
-// instead of three half-rate M=64 MMAs (measured: the M=64 SS-mode chain of 96 MMAs took 4.1 us of an 8 us step).
-// The epilogue adds the three pieces: the warps of TMEM lane quadrants 2,3 pass the A_lo*B_hi rows through a small
-// smem buffer to the warps of quadrants 0,1, which own the 64 batch rows.
 // All waits are clock-bounded and trap instead of hanging.
 // ============================================================================================================
-constexpr int RSTAGE = 2 * A_HALF;             // 16 KiB: A_hi + A_lo of one k-block = one 128-row tile
 constexpr int MAX_RES_KB = 8;                  // resident weight k-blocks (16 KiB each)
-constexpr int FSTAGES = 5, BSTAGES = 4;        // activation ring depth: forward / backward (which also needs the red buffer)
-constexpr int SEQ_EPI_THREADS = 256;
-constexpr int SLO_LD = 68;                     // padded row (floats) of the A_lo*B_hi hand-over buffer
-constexpr int SLO_BYTES = LM * SLO_LD * 4;     // 17 KiB
-constexpr uint32_t SEQ_TMEM_COLS = 128;
 
 struct SeqParams {
   int B, H, T, num_kb;          // num_kb: k-blocks of the full K (fwd: H/64, bwd: 4H/64)
@@ -481,11 +466,11 @@ struct SeqParams {
   __nv_bfloat16* o_lo;
   const float* dh_all;          // bwd: [T*B][H]
   float* dc;                    // unused by the sequence kernels (dc is carried in registers)
-  unsigned int* counters;       // one per m-tile, zeroed before launch
-  unsigned long long* trace;    // optional [T][8] globaltimer stamps of CTA (0,0) (LRCN_SEQ_TRACE=1), else null
+  unsigned int* counters;       // one per (m-tile, chain), zeroed before launch
+  unsigned long long* trace;    // optional [T][4 chains][8] globaltimer stamps of CTA (0,0) (LRCN_SEQ_TRACE=1), else null
   float* dbias;                 // bwd (optional): bias gradient [4H] += column sums of dG over all rows and steps (zero on entry)
-  int sync_flags;               // seq2 forward experiments: 1 = no writer-side proxy fence, 2 = per-warp arrive, 4 = relaxed polling
-  int no_mcast;                 // seq2 forward: every CTA fetches its own copy of the h tile (no cluster multicast)
+  int sync_flags;               // diagnostics (LRCN_SEQ_SYNC): 8 = fwd issuer waits for the whole chunk, 16 = no anti-phase delay,
+                                // bits 8 and up = the anti-phase delay in ns (0: 2800)
 };
 
 __device__ __forceinline__ void grid_arrive(unsigned int* ctr) {
@@ -508,577 +493,12 @@ __device__ __forceinline__ void grid_wait(const unsigned int* ctr, unsigned int 
     }
   }
 }
-// poll with relaxed loads, acquire once the target is reached
-__device__ __forceinline__ void grid_wait_relaxed(const unsigned int* ctr, unsigned int target) {
-  const long long t0 = clock64();
-  unsigned int spins = 0;
-  while (true) {
-    unsigned int v;
-    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(ctr) : "memory");
-    if (v >= target) break;
-    if ((++spins & 63u) == 0u) {
-      if (dev_aborted()) break;
-      if (clock64() - t0 > WAIT_LIMIT_CLK) {
-        printf("lrcn lstm_seq: grid barrier timeout (block %d,%d have %u want %u)\n", blockIdx.x, blockIdx.y, v, target);
-        dev_abort_set();
-        break;
-      }
-    }
-  }
-  asm volatile("fence.acq_rel.gpu;" ::: "memory");
-}
 __device__ __forceinline__ unsigned long long gtime() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-#define LRCN_TRACE(slot) do { if (p.trace && blockIdx.x == 0 && blockIdx.y == 0) p.trace[(size_t)t * 8 + (slot)] = gtime(); } while (0)
 __device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-__device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(SEQ_EPI_THREADS) : "memory"); }
-__device__ __forceinline__ void slo_bar_sync() { asm volatile("bar.sync 2, %0;" ::"n"(SEQ_EPI_THREADS) : "memory"); }
-__device__ __forceinline__ void slo_bar_arrive() { asm volatile("bar.arrive 2, %0;" ::"n"(SEQ_EPI_THREADS) : "memory"); }
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  const long long t0 = clock64();
-  unsigned int spins = 0;
-  while (true) {
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    if (done) break;
-    if ((++spins & 255u) == 0u && dev_aborted()) break;
-    if (clock64() - t0 > WAIT_LIMIT_CLK) {
-      printf("lrcn lstm_seq: cluster mbarrier timeout (block %d,%d thread %d)\n", blockIdx.x, blockIdx.y, threadIdx.x);
-      dev_abort_set();
-      break;
-    }
-  }
-}
-
-struct SeqSmem {
-  uint32_t res, ring, full0, empty0, wbar, tfull, tempty, redfull, redempty;
-  uint32_t* tmem_slot;
-  float* slo;
-  float* red;
-};
-template <int NSTAGES, bool WITH_RED>
-__device__ __forceinline__ SeqSmem seq_smem(uint8_t* smem_raw, int res_kb) {
-  SeqSmem s;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* al = smem_raw + (base - smem_u32(smem_raw));
-  s.res = base;                                   // res_kb x {B_hi 8 KiB, B_lo 8 KiB}
-  s.ring = base + (uint32_t)res_kb * 2 * B_HALF;  // NSTAGES x {A_hi, A_lo}
-  uint8_t* after = al + (size_t)res_kb * 2 * B_HALF + NSTAGES * RSTAGE;
-  s.slo = reinterpret_cast<float*>(after);
-  s.red = reinterpret_cast<float*>(after + SLO_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(after + SLO_BYTES + (WITH_RED ? RED_BYTES : 0));
-  s.full0 = smem_u32(bars);
-  s.empty0 = smem_u32(bars + NSTAGES);
-  s.wbar = smem_u32(bars + 2 * NSTAGES);
-  s.tfull = smem_u32(bars + 2 * NSTAGES + 1);
-  s.tempty = smem_u32(bars + 2 * NSTAGES + 2);
-  s.redfull = smem_u32(bars + 2 * NSTAGES + 3);
-  s.redempty = smem_u32(bars + 2 * NSTAGES + 4);
-  s.tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * NSTAGES + 5);
-  return s;
-}
-static int seq_smem_bytes(int res_kb, bool bwd) {
-  return res_kb * 2 * B_HALF + (bwd ? BSTAGES : FSTAGES) * RSTAGE + SLO_BYTES + (bwd ? RED_BYTES : 0) + 1024 + 256;
-}
-
-// one stacked MMA per 16-wide k-step: A tile = 128 rows {hi;lo} at `sa`, B tile = 128 rows {hi;lo} at `sb`
-__device__ __forceinline__ void stacked_mma_kblock(uint32_t tmem_base, uint32_t sa, uint32_t sb, uint32_t idesc, bool first_kb) {
-  const uint32_t a_lo = desc_lo_kmajor(sa), b_lo = desc_lo_kmajor(sb);
-  umma_bf16_lo(tmem_base, a_lo, b_lo, idesc, first_kb ? 0u : 1u);
-#pragma unroll
-  for (int k = 1; k < LBK / 16; k++) umma_bf16_lo(tmem_base, a_lo + 2u * k, b_lo + 2u * k, idesc, 1u);
-}
-
-// Epilogue helper: returns in out[32] the finished accumulator row r (= 32*quad + lane, quad in {0,1}) for columns
-// [32*half, +32) as hi*hi + hi*lo + lo*hi.  Warps of quadrants 2,3 only feed the hand-over buffer and get nothing back.
-__device__ __forceinline__ void stacked_collect(const SeqSmem& sm, uint32_t tmem_base, int quad, int half, int lane, float (&out)[32]) {
-  const uint32_t tl = tmem_base + ((uint32_t)(quad * 32) << 16);
-  if (quad >= 2) {
-    uint32_t v[32];
-    LRCN_TMEM_LD_32(tl + (uint32_t)(32 * half), v);  // A_lo*B_hi, rows r = 32*(quad-2)+lane
-    tmem_ld_wait();
-    float* dst = sm.slo + (size_t)(32 * (quad - 2) + lane) * SLO_LD + 32 * half;
-#pragma unroll
-    for (int q = 0; q < 8; q++)
-      *reinterpret_cast<float4*>(dst + 4 * q) = make_float4(__uint_as_float(v[4 * q]), __uint_as_float(v[4 * q + 1]), __uint_as_float(v[4 * q + 2]),
-                                                             __uint_as_float(v[4 * q + 3]));
-    slo_bar_arrive();
-  } else {
-    uint32_t v[32], w[32];
-    LRCN_TMEM_LD_32(tl + (uint32_t)(32 * half), v);        // A_hi*B_hi
-    LRCN_TMEM_LD_32(tl + (uint32_t)(64 + 32 * half), w);   // A_hi*B_lo
-    tmem_ld_wait();
-    slo_bar_sync();
-    const float* src = sm.slo + (size_t)(32 * quad + lane) * SLO_LD + 32 * half;
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-      const float4 x = *reinterpret_cast<const float4*>(src + 4 * q);
-      out[4 * q] = __uint_as_float(v[4 * q]) + __uint_as_float(w[4 * q]) + x.x;
-      out[4 * q + 1] = __uint_as_float(v[4 * q + 1]) + __uint_as_float(w[4 * q + 1]) + x.y;
-      out[4 * q + 2] = __uint_as_float(v[4 * q + 2]) + __uint_as_float(w[4 * q + 2]) + x.z;
-      out[4 * q + 3] = __uint_as_float(v[4 * q + 3]) + __uint_as_float(w[4 * q + 3]) + x.w;
-    }
-  }
-}
-
-// ---- forward: all T steps of one layer.  grid = (n-tiles padded to CL, m-tiles), cluster = CL along n (multicast of h).
-// Weight rows are UNIT-major: row u*4+g of the CTA's block = gate g of its unit u, so the 32 columns a thread finishes are
-// the f,i,o,g of 8 consecutive hidden units.
-__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(L_THREADS, 1)
-lstm_fwd_seq_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                    const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo, const SeqParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const SeqSmem sm = seq_smem<FSTAGES, false>(smem_raw, p.num_kb);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int nt = blockIdx.x, mt = blockIdx.y, m0 = mt * LM;
-  const int num_kb = p.num_kb, T = p.T, B = p.B, H = p.H;
-  const unsigned int ctas_per_mtile = gridDim.x;
-  unsigned int* ctr = p.counters + mt;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < FSTAGES; s++) { mbar_init(sm.full0 + 8 * s, 1); mbar_init(sm.empty0 + 8 * s, CL); }
-    mbar_init(sm.wbar, 1); mbar_init(sm.tfull, 1); mbar_init(sm.tempty, 8);
-    mbar_init_fence();
-  }
-  if (warp == 0 && lane == 0) {
-    prefetch_tensormap(&tmA_hi); prefetch_tensormap(&tmA_lo); prefetch_tensormap(&tmB_hi); prefetch_tensormap(&tmB_lo);
-  }
-  if (warp == 1) tmem_alloc<SEQ_TMEM_COLS>(smem_u32(sm.tmem_slot));
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *sm.tmem_slot;
-
-  // Resident weights, loaded once.  They are written by the weight-prep kernels at the very start of the step, i.e. more
-  // than two launches upstream, so (PDL discipline, kernels.cuh) they are complete before this kernel can start: the load
-  // is issued BEFORE the dependency wait and overlaps the previous kernel's tail.
-  if (warp == 0 && lane == 0) {
-    mbar_expect_tx(sm.wbar, (uint32_t)num_kb * 2 * B_HALF);
-    for (int kb = 0; kb < num_kb; kb++) {
-      tma_load_2d(sm.res + kb * 2 * B_HALF, &tmB_hi, sm.wbar, kb * LBK, nt * NT);
-      tma_load_2d(sm.res + kb * 2 * B_HALF + B_HALF, &tmB_lo, sm.wbar, kb * LBK, nt * NT);
-    }
-  }
-  pdl_wait();
-  pdl_trigger();
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int it = 0;
-      for (int t = 1; t < T; t++) {
-        grid_wait(ctr, (unsigned int)t * ctas_per_mtile);  // h_{t-1} rows of this m-tile are complete in global memory
-        LRCN_TRACE(0);
-        fence_proxy_async_global();
-        // The cluster shares the h tile: k-block kb is fetched by rank kb % CL as two 8 KiB boxes (hi, lo; all 64 rows) and
-        // multicast to all CL CTAs -- 4x fewer, 4x larger TMA operations per SM than row-sliced multicast.
-        const int arow = t * B + m0;  // slot t of hs = h_{t-1}
-        for (int kb = 0; kb < num_kb; kb++, it++) {
-          const int s = it % FSTAGES;
-          mbar_wait(sm.empty0 + 8 * s, ((it / FSTAGES) & 1) ^ 1);  // every CTA of the cluster has consumed this stage
-          const uint32_t full = sm.full0 + 8 * s;
-          mbar_expect_tx(full, RSTAGE);
-          if ((uint32_t)(kb % CL) == rank) {
-            const uint32_t st = sm.ring + s * RSTAGE;
-            tma_load_2d_mcast(st, &tmA_hi, full, kb * LBK, arow, (uint16_t)((1u << CL) - 1));
-            tma_load_2d_mcast(st + A_HALF, &tmA_lo, full, kb * LBK, arow, (uint16_t)((1u << CL) - 1));
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      const uint32_t idesc = idesc_bf16(128, 128, false, false);
-      mbar_wait(sm.wbar, 0);
-      int it = 0;
-      for (int t = 1; t < T; t++) {
-        if (t >= 2) { mbar_wait(sm.tempty, (t - 2) & 1); tc_fence_after(); }  // epilogue of step t-1 has drained the accumulator
-        for (int kb = 0; kb < num_kb; kb++, it++) {
-          const int s = it % FSTAGES;
-          mbar_wait(sm.full0 + 8 * s, (it / FSTAGES) & 1);
-          if (kb == 0) LRCN_TRACE(1);
-          tc_fence_after();
-          stacked_mma_kblock(tmem_base, sm.ring + s * RSTAGE, sm.res + kb * 2 * B_HALF, idesc, kb == 0);
-          umma_commit_mcast(sm.empty0 + 8 * s, (uint16_t)((1u << CL) - 1));
-        }
-        umma_commit(sm.tfull);
-        LRCN_TRACE(2);
-      }
-    }
-  } else {
-    const int ew = warp - 2, quad = warp & 3, half = ew >> 2;
-    constexpr int NH = NT / 4;                       // 16 units per CTA
-    const bool owner = quad < 2;                     // warps of lane quadrants 0,1 own the 64 batch rows
-    const int m = m0 + 32 * quad + lane;             // (owner only)
-    const int j = nt * NH + 8 * half;                // first of this thread's 8 units (H % 8 == 0)
-    const bool active = owner && m < B && j < H;
-    // Off the step-to-step critical path: the x-part of the gates is prefetched one step ahead, c stays in registers, and
-    // only the bf16 split of h_t (what the other CTAs' TMA reads) is stored before the barrier arrive.
-    float creg[8];
-#pragma unroll
-    for (int e = 0; e < 8; e++) creg[e] = 0.f;
-    float4 xg[4][2];
-#pragma unroll
-    for (int g = 0; g < 4; g++) xg[g][0] = xg[g][1] = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (active) {
-      const float* g0 = p.acts + (size_t)m * 4 * H + j;
-#pragma unroll
-      for (int g = 0; g < 4; g++) { xg[g][0] = *reinterpret_cast<const float4*>(g0 + g * H); xg[g][1] = *reinterpret_cast<const float4*>(g0 + g * H + 4); }
-    }
-    for (int t = 0; t < T; t++) {
-      float acc[32];  // unit-major: acc[u*4 + g]
-      if (t > 0) {
-        mbar_wait(sm.tfull, (t - 1) & 1);
-        if (threadIdx.x == 64) LRCN_TRACE(3);
-        tc_fence_after();
-        stacked_collect(sm, tmem_base, quad, half, lane, acc);
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(sm.tempty);
-      } else {
-#pragma unroll
-        for (int c = 0; c < 32; c++) acc[c] = 0.f;
-      }
-      float f[8], in[8], o[8], ch[8], hn[8];
-      const size_t hnext = ((size_t)(t + 1) * B + m) * H + j;
-      if (active) {
-        const float xf[8] = {xg[0][0].x, xg[0][0].y, xg[0][0].z, xg[0][0].w, xg[0][1].x, xg[0][1].y, xg[0][1].z, xg[0][1].w};
-        const float xi[8] = {xg[1][0].x, xg[1][0].y, xg[1][0].z, xg[1][0].w, xg[1][1].x, xg[1][1].y, xg[1][1].z, xg[1][1].w};
-        const float xo[8] = {xg[2][0].x, xg[2][0].y, xg[2][0].z, xg[2][0].w, xg[2][1].x, xg[2][1].y, xg[2][1].z, xg[2][1].w};
-        const float xc[8] = {xg[3][0].x, xg[3][0].y, xg[3][0].z, xg[3][0].w, xg[3][1].x, xg[3][1].y, xg[3][1].z, xg[3][1].w};
-        __nv_bfloat16 hh[8], ll[8];
-#pragma unroll
-        for (int e = 0; e < 8; e++) {
-          f[e] = sigm_fast(xf[e] + acc[4 * e]);
-          in[e] = sigm_fast(xi[e] + acc[4 * e + 1]);
-          o[e] = sigm_fast(xo[e] + acc[4 * e + 2]);
-          ch[e] = tanh_fast(xc[e] + acc[4 * e + 3]);
-          creg[e] = creg[e] * f[e] + in[e] * ch[e];
-          hn[e] = o[e] * tanh_fast(creg[e]);
-          split_bf16(hn[e], hh[e], ll[e]);
-        }
-        *reinterpret_cast<uint4*>(p.o_hi + hnext) = *reinterpret_cast<uint4*>(hh);
-        *reinterpret_cast<uint4*>(p.o_lo + hnext) = *reinterpret_cast<uint4*>(ll);
-      }
-      if (t + 1 < T) {
-        // publish h_t: bar.sync orders every epilogue thread's stores before thread 64's gpu-scope release (cumulativity);
-        // the reading producers fence generic->async proxy after their acquire
-        if (threadIdx.x == 64) LRCN_TRACE(4);
-        epi_bar_sync();
-        if (threadIdx.x == 64) { LRCN_TRACE(5); fence_proxy_async_global(); grid_arrive(ctr); LRCN_TRACE(6); }
-      }
-      if (active) {  // off the critical path: what only later kernels read
-        float* grow = p.acts + ((size_t)t * B + m) * 4 * H + j;
-        *reinterpret_cast<float4*>(grow) = make_float4(f[0], f[1], f[2], f[3]);
-        *reinterpret_cast<float4*>(grow + 4) = make_float4(f[4], f[5], f[6], f[7]);
-        *reinterpret_cast<float4*>(grow + H) = make_float4(in[0], in[1], in[2], in[3]);
-        *reinterpret_cast<float4*>(grow + H + 4) = make_float4(in[4], in[5], in[6], in[7]);
-        *reinterpret_cast<float4*>(grow + 2 * H) = make_float4(o[0], o[1], o[2], o[3]);
-        *reinterpret_cast<float4*>(grow + 2 * H + 4) = make_float4(o[4], o[5], o[6], o[7]);
-        *reinterpret_cast<float4*>(grow + 3 * H) = make_float4(ch[0], ch[1], ch[2], ch[3]);
-        *reinterpret_cast<float4*>(grow + 3 * H + 4) = make_float4(ch[4], ch[5], ch[6], ch[7]);
-        *reinterpret_cast<float4*>(p.cs + hnext) = make_float4(creg[0], creg[1], creg[2], creg[3]);
-        *reinterpret_cast<float4*>(p.cs + hnext + 4) = make_float4(creg[4], creg[5], creg[6], creg[7]);
-        *reinterpret_cast<float4*>(p.hs + hnext) = make_float4(hn[0], hn[1], hn[2], hn[3]);
-        *reinterpret_cast<float4*>(p.hs + hnext + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
-        if (t + 1 < T) {  // prefetch the next step's x-part
-          const float* gn = p.acts + ((size_t)(t + 1) * B + m) * 4 * H + j;
-#pragma unroll
-          for (int g = 0; g < 4; g++) { xg[g][0] = *reinterpret_cast<const float4*>(gn + g * H); xg[g][1] = *reinterpret_cast<const float4*>(gn + g * H + 4); }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<SEQ_TMEM_COLS>(tmem_base);
-  }
-}
-
-// ============================================================================================================
-// Two interleaved dependency chains per CTA ("seq2").  A step of the recurrence is latency bound: of the ~7 us a
-// 64-row tile needs per step, ~2.7 us are communication (store visibility, grid barrier, TMA of the new h tile) during
-// which the CTA's tensor core and epilogue warps idle.  Batch rows are independent, so the CTA's 64 rows are split into
-// two HALF tiles of 32 rows with their own grid-barrier counter, TMEM accumulator and hand-over buffer; the roles
-// process (t,half 0), (t,half 1), (t+1,half 0), ... so one half computes while the other one communicates.
-// Per half tile the MMA is M=64: A = {h_hi 32 rows; h_lo 32 rows} (one 8 KiB K-major tile per k-block), B = the resident
-// {W_hi 64; W_lo 64} block, N = 128.  UMMA M=64 accumulator: tile row r -> TMEM lane (r%16) + 32*(r/16), i.e.
-//   lane quadrant 0: h_hi rows 0-15    quadrant 1: h_hi rows 16-31    quadrant 2: h_lo rows 0-15    quadrant 3: h_lo rows 16-31
-// (lanes 0-15 of each quadrant);  columns 0-63 = * W_hi,  64-127 = * W_lo.
-// ============================================================================================================
-constexpr int HM = 32;                        // batch rows per half tile
-constexpr int H_AHALF = HM * LBK * 2;         // 4 KiB: {hi | lo} of one k-block of a half tile
-constexpr int H_STAGE = 2 * H_AHALF;          // 8 KiB
-constexpr int F2STAGES = 10;
-constexpr int SLO2_BYTES = HM * SLO_LD * 4;   // per half tile
-constexpr uint32_t SEQ2_TMEM_COLS = 256;      // 2 accumulators x 128 columns
-
-struct Seq2Smem {
-  uint32_t res, ring, full0, empty0, wbar, tfull0, tempty0;
-  uint32_t* tmem_slot;
-  float* slo;  // [2][HM][SLO_LD]
-};
-__device__ __forceinline__ Seq2Smem seq2_smem(uint8_t* smem_raw, int res_kb) {
-  Seq2Smem s;
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* al = smem_raw + (base - smem_u32(smem_raw));
-  s.res = base;
-  s.ring = base + (uint32_t)res_kb * 2 * B_HALF;
-  uint8_t* after = al + (size_t)res_kb * 2 * B_HALF + F2STAGES * H_STAGE;
-  s.slo = reinterpret_cast<float*>(after);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(after + 2 * SLO2_BYTES);
-  s.full0 = smem_u32(bars);
-  s.empty0 = smem_u32(bars + F2STAGES);
-  s.wbar = smem_u32(bars + 2 * F2STAGES);
-  s.tfull0 = smem_u32(bars + 2 * F2STAGES + 1);   // [2]
-  s.tempty0 = smem_u32(bars + 2 * F2STAGES + 3);  // [2]
-  s.tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * F2STAGES + 5);
-  return s;
-}
-static int seq2_smem_bytes(int res_kb) { return res_kb * 2 * B_HALF + F2STAGES * H_STAGE + 2 * SLO2_BYTES + 1024 + 256; }
-
-// named barriers 2 + half: hand-over of the h_lo*W_hi rows from the warps of quadrants 2,3 to the owners (quadrants 0,1)
-__device__ __forceinline__ void slo2_bar_sync(int half) { asm volatile("bar.sync %0, %1;" ::"r"(2 + half), "n"(SEQ_EPI_THREADS) : "memory"); }
-__device__ __forceinline__ void slo2_bar_arrive(int half) { asm volatile("bar.arrive %0, %1;" ::"r"(2 + half), "n"(SEQ_EPI_THREADS) : "memory"); }
-
-// Finished accumulator values of one half tile.  Owner warp (quad 0|1, colhalf): lanes 0-15 hold tile row 16*quad + lane,
-// columns [32*colhalf, +32) = 8 units x 4 gates; units 4-7 move to lanes 16-31 so that every lane ends with 4 units
-// (acc[u*4 + g]) of row 16*quad + (lane & 15).
-__device__ __forceinline__ void half_collect(const Seq2Smem& sm, uint32_t tmem_acc, int hf, int quad, int colhalf, int lane, float (&acc)[16]) {
-  const uint32_t tl = tmem_acc + ((uint32_t)(quad * 32) << 16);
-  float* slo = sm.slo + (size_t)hf * HM * SLO_LD;
-  if (quad >= 2) {
-    uint32_t v[32];
-    LRCN_TMEM_LD_32(tl + (uint32_t)(32 * colhalf), v);  // h_lo * W_hi, tile rows 16*(quad-2) + lane (lanes 0-15)
-    tmem_ld_wait();
-    if (lane < 16) {
-      float* dst = slo + (size_t)(16 * (quad - 2) + lane) * SLO_LD + 32 * colhalf;
-#pragma unroll
-      for (int q = 0; q < 8; q++)
-        *reinterpret_cast<float4*>(dst + 4 * q) = make_float4(__uint_as_float(v[4 * q]), __uint_as_float(v[4 * q + 1]), __uint_as_float(v[4 * q + 2]),
-                                                               __uint_as_float(v[4 * q + 3]));
-    }
-    slo2_bar_arrive(hf);
-  } else {
-    uint32_t v[32], w[32];
-    LRCN_TMEM_LD_32(tl + (uint32_t)(32 * colhalf), v);        // h_hi * W_hi
-    LRCN_TMEM_LD_32(tl + (uint32_t)(64 + 32 * colhalf), w);   // h_hi * W_lo
-    tmem_ld_wait();
-    slo2_bar_sync(hf);
-    const float* src = slo + (size_t)(16 * quad + (lane & 15)) * SLO_LD + 32 * colhalf;
-    float sum[32];
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-      const float4 x = *reinterpret_cast<const float4*>(src + 4 * q);
-      sum[4 * q] = __uint_as_float(v[4 * q]) + __uint_as_float(w[4 * q]) + x.x;
-      sum[4 * q + 1] = __uint_as_float(v[4 * q + 1]) + __uint_as_float(w[4 * q + 1]) + x.y;
-      sum[4 * q + 2] = __uint_as_float(v[4 * q + 2]) + __uint_as_float(w[4 * q + 2]) + x.z;
-      sum[4 * q + 3] = __uint_as_float(v[4 * q + 3]) + __uint_as_float(w[4 * q + 3]) + x.w;
-    }
-#pragma unroll
-    for (int c = 0; c < 16; c++) {
-      const float up = __shfl_sync(0xffffffffu, sum[16 + c], lane & 15);  // units 4-7 of the row held by lane & 15
-      acc[c] = lane < 16 ? sum[c] : up;
-    }
-  }
-}
-
-__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(L_THREADS, 1)
-lstm_fwd_seq2_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                     const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo, const SeqParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const Seq2Smem sm = seq2_smem(smem_raw, p.num_kb);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int nt = blockIdx.x, mt = blockIdx.y, m0 = mt * LM;
-  const int num_kb = p.num_kb, T = p.T, B = p.B, H = p.H;
-  const unsigned int ctas_per_mtile = gridDim.x;
-  unsigned int* ctr = p.counters + 2 * mt;  // [half]
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < F2STAGES; s++) { mbar_init(sm.full0 + 8 * s, 1); mbar_init(sm.empty0 + 8 * s, p.no_mcast ? 1 : CL); }
-    mbar_init(sm.wbar, 1);
-    for (int hf = 0; hf < 2; hf++) { mbar_init(sm.tfull0 + 8 * hf, 1); mbar_init(sm.tempty0 + 8 * hf, 8); }
-    mbar_init_fence();
-  }
-  if (warp == 0 && lane == 0) {
-    prefetch_tensormap(&tmA_hi); prefetch_tensormap(&tmA_lo); prefetch_tensormap(&tmB_hi); prefetch_tensormap(&tmB_lo);
-  }
-  if (warp == 1) tmem_alloc<SEQ2_TMEM_COLS>(smem_u32(sm.tmem_slot));
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *sm.tmem_slot;
-
-  if (warp == 0 && lane == 0) {  // resident weights before the dependency wait (see lstm_fwd_seq_kernel)
-    mbar_expect_tx(sm.wbar, (uint32_t)num_kb * 2 * B_HALF);
-    for (int kb = 0; kb < num_kb; kb++) {
-      tma_load_2d(sm.res + kb * 2 * B_HALF, &tmB_hi, sm.wbar, kb * LBK, nt * NT);
-      tma_load_2d(sm.res + kb * 2 * B_HALF + B_HALF, &tmB_lo, sm.wbar, kb * LBK, nt * NT);
-    }
-  }
-  pdl_wait();
-  pdl_trigger();
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int it = 0;
-      for (int t = 1; t < T; t++) {
-        for (int hf = 0; hf < 2; hf++) {
-          const unsigned int want = (unsigned int)t * ctas_per_mtile * ((p.sync_flags & 2) ? 4u : 1u);
-          if (p.sync_flags & 4) grid_wait_relaxed(ctr + hf, want);
-          else grid_wait(ctr + hf, want);  // h_{t-1} rows of this half tile are complete in global memory
-          if (hf == 0) LRCN_TRACE(0);
-          fence_proxy_async_global();
-          const int arow = t * B + m0 + HM * hf;  // slot t of hs = h_{t-1}
-          for (int kb = 0; kb < num_kb; kb++, it++) {
-            const int s = it % F2STAGES;
-            mbar_wait(sm.empty0 + 8 * s, ((it / F2STAGES) & 1) ^ 1);  // every CTA of the cluster has consumed this stage
-            const uint32_t full = sm.full0 + 8 * s;
-            mbar_expect_tx(full, H_STAGE);
-            const uint32_t st = sm.ring + s * H_STAGE;
-            if (p.no_mcast) {
-              tma_load_2d(st, &tmA_hi, full, kb * LBK, arow);
-              tma_load_2d(st + H_AHALF, &tmA_lo, full, kb * LBK, arow);
-            } else if ((uint32_t)(kb % CL) == rank) {  // k-block kb is fetched by one rank and multicast to the cluster
-              tma_load_2d_mcast(st, &tmA_hi, full, kb * LBK, arow, (uint16_t)((1u << CL) - 1));
-              tma_load_2d_mcast(st + H_AHALF, &tmA_lo, full, kb * LBK, arow, (uint16_t)((1u << CL) - 1));
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      const uint32_t idesc = idesc_bf16(64, 128, false, false);
-      mbar_wait(sm.wbar, 0);
-      int it = 0;
-      for (int t = 1; t < T; t++) {
-        for (int hf = 0; hf < 2; hf++) {
-          if (t >= 2) { mbar_wait(sm.tempty0 + 8 * hf, (t - 2) & 1); tc_fence_after(); }  // epilogue (t-1, hf) has drained this accumulator
-          const uint32_t acc = tmem_base + (uint32_t)(128 * hf);
-          for (int kb = 0; kb < num_kb; kb++, it++) {
-            const int s = it % F2STAGES;
-            mbar_wait(sm.full0 + 8 * s, (it / F2STAGES) & 1);
-            if (hf == 0) { if (kb == 0) LRCN_TRACE(1); else if (kb == 3) LRCN_TRACE(5); else if (kb == num_kb - 1) LRCN_TRACE(7); }
-            tc_fence_after();
-            stacked_mma_kblock(acc, sm.ring + s * H_STAGE, sm.res + kb * 2 * B_HALF, idesc, kb == 0);
-            if (p.no_mcast) umma_commit(sm.empty0 + 8 * s);
-            else umma_commit_mcast(sm.empty0 + 8 * s, (uint16_t)((1u << CL) - 1));
-          }
-          umma_commit(sm.tfull0 + 8 * hf);
-          if (hf == 0) LRCN_TRACE(2);
-        }
-      }
-    }
-  } else {
-    const int ew = warp - 2, quad = warp & 3, colhalf = ew >> 2;
-    const bool owner = quad < 2;
-    const int rih = 16 * quad + (lane & 15);                  // row inside the half tile (owner only)
-    const int j = nt * (NT / 4) + 8 * colhalf + 4 * (lane >> 4);  // first of this thread's 4 units
-    bool active[2];
-    int mrow[2];
-    float creg[2][4];
-    float4 xg[2][4];
-#pragma unroll
-    for (int hf = 0; hf < 2; hf++) {
-      mrow[hf] = m0 + HM * hf + rih;
-      active[hf] = owner && mrow[hf] < B && j < H;
-#pragma unroll
-      for (int e = 0; e < 4; e++) creg[hf][e] = 0.f;
-#pragma unroll
-      for (int g = 0; g < 4; g++) xg[hf][g] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (active[hf]) {
-        const float* g0 = p.acts + (size_t)mrow[hf] * 4 * H + j;
-#pragma unroll
-        for (int g = 0; g < 4; g++) xg[hf][g] = *reinterpret_cast<const float4*>(g0 + g * H);
-      }
-    }
-    for (int t = 0; t < T; t++) {
-#pragma unroll
-      for (int hf = 0; hf < 2; hf++) {
-        float acc[16];  // unit-major: acc[u*4 + g]
-        if (t > 0) {
-          mbar_wait(sm.tfull0 + 8 * hf, (t - 1) & 1);
-          if (threadIdx.x == 64 && hf == 0) LRCN_TRACE(3);
-          tc_fence_after();
-          half_collect(sm, tmem_base + (uint32_t)(128 * hf), hf, quad, colhalf, lane, acc);
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(sm.tempty0 + 8 * hf);
-        } else {
-#pragma unroll
-          for (int c = 0; c < 16; c++) acc[c] = 0.f;
-        }
-        float f[4], in[4], o[4], ch[4], hn[4];
-        const size_t hnext = ((size_t)(t + 1) * B + mrow[hf]) * H + j;
-        if (active[hf]) {
-          const float xf[4] = {xg[hf][0].x, xg[hf][0].y, xg[hf][0].z, xg[hf][0].w}, xi[4] = {xg[hf][1].x, xg[hf][1].y, xg[hf][1].z, xg[hf][1].w};
-          const float xo[4] = {xg[hf][2].x, xg[hf][2].y, xg[hf][2].z, xg[hf][2].w}, xc[4] = {xg[hf][3].x, xg[hf][3].y, xg[hf][3].z, xg[hf][3].w};
-          __nv_bfloat16 hh[4], ll[4];
-#pragma unroll
-          for (int e = 0; e < 4; e++) {
-            f[e] = sigm_fast(xf[e] + acc[4 * e]);
-            in[e] = sigm_fast(xi[e] + acc[4 * e + 1]);
-            o[e] = sigm_fast(xo[e] + acc[4 * e + 2]);
-            ch[e] = tanh_fast(xc[e] + acc[4 * e + 3]);
-            creg[hf][e] = creg[hf][e] * f[e] + in[e] * ch[e];
-            hn[e] = o[e] * tanh_fast(creg[hf][e]);
-            split_bf16(hn[e], hh[e], ll[e]);
-          }
-          *reinterpret_cast<uint2*>(p.o_hi + hnext) = *reinterpret_cast<uint2*>(hh);
-          *reinterpret_cast<uint2*>(p.o_lo + hnext) = *reinterpret_cast<uint2*>(ll);
-        }
-        if (t + 1 < T) {
-          // publish h_t of this half tile: bar.sync orders every epilogue thread's stores before thread 64's gpu-scope release
-          if (p.sync_flags & 2) {  // every owner warp publishes its own rows (the slo / accumulator reuse is ordered by the data flow)
-            if (owner) {
-              __syncwarp();
-              if (lane == 0) { if (!(p.sync_flags & 1)) fence_proxy_async_global(); grid_arrive(ctr + hf); }
-            }
-          } else {
-            epi_bar_sync();
-            if (threadIdx.x == 64 && hf == 0) LRCN_TRACE(4);
-            if (threadIdx.x == 64) { if (!(p.sync_flags & 1)) fence_proxy_async_global(); grid_arrive(ctr + hf); if (hf == 0) LRCN_TRACE(6); }
-          }
-        }
-        if (active[hf]) {  // off the critical path: what only later kernels read
-          float* grow = p.acts + ((size_t)t * B + mrow[hf]) * 4 * H + j;
-          *reinterpret_cast<float4*>(grow) = make_float4(f[0], f[1], f[2], f[3]);
-          *reinterpret_cast<float4*>(grow + H) = make_float4(in[0], in[1], in[2], in[3]);
-          *reinterpret_cast<float4*>(grow + 2 * H) = make_float4(o[0], o[1], o[2], o[3]);
-          *reinterpret_cast<float4*>(grow + 3 * H) = make_float4(ch[0], ch[1], ch[2], ch[3]);
-          *reinterpret_cast<float4*>(p.cs + hnext) = make_float4(creg[hf][0], creg[hf][1], creg[hf][2], creg[hf][3]);
-          *reinterpret_cast<float4*>(p.hs + hnext) = make_float4(hn[0], hn[1], hn[2], hn[3]);
-          if (t + 1 < T) {  // prefetch the next step's x-part
-            const float* gn = p.acts + ((size_t)(t + 1) * B + mrow[hf]) * 4 * H + j;
-#pragma unroll
-            for (int g = 0; g < 4; g++) xg[hf][g] = *reinterpret_cast<const float4*>(gn + g * H);
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<SEQ2_TMEM_COLS>(tmem_base);
-  }
-}
 
 // ============================================================================================================
 // TRANSPOSED, TWO-CHAIN forward sequence kernel, recurrent weights resident in TENSOR MEMORY + shared memory ("seq4", round 2).
@@ -1464,245 +884,6 @@ lstm_fwd_seq4_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_co
   if (warp == T4_MAXCH) {
     tc_fence_after();
     tmem_dealloc<T4_TMEM_COLS>(tmem_base);
-  }
-}
-
-// ---- backward: all T steps of one layer, t = T-1 .. 0.  grid = (n-tiles*CL, m-tiles); the CL CTAs of a cluster are the
-// K-slices of one 64x64 output tile; partials are exchanged through DSMEM with remote mbarrier arrives.
-__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(L_THREADS, 1)
-lstm_bwd_seq_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
-                    const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo, const SeqParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  const int kb_per = (p.num_kb + CL - 1) / CL;
-  const SeqSmem sm = seq_smem<BSTAGES, true>(smem_raw, kb_per);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int nt = blockIdx.x / CL, mt = blockIdx.y, m0 = mt * LM;
-  const int T = p.T, B = p.B, H = p.H;
-  const int kb_begin = (int)rank * kb_per;
-  const int nkb = max(0, min(p.num_kb, kb_begin + kb_per) - kb_begin);
-  const unsigned int ctas_per_mtile = gridDim.x;
-  unsigned int* ctr = p.counters + mt;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < BSTAGES; s++) { mbar_init(sm.full0 + 8 * s, 1); mbar_init(sm.empty0 + 8 * s, 1); }
-    mbar_init(sm.wbar, 1); mbar_init(sm.tfull, 1); mbar_init(sm.tempty, 8);
-    mbar_init(sm.redfull, CL * 64); mbar_init(sm.redempty, CL);
-    mbar_init_fence();
-  }
-  if (warp == 0 && lane == 0) {
-    prefetch_tensormap(&tmA_hi); prefetch_tensormap(&tmA_lo); prefetch_tensormap(&tmB_hi); prefetch_tensormap(&tmB_lo);
-  }
-  if (warp == 1) tmem_alloc<SEQ_TMEM_COLS>(smem_u32(sm.tmem_slot));
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *sm.tmem_slot;
-
-  if (warp == 0 && lane == 0 && nkb > 0) {  // resident weights before the dependency wait (see lstm_fwd_seq_kernel)
-    mbar_expect_tx(sm.wbar, (uint32_t)nkb * 2 * B_HALF);
-    for (int i = 0; i < nkb; i++) {
-      tma_load_2d(sm.res + i * 2 * B_HALF, &tmB_hi, sm.wbar, (kb_begin + i) * LBK, nt * NT);
-      tma_load_2d(sm.res + i * 2 * B_HALF + B_HALF, &tmB_lo, sm.wbar, (kb_begin + i) * LBK, nt * NT);
-    }
-  }
-  pdl_wait();
-  pdl_trigger();
-
-  if (warp == 0) {
-    if (lane == 0 && nkb > 0) {
-      int it = 0;
-      for (int t = T - 2; t >= 0; t--) {
-        grid_wait(ctr, (unsigned int)(T - 1 - t) * ctas_per_mtile);  // dG_{t+1} rows of this m-tile are complete
-        fence_proxy_async_global();
-        const int arow = (t + 1) * B + m0;
-        for (int i = 0; i < nkb; i++, it++) {
-          const int s = it % BSTAGES;
-          mbar_wait(sm.empty0 + 8 * s, ((it / BSTAGES) & 1) ^ 1);
-          const uint32_t full = sm.full0 + 8 * s;
-          mbar_expect_tx(full, RSTAGE);
-          const uint32_t st = sm.ring + s * RSTAGE;
-          tma_load_2d(st, &tmA_hi, full, (kb_begin + i) * LBK, arow);
-          tma_load_2d(st + A_HALF, &tmA_lo, full, (kb_begin + i) * LBK, arow);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0 && nkb > 0) {
-      const uint32_t idesc = idesc_bf16(128, 128, false, false);
-      mbar_wait(sm.wbar, 0);
-      int it = 0, n = 0;
-      for (int t = T - 2; t >= 0; t--, n++) {
-        if (n >= 1) { mbar_wait(sm.tempty, (n - 1) & 1); tc_fence_after(); }
-        for (int i = 0; i < nkb; i++, it++) {
-          const int s = it % BSTAGES;
-          mbar_wait(sm.full0 + 8 * s, (it / BSTAGES) & 1);
-          tc_fence_after();
-          stacked_mma_kblock(tmem_base, sm.ring + s * RSTAGE, sm.res + i * 2 * B_HALF, idesc, i == 0);
-          umma_commit(sm.empty0 + 8 * s);
-        }
-        umma_commit(sm.tfull);
-      }
-    }
-  } else {
-    const int ew = warp - 2, quad = warp & 3, half = ew >> 2, upper = lane >> 4;
-    // phase-2 ownership (independent of the TMEM layout): 256 threads x 4 units of this CTA's 16 units
-    const int row = (ew & 3) * 16 + (lane & 15);
-    const int ug = 2 * half + upper;
-    const int m = m0 + row;
-    const int j = nt * NT + 16 * (int)rank + 4 * ug;
-    const bool active = m < B && j < H;
-    // Off the step-to-step critical path: the stored activations / cell states / dh of step t are prefetched while step
-    // t+1 is still in flight, dc stays in registers, and only the bf16 split of dG_t is stored before the barrier arrive.
-    float dcreg[4] = {0.f, 0.f, 0.f, 0.f};
-    float bsum[4][4];  // [gate][unit]: this thread's share of the bias gradient (sum of dG over its row and all steps)
-#pragma unroll
-    for (int g = 0; g < 4; g++)
-#pragma unroll
-      for (int e = 0; e < 4; e++) bsum[g][e] = 0.f;
-    float4 pf, pi, po, pg, pcp, pcc, pdh;
-    pf = pi = po = pg = pcp = pcc = pdh = make_float4(0.f, 0.f, 0.f, 0.f);
-    auto prefetch = [&](int tt) {
-      const float* g0 = p.acts + ((size_t)tt * B + m) * 4 * H + j;
-      pf = *reinterpret_cast<const float4*>(g0); pi = *reinterpret_cast<const float4*>(g0 + H);
-      po = *reinterpret_cast<const float4*>(g0 + 2 * H); pg = *reinterpret_cast<const float4*>(g0 + 3 * H);
-      pcp = *reinterpret_cast<const float4*>(p.cs + ((size_t)tt * B + m) * H + j);
-      pcc = *reinterpret_cast<const float4*>(p.cs + ((size_t)(tt + 1) * B + m) * H + j);
-      pdh = *reinterpret_cast<const float4*>(p.dh_all + ((size_t)tt * B + m) * H + j);
-    };
-    if (active) prefetch(T - 1);
-    int n = 0;  // index of the recurrent step (steps with a partial product)
-    for (int t = T - 1; t >= 0; t--) {
-      const bool has_rec = t < T - 1;
-      float rec[4] = {0.f, 0.f, 0.f, 0.f};
-      if (has_rec) {
-        // phase 1: finish my partial (hi*hi + hi*lo + lo*hi) and scatter it to the owners of its columns
-        float part[32];
-        if (nkb > 0) {
-          mbar_wait(sm.tfull, n & 1);
-          tc_fence_after();
-          stacked_collect(sm, tmem_base, quad, half, lane, part);
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(sm.tempty);
-        } else {
-#pragma unroll
-          for (int c = 0; c < 32; c++) part[c] = 0.f;
-        }
-        if (n >= 1) mbar_wait_cluster(sm.redempty, (n - 1) & 1);  // every owner has consumed my previous partial
-        if (quad < 2) {
-          const int prow = 32 * quad + lane;  // tile row held by this thread; its columns are [32*half, +32)
-          const uint32_t local = smem_u32(sm.red) + (uint32_t)(((int)rank * LM + prow) * (NT / CL)) * 4u;
-#pragma unroll
-          for (int d2 = 0; d2 < 2; d2++) {
-            const uint32_t dst = (uint32_t)(2 * half + d2);
-            const uint32_t ra = dsmem_addr(local, dst);
-#pragma unroll
-            for (int q = 0; q < 4; q++)
-              dsmem_st_f4(ra + 16u * q, make_float4(part[16 * d2 + 4 * q], part[16 * d2 + 4 * q + 1], part[16 * d2 + 4 * q + 2], part[16 * d2 + 4 * q + 3]));
-            mbar_arrive_remote(dsmem_addr(sm.redfull, dst));  // release.cluster: orders my stores before the owner's acquire
-          }
-        }
-        // phase 2: sum the CL partials of my 16 units
-        mbar_wait_cluster(sm.redfull, n & 1);
-#pragma unroll
-        for (int src = 0; src < CL; src++) {
-          const float4 x = *reinterpret_cast<const float4*>(sm.red + (size_t)(src * LM + row) * (NT / CL) + 4 * ug);
-          rec[0] += x.x; rec[1] += x.y; rec[2] += x.z; rec[3] += x.w;
-        }
-        n++;
-      }
-      float r0[4], r1[4], r2[4], r3[4];
-      const size_t gidx = ((size_t)t * B + m) * 4 * H + j;
-      if (active) {
-        const float f[4] = {pf.x, pf.y, pf.z, pf.w}, in[4] = {pi.x, pi.y, pi.z, pi.w}, o[4] = {po.x, po.y, po.z, po.w}, ch[4] = {pg.x, pg.y, pg.z, pg.w};
-        const float cpv[4] = {pcp.x, pcp.y, pcp.z, pcp.w}, ccv[4] = {pcc.x, pcc.y, pcc.z, pcc.w}, dhv[4] = {pdh.x, pdh.y, pdh.z, pdh.w};
-#pragma unroll
-        for (int e = 0; e < 4; e++) {
-          const float dh = dhv[e] + rec[e];
-          const float tc = tanh_fast(ccv[e]);
-          const float dcv = dcreg[e] + dh * o[e] * (1.f - tc * tc);
-          const float dO = dh * tc, dF = dcv * cpv[e], dI = dcv * ch[e], dG = dcv * in[e];
-          dcreg[e] = dcv * f[e];
-          r0[e] = dF * f[e] * (1.f - f[e]);
-          r1[e] = dI * in[e] * (1.f - in[e]);
-          r2[e] = dO * o[e] * (1.f - o[e]);
-          r3[e] = dG * (1.f - ch[e] * ch[e]);
-        }
-        const float* rr[4] = {r0, r1, r2, r3};
-#pragma unroll
-        for (int g = 0; g < 4; g++)
-#pragma unroll
-          for (int e = 0; e < 4; e++) bsum[g][e] += rr[g][e];
-#pragma unroll
-        for (int g = 0; g < 4; g++) {  // the bf16 split of dG_t is what the next step's TMA reads: store it first
-          __nv_bfloat16 hh[4], ll[4];
-#pragma unroll
-          for (int e = 0; e < 4; e++) split_bf16(rr[g][e], hh[e], ll[e]);
-          *reinterpret_cast<uint2*>(p.o_hi + gidx + (size_t)g * H) = *reinterpret_cast<uint2*>(hh);
-          *reinterpret_cast<uint2*>(p.o_lo + gidx + (size_t)g * H) = *reinterpret_cast<uint2*>(ll);
-        }
-      }
-      if (t > 0) {  // publish dG_t
-        epi_bar_sync();  // orders all epilogue stores before the release below; also: all 256 readers are done with red
-        if (threadIdx.x == 64) {
-          fence_proxy_async_global();
-          grid_arrive(ctr);
-          if (has_rec) {
-#pragma unroll
-            for (int d = 0; d < CL; d++) mbar_arrive_remote(dsmem_addr(sm.redempty, (uint32_t)d));  // my red slots are free again
-          }
-        }
-      }
-      if (active) {  // off the critical path
-        float* grow = p.acts + gidx;
-        *reinterpret_cast<float4*>(grow) = make_float4(r0[0], r0[1], r0[2], r0[3]);
-        *reinterpret_cast<float4*>(grow + H) = make_float4(r1[0], r1[1], r1[2], r1[3]);
-        *reinterpret_cast<float4*>(grow + 2 * H) = make_float4(r2[0], r2[1], r2[2], r2[3]);
-        *reinterpret_cast<float4*>(grow + 3 * H) = make_float4(r3[0], r3[1], r3[2], r3[3]);
-        if (t > 0) prefetch(t - 1);
-      }
-    }
-    if (p.dbias) {
-      // bias gradient: sum over the 16 rows of each half warp by shuffles, over the 4 warps sharing a unit group through smem
-      // (the hand-over buffer is free now), then one atomic per (gate, unit) and CTA onto the zero-initialised gradient
-#pragma unroll
-      for (int g = 0; g < 4; g++)
-#pragma unroll
-        for (int e = 0; e < 4; e++) {
-          float v = bsum[g][e];
-          v += __shfl_xor_sync(0xffffffffu, v, 1); v += __shfl_xor_sync(0xffffffffu, v, 2);
-          v += __shfl_xor_sync(0xffffffffu, v, 4); v += __shfl_xor_sync(0xffffffffu, v, 8);
-          bsum[g][e] = v;
-        }
-      epi_bar_sync();  // every epilogue thread is past its last use of the hand-over buffer
-      float* bred = sm.slo;  // [8 warps][2 upper][16]
-      if ((lane & 15) == 0) {
-#pragma unroll
-        for (int g = 0; g < 4; g++)
-#pragma unroll
-          for (int e = 0; e < 4; e++) bred[(ew * 2 + upper) * 16 + g * 4 + e] = bsum[g][e];
-      }
-      epi_bar_sync();
-      const int tid = threadIdx.x - 64;  // 0..255 among the epilogue threads
-      if (tid < 64) {
-        const int ugq = tid >> 4, ge = tid & 15, g = ge >> 2, e = ge & 3;  // unit group, gate, unit within the group
-        const int hf = ugq >> 1, up = ugq & 1;
-        float v = 0.f;
-#pragma unroll
-        for (int w4 = 0; w4 < 4; w4++) v += bred[((hf * 4 + w4) * 2 + up) * 16 + ge];
-        const int jj = nt * NT + 16 * (int)rank + 4 * ugq + e;
-        if (jj < H) atomicAdd(p.dbias + (size_t)g * H + jj, v);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<SEQ_TMEM_COLS>(tmem_base);
   }
 }
 
@@ -2203,11 +1384,11 @@ bool lstm_bwd_step(cudaStream_t s, int B, int H, bool has_rec, const __nv_bfloat
 }
 
 static int g_lstm_sms = 0;
-// Can the persistent kernels be used?  (weights must fit beside the ring; the whole grid must be co-resident)
-static bool seq_fits(const void* kernel, int res_kb, dim3 grid, int smem_bytes, int threads = L_THREADS) {
+// Can the persistent kernel be used?  (its weight k-blocks must fit on chip; the whole grid must be co-resident)
+static bool seq_fits(const void* kernel, int res_kb, dim3 grid, int smem_bytes) {
   if (res_kb > MAX_RES_KB) return false;
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem_bytes;
+  cfg.gridDim = grid; cfg.blockDim = dim3(T4_THREADS); cfg.dynamicSmemBytes = smem_bytes;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
@@ -2216,62 +1397,38 @@ static bool seq_fits(const void* kernel, int res_kb, dim3 grid, int smem_bytes, 
   return (long long)nclusters * CL >= (long long)grid.x * grid.y;
 }
 
-// whole-sequence forward of one layer; returns false (nothing launched) when the persistent kernel does not apply
+// whole-sequence forward of one layer; returns true with *launched = false when the persistent kernel does not apply
 bool lstm_fwd_seq(cudaStream_t s, int B, int H, int T, const __nv_bfloat16* wperm_hi, const __nv_bfloat16* wperm_lo, float* acts, float* hs,
                   float* cs, __nv_bfloat16* hs_hi, __nv_bfloat16* hs_lo, unsigned int* counters, bool* launched, unsigned long long* trace) {
   *launched = false;
+  if (T < 2) return true;
   const int num_kb = (H + LBK - 1) / LBK;
   const int nt = (H + F_NH - 1) / F_NH;
-  static const bool no_seq4 = getenv("LRCN_SEQ_V2") != nullptr || getenv("LRCN_SEQ_V1") != nullptr;  // round-1 kernels
-  if (!no_seq4 && T >= 2) {
-    // transposed multi-chain kernel: the fewest chains per CTA (= the most CTAs) whose grid is still co-resident
-    for (int nch = 1; nch <= T4_MAXCH; nch *= 2) {
-      const int rows = T4_ROWS * nch;
-      dim3 grid4((nt + CL - 1) / CL * CL, (B + rows - 1) / rows);
-      if (grid4.y * T4_MAXCH > 64) continue;  // one counter per (m-tile, chain)
-      if (!seq_fits((const void*)lstm_fwd_seq4_kernel, num_kb, grid4, seq4_smem_bytes(), T4_THREADS)) continue;
-      const int Hp = (H + 7) / 8 * 8, wrows = fwd_rows(H);
-      CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo;
-      if (!get_tensor_map_bf16(&tb_hi, wperm_hi, H, wrows, Hp, F_NT) || !get_tensor_map_bf16(&tb_lo, wperm_lo, H, wrows, Hp, F_NT)) return false;
-      const uint64_t R = (uint64_t)(T + 1) * B;
-      if (!get_tensor_map_bf16(&ta_hi, hs_hi, H, R, H, T4_ROWS) || !get_tensor_map_bf16(&ta_lo, hs_lo, H, R, H, T4_ROWS)) return false;
-      SeqParams p{};
-      p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.hs = hs; p.cs = cs; p.o_hi = hs_hi; p.o_lo = hs_lo; p.counters = counters;
-      p.trace = trace;
-      static const int dbg_flags = getenv("LRCN_SEQ_SYNC") ? atoi(getenv("LRCN_SEQ_SYNC")) : 0;
-      p.sync_flags = dbg_flags;
-      launch_pdl(lstm_fwd_seq4_kernel, grid4, dim3(T4_THREADS), seq4_smem_bytes(), s, ta_hi, ta_lo, tb_hi, tb_lo, wperm_hi, wperm_lo, wrows, Hp, p, nch);
-      if (g_counter) g_counter->n++;
-      *launched = true;
-      return check_launch("lstm_fwd_seq4 launch");
-    }
+  // the fewest chains per CTA (= the most CTAs) whose grid is still co-resident
+  for (int nch = 1; nch <= T4_MAXCH; nch *= 2) {
+    const int rows = T4_ROWS * nch;
+    dim3 grid4((nt + CL - 1) / CL * CL, (B + rows - 1) / rows);
+    if (grid4.y * T4_MAXCH > 64) continue;  // one counter per (m-tile, chain)
+    if (!seq_fits((const void*)lstm_fwd_seq4_kernel, num_kb, grid4, seq4_smem_bytes())) continue;
+    const int Hp = (H + 7) / 8 * 8, wrows = fwd_rows(H);
+    CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo;
+    if (!get_tensor_map_bf16(&tb_hi, wperm_hi, H, wrows, Hp, F_NT) || !get_tensor_map_bf16(&tb_lo, wperm_lo, H, wrows, Hp, F_NT)) return false;
+    const uint64_t R = (uint64_t)(T + 1) * B;
+    if (!get_tensor_map_bf16(&ta_hi, hs_hi, H, R, H, T4_ROWS) || !get_tensor_map_bf16(&ta_lo, hs_lo, H, R, H, T4_ROWS)) return false;
+    SeqParams p{};
+    p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.hs = hs; p.cs = cs; p.o_hi = hs_hi; p.o_lo = hs_lo; p.counters = counters;
+    p.trace = trace;
+    static const int dbg_flags = getenv("LRCN_SEQ_SYNC") ? atoi(getenv("LRCN_SEQ_SYNC")) : 0;
+    p.sync_flags = dbg_flags;
+    launch_pdl(lstm_fwd_seq4_kernel, grid4, dim3(T4_THREADS), seq4_smem_bytes(), s, ta_hi, ta_lo, tb_hi, tb_lo, wperm_hi, wperm_lo, wrows, Hp, p, nch);
+    if (g_counter) g_counter->n++;
+    *launched = true;
+    return check_launch("lstm_fwd_seq4 launch");
   }
-  dim3 grid((nt + CL - 1) / CL * CL, (B + LM - 1) / LM);
-  static const bool v1 = getenv("LRCN_SEQ_V1") != nullptr;  // the single-chain kernel (one 64-row tile per step)
-  const bool two = !v1 && grid.y * 2 <= 64;                // seq2: two interleaved 32-row chains, one counter per half tile
-  if (T < 2) return true;
-  if (two ? !seq_fits((const void*)lstm_fwd_seq2_kernel, num_kb, grid, seq2_smem_bytes(num_kb))
-          : !seq_fits((const void*)lstm_fwd_seq_kernel, num_kb, grid, seq_smem_bytes(num_kb, false)))
-    return true;
-  const int Hp = (H + 7) / 8 * 8, rows = fwd_rows(H);
-  CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo;
-  if (!get_tensor_map_bf16(&tb_hi, wperm_hi, H, rows, Hp, F_NT) || !get_tensor_map_bf16(&tb_lo, wperm_lo, H, rows, Hp, F_NT)) return false;
-  const uint64_t R = (uint64_t)(T + 1) * B;
-  const uint32_t box_rows = two ? HM : LM;
-  if (!get_tensor_map_bf16(&ta_hi, hs_hi, H, R, H, box_rows) || !get_tensor_map_bf16(&ta_lo, hs_lo, H, R, H, box_rows)) return false;
-  SeqParams p{};
-  p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.hs = hs; p.cs = cs; p.o_hi = hs_hi; p.o_lo = hs_lo; p.counters = counters; p.trace = trace;
-  static const bool no_mcast = getenv("LRCN_SEQ_NOMCAST") != nullptr;
-  p.no_mcast = no_mcast ? 1 : 0;
-  static const int sync_flags = getenv("LRCN_SEQ_SYNC") ? atoi(getenv("LRCN_SEQ_SYNC")) : 0;
-  p.sync_flags = sync_flags;
-  if (two) launch_pdl(lstm_fwd_seq2_kernel, grid, dim3(L_THREADS), seq2_smem_bytes(num_kb), s, ta_hi, ta_lo, tb_hi, tb_lo, p);
-  else launch_pdl(lstm_fwd_seq_kernel, grid, dim3(L_THREADS), seq_smem_bytes(num_kb, false), s, ta_hi, ta_lo, tb_hi, tb_lo, p);
-  if (g_counter) g_counter->n++;
-  *launched = true;
-  return check_launch("lstm_fwd_seq launch");
+  return true;
 }
 
+// whole-sequence backward of one layer; same contract as lstm_fwd_seq
 bool lstm_bwd_seq(cudaStream_t s, int B, int H, int T, const __nv_bfloat16* wt_hi, const __nv_bfloat16* wt_lo, float* acts,
                   __nv_bfloat16* acts_hi, __nv_bfloat16* acts_lo, float* cs, const float* dh_all, float* dc, unsigned int* counters,
                   bool* launched, float* dbias, unsigned long long* trace) {
@@ -2280,40 +1437,26 @@ bool lstm_bwd_seq(cudaStream_t s, int B, int H, int T, const __nv_bfloat16* wt_h
   const int num_kb = (int)((K + LBK - 1) / LBK);
   const int kb_per = (num_kb + CL - 1) / CL;
   const int nt = (H + R_NT - 1) / R_NT;
-  static const bool no_seq4 = getenv("LRCN_SEQ_V2") != nullptr || getenv("LRCN_SEQ_V1") != nullptr;  // round-1 kernel
-  if (!no_seq4 && T >= 2 && kb_per <= MAX_RES_KB) {
-    for (int nch = 1; nch <= T4_MAXCH; nch *= 2) {
-      const int rows = T4_ROWS * nch;
-      dim3 grid4(nt * CL, (B + rows - 1) / rows);
-      if (grid4.y * T4_MAXCH > 64) continue;  // one counter per (m-tile, chain)
-      if (!seq_fits((const void*)lstm_bwd_seq4_kernel, kb_per, grid4, bwd4_smem_bytes(), T4_THREADS)) continue;
-      CUtensorMap ta_hi, ta_lo;
-      const uint64_t R = (uint64_t)T * B;
-      if (!get_tensor_map_bf16(&ta_hi, acts_hi, K, R, K, T4_ROWS) || !get_tensor_map_bf16(&ta_lo, acts_lo, K, R, K, T4_ROWS)) return false;
-      SeqParams p{};
-      p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.cs = cs; p.o_hi = acts_hi; p.o_lo = acts_lo; p.dh_all = dh_all; p.dc = dc;
-      p.counters = counters; p.dbias = dbias; p.trace = trace;
-      static const int dbg_flags = getenv("LRCN_SEQ_SYNC") ? atoi(getenv("LRCN_SEQ_SYNC")) : 0;
-      p.sync_flags = dbg_flags;
-      launch_pdl(lstm_bwd_seq4_kernel, grid4, dim3(T4_THREADS), bwd4_smem_bytes(), s, ta_hi, ta_lo, wt_hi, wt_lo, bwd_rows(H), p, nch);
-      if (g_counter) g_counter->n++;
-      *launched = true;
-      return check_launch("lstm_bwd_seq4 launch");
-    }
+  if (T < 2 || kb_per > MAX_RES_KB) return true;
+  for (int nch = 1; nch <= T4_MAXCH; nch *= 2) {
+    const int rows = T4_ROWS * nch;
+    dim3 grid4(nt * CL, (B + rows - 1) / rows);
+    if (grid4.y * T4_MAXCH > 64) continue;  // one counter per (m-tile, chain)
+    if (!seq_fits((const void*)lstm_bwd_seq4_kernel, kb_per, grid4, bwd4_smem_bytes())) continue;
+    CUtensorMap ta_hi, ta_lo;
+    const uint64_t R = (uint64_t)T * B;
+    if (!get_tensor_map_bf16(&ta_hi, acts_hi, K, R, K, T4_ROWS) || !get_tensor_map_bf16(&ta_lo, acts_lo, K, R, K, T4_ROWS)) return false;
+    SeqParams p{};
+    p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.cs = cs; p.o_hi = acts_hi; p.o_lo = acts_lo; p.dh_all = dh_all; p.dc = dc;
+    p.counters = counters; p.dbias = dbias; p.trace = trace;
+    static const int dbg_flags = getenv("LRCN_SEQ_SYNC") ? atoi(getenv("LRCN_SEQ_SYNC")) : 0;
+    p.sync_flags = dbg_flags;
+    launch_pdl(lstm_bwd_seq4_kernel, grid4, dim3(T4_THREADS), bwd4_smem_bytes(), s, ta_hi, ta_lo, wt_hi, wt_lo, bwd_rows(H), p, nch);
+    if (g_counter) g_counter->n++;
+    *launched = true;
+    return check_launch("lstm_bwd_seq4 launch");
   }
-  dim3 grid(nt * CL, (B + LM - 1) / LM);
-  if (T < 2 || !seq_fits((const void*)lstm_bwd_seq_kernel, kb_per, grid, seq_smem_bytes(kb_per, true))) return true;
-  CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo;
-  if (!get_tensor_map_bf16(&tb_hi, wt_hi, K, bwd_rows(H), K, R_NT) || !get_tensor_map_bf16(&tb_lo, wt_lo, K, bwd_rows(H), K, R_NT)) return false;
-  const uint64_t R = (uint64_t)T * B;
-  if (!get_tensor_map_bf16(&ta_hi, acts_hi, K, R, K, LM) || !get_tensor_map_bf16(&ta_lo, acts_lo, K, R, K, LM)) return false;
-  SeqParams p{};
-  p.B = B; p.H = H; p.T = T; p.num_kb = num_kb; p.acts = acts; p.cs = cs; p.o_hi = acts_hi; p.o_lo = acts_lo; p.dh_all = dh_all; p.dc = dc;
-  p.counters = counters; p.dbias = dbias;
-  launch_pdl(lstm_bwd_seq_kernel, grid, dim3(L_THREADS), seq_smem_bytes(kb_per, true), s, ta_hi, ta_lo, tb_hi, tb_lo, p);
-  if (g_counter) g_counter->n++;
-  *launched = true;
-  return check_launch("lstm_bwd_seq launch");
+  return true;
 }
 
 bool lstm_bind_abort(unsigned int* host_flag) { return dev_abort_bind(host_flag) == cudaSuccess; }
@@ -2321,9 +1464,6 @@ bool lstm_bind_abort(unsigned int* host_flag) { return dev_abort_bind(host_flag)
 bool init_lstm_sm100() {
   cudaError_t e = cudaFuncSetAttribute(lstm_fwd_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_bwd_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_fwd_seq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, seq_smem_bytes(MAX_RES_KB, false));
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_bwd_seq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, seq_smem_bytes(MAX_RES_KB, true));
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_fwd_seq2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, seq2_smem_bytes(MAX_RES_KB));
   if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_fwd_seq4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, seq4_smem_bytes());
   if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_bwd_seq4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bwd4_smem_bytes());
   if (e != cudaSuccess) { set_sm100_error((std::string("cudaFuncSetAttribute(lstm): ") + cudaGetErrorString(e)).c_str()); return false; }

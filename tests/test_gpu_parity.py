@@ -126,6 +126,8 @@ CASES = [
     dict(E=64, H1=512, H2=512, V=300, B=80, l=7, scale=1.5),   # bench-sized hidden state: 8 k-blocks, 2 m-tiles (second one ragged)
     dict(E=64, H1=640, H2=320, V=200, B=70, l=4, scale=1.5),   # H1 too large for weight residency -> per-step kernels for layer 1
     dict(E=104, H1=200, H2=200, V=333, B=33, l=5, scale=2.0),  # coco_2f-like ragged dims (H=1000 there): K, N not multiples of 64/16
+    dict(E=64, H1=64, H2=64, V=300, B=2048, l=3),   # the largest batch the persistent LSTM kernels take (32 m-tiles x 2 chains)
+    dict(E=64, H1=64, H2=64, V=300, B=2049, l=3),   # one row more: per-step LSTM kernels
 ]
 
 

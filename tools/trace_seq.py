@@ -23,36 +23,24 @@ for i in range(4):
     h.train_step_staged(0, 0.0, i)
 h.sync()
 T = l + 1
-if os.environ.get("LRCN_SEQ_V2"):
-    tr = h.get_trace(T).astype(np.int64)
-    names = ["0 grid_wait done", "1 kb0 landed", "2 MMAs issued+commit", "3 epilogue: tfull seen", "4 all epilogue warps done (bar.sync)", "5 kb3 landed", "6 release done", "7 last kb landed"]
-    print("step | " + " | ".join(names) + "   (ns relative to this step's grid_wait)")
-    for t in range(1, l + 1):
-        base = tr[t, 0]
-        row = [int(tr[t, k] - base) if tr[t, k] else -1 for k in range(8)]
-        nxt = tr[t + 1, 0] - base if t + 1 <= l and tr[t + 1, 0] else -1
-        print(t, row, "next grid_wait at", nxt)
-else:
-    # seq4: [T][4 chains][8]: 0 barrier open (producer) | 1 chunk's TMAs issued | 2 kb0 landed (issuer) | 3 last kb landed | 4 tfull committed |
-    #                         5 epilogue saw tfull | 6 team done (cells, h stored) | 7 release done
-    raw = np.zeros((T * 4, 8), dtype=np.uint64)
-    abi.check(h.lib.lrcn_get_trace(h._h, raw.ctypes.data_as(abi._p(abi.C.c_uint64)), raw.size))
-    tr = raw.astype(np.int64).reshape(T, 4, 8)
-    if os.environ.get("LRCN_TRACE_BWD"):
-        print("BACKWARD kernel. ns relative to chain 0's barrier-open of the step; per chain: open, tma_issued, kb0, kbLast, tfull_commit, epi_start, sent, received")
-        for t in range(T - 2, -1, -1):
-            base = tr[t, 0, 0]
-            for c in range(2):
-                print(f"t={t:2d} c={c}", [int(x - base) if x else -1 for x in tr[t, c]])
-            if t > 0:
-                print("      next step's chain-0 barrier opens at", int(tr[t - 1, 0, 0] - base))
-        h.close()
-        sys.exit(0)
-    print("ns relative to chain 0's barrier-open of the step; per chain: open, tma_issued, kb0, kbLast, tfull_commit, epi_start, team_done, released")
-    for t in range(1, T):
+# seq4: [T][4 chains][8]: 0 barrier open (producer) | 1 chunk's TMAs issued | 2 kb0 landed (issuer) | 3 last kb landed | 4 tfull committed |
+#                         5 epilogue saw tfull | 6 team done (cells, h stored) | 7 release done
+tr = h.get_trace(T).astype(np.int64)
+if os.environ.get("LRCN_TRACE_BWD"):
+    print("BACKWARD kernel. ns relative to chain 0's barrier-open of the step; per chain: open, tma_issued, kb0, kbLast, tfull_commit, epi_start, sent, received")
+    for t in range(T - 2, -1, -1):
         base = tr[t, 0, 0]
-        for c in range(4):
+        for c in range(2):
             print(f"t={t:2d} c={c}", [int(x - base) if x else -1 for x in tr[t, c]])
-        if t + 1 < T:
-            print("      next step's chain-0 barrier opens at", int(tr[t + 1, 0, 0] - base))
+        if t > 0:
+            print("      next step's chain-0 barrier opens at", int(tr[t - 1, 0, 0] - base))
+    h.close()
+    sys.exit(0)
+print("ns relative to chain 0's barrier-open of the step; per chain: open, tma_issued, kb0, kbLast, tfull_commit, epi_start, team_done, released")
+for t in range(1, T):
+    base = tr[t, 0, 0]
+    for c in range(4):
+        print(f"t={t:2d} c={c}", [int(x - base) if x else -1 for x in tr[t, c]])
+    if t + 1 < T:
+        print("      next step's chain-0 barrier opens at", int(tr[t + 1, 0, 0] - base))
 h.close()
