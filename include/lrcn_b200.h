@@ -42,7 +42,8 @@ extern "C" {
 
 /* 2: lrcn_config gained n_gpus / device_ids (single-process multi-GPU group); sticky errors; lrcn_checkpoint_save / _load;
  *    lrcn_train_epoch / lrcn_loss_epoch (epoch-level calls, batches staged on the device: additive, same version);
- *    lrcn_set_cnn_param / lrcn_get_cnn_param / lrcn_extract_features (VGG-16 fc7 producer: additive, same version) */
+ *    lrcn_set_cnn_param / lrcn_get_cnn_param / lrcn_extract_features (VGG-16 fc7 producer: additive, same version);
+ *    lrcn_set_gclip / lrcn_grad_norms (per-tensor gradient clipping: additive, same version) */
 #define LRCN_ABI_VERSION 2
 #define LRCN_F_CNN 4096 /* lrcn.jl:28  const cnnout = 4096 */
 #define LRCN_NUM_PARAMS 9
@@ -65,7 +66,8 @@ typedef struct lrcn_handle lrcn_handle;
 
 /* Hot-path configuration.  Defaults mirror the reference: lrcn.jl:39-40 (--hidden 1000 1000,
  * --embed 1000), lrcn.jl:402 Adam() (lr 1e-3, b1 .9, b2 .999, eps 1e-8; --lr/--gclip are ignored
- * by the reference, lrcn.jl:330,386-393), lrcn.jl:353 (captions longer than 28 are skipped). */
+ * by the reference, lrcn.jl:330,386-393), lrcn.jl:353 (captions longer than 28 are skipped).
+ * Gradient clipping (Knet's Adam(gclip=...)) is off by default, like the reference; lrcn_set_gclip turns it on. */
 typedef struct {
   int32_t embed;        /* E  */
   int32_t hidden1;      /* H1 */
@@ -126,6 +128,18 @@ LRCN_API int lrcn_grad(lrcn_handle* h, int split, const int64_t* image_ids, cons
 LRCN_API int lrcn_adam_update(lrcn_handle* h);
 LRCN_API int lrcn_train_step(lrcn_handle* h, int split, const int64_t* image_ids, const int64_t* tokens, int l, int B,
                     float pdrop, uint64_t seed, double* loss_out);
+/* ---- gradient clipping: Knet's Adam(gclip=...) (the natural home of lrcn.jl:44-45 --gclip; the reference ignores the flag).
+ * Per parameter tensor, like Knet's update!(w, g, ::Adam) -> gclip!(g, gclip): tensor k's gradient is scaled by
+ * (float)(gclip / |g_k|) when |g_k| > gclip (|g_k| accumulated in fp64), and is used unchanged otherwise -- NOT one global norm over
+ * the nine tensors.  The held gradient is not modified: lrcn_get_grad still returns the unclipped one.
+ * lrcn_set_gclip: 0 = off = the reference (default).  Applies to every later lrcn_train_step / lrcn_train_step_staged /
+ * lrcn_train_epoch / lrcn_adam_update.  LRCN_ERR_ARG: gclip < 0, NaN or inf (the previous value stays).  LRCN_ERR_STATE: gclip > 0 on
+ * a handle with more than one GPU (group handle, p2p or NCCL ranks); an update call on a handle whose ranks were joined after a
+ * gclip > 0 was set fails with LRCN_ERR_STATE before anything is launched.
+ * lrcn_grad_norms: L2 norm of each of the 9 gradients currently held (last lrcn_grad / train step), model order, computed on the
+ * device by the same reduction the clip uses.  LRCN_ERR_STATE before any gradient exists, or on a multi-GPU handle. */
+LRCN_API int lrcn_set_gclip(lrcn_handle* h, double gclip);
+LRCN_API int lrcn_grad_norms(lrcn_handle* h, double norms_out[9]);
 /* ---- one epoch of the train1 hot loop in ONE call (lrcn.jl:336-396; SURVEY 8 row f-1: batch staging on the device).
  * sequence: the [n_rows][B] time-major token matrix minibatch() builds (lrcn.jl:257-297: batch b owns lengths[b] consecutive
  * rows), input_ids: [n_batches][B], lengths: [n_batches], order: the host's shuffled batch order (lrcn.jl:351; NULL = 0..n-1).

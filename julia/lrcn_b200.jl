@@ -42,7 +42,8 @@ end
 # gpus: vector of CUDA ordinals.  One entry = one GPU.  Several = single-process data parallelism: lrcn.jl stays ONE
 # process with ONE net; train_step!/loss take the GLOBAL batch (batchsize = global rows) and the library shards the rows,
 # exchanges gradients over NVLink peer memory and shards beam search by image -- no launcher, no MPI.
-function create(embed, hidden, vocab_size, batchsize; max_len=28, max_gen_rows=1024, gpus=[0], precision=1)
+# gclip: Knet Adam(gclip=...) per parameter tensor (set_gclip!); 0 = off, which is what the reference trains with.
+function create(embed, hidden, vocab_size, batchsize; max_len=28, max_gen_rows=1024, gpus=[0], precision=1, gclip=0.0)
     c = default_config()
     c.embed = embed; c.hidden1 = hidden[1]; c.hidden2 = hidden[2]; c.vocab = vocab_size
     c.max_batch = batchsize; c.max_len = max_len; c.max_gen_rows = max_gen_rows
@@ -53,6 +54,7 @@ function create(embed, hidden, vocab_size, batchsize; max_len=28, max_gen_rows=1
     check(ccall((:lrcn_create, lib), Cint, (Ptr{Config}, Ptr{Ptr{Void}}), Ref(c), h))
     net = Net(h[], vocab_size)
     finalizer(net, n -> ccall((:lrcn_destroy, lib), Cint, (Ptr{Void},), n.handle))
+    gclip > 0 && set_gclip!(net, gclip)
     return net
 end
 
@@ -137,6 +139,14 @@ function lossgradient(net, split, ids, sequence, range; pdrop=0.0, seed=0)   # l
 end
 
 update!(net) = check(ccall((:lrcn_adam_update, lib), Cint, (Ptr{Void},), net.handle))   # lrcn.jl:394
+
+# Adam(gclip=o[:gclip]) (lrcn.jl:44-45,402): each of the 9 gradients is scaled to norm g when its norm exceeds g; 0 = off.
+# One GPU only.  grad_norms: the 9 norms of the gradients currently held, computed on the device.
+set_gclip!(net, g) = check(ccall((:lrcn_set_gclip, lib), Cint, (Ptr{Void}, Float64), net.handle, g))
+function grad_norms(net)
+    n = zeros(Float64, 9)
+    check(ccall((:lrcn_grad_norms, lib), Cint, (Ptr{Void}, Ptr{Float64}), net.handle, n)); return n
+end
 
 function train_step!(net, split, ids, sequence, range; pdrop=0.0, seed=0)   # lrcn.jl:378 + :394 fused
     tok = tokmat(sequence, range); l = Ref{Float64}(0)

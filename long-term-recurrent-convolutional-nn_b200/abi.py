@@ -72,6 +72,8 @@ SIGNATURES = {
     "lrcn_grad": (C.c_int, [_H, C.c_int, _i64p, _i64p, C.c_int, C.c_int, C.c_float, C.c_uint64, _f64p]),
     "lrcn_adam_update": (C.c_int, [_H]),
     "lrcn_train_step": (C.c_int, [_H, C.c_int, _i64p, _i64p, C.c_int, C.c_int, C.c_float, C.c_uint64, _f64p]),
+    "lrcn_set_gclip": (C.c_int, [_H, C.c_double]),
+    "lrcn_grad_norms": (C.c_int, [_H, _f64p]),
     "lrcn_train_epoch": (C.c_int, [_H, C.c_int, _i64p, C.c_int64, _i64p, _i64p, C.c_int64, C.c_int, _i64p, C.c_int64, C.c_float, C.c_uint64,
                                    _f64p, _i64p]),
     "lrcn_loss_epoch": (C.c_int, [_H, C.c_int, _i64p, C.c_int64, _i64p, _i64p, C.c_int64, C.c_int, _f64p, _i64p]),
@@ -332,6 +334,16 @@ class Handle:
 
     def adam_update(self):
         check(self.lib.lrcn_adam_update(self._h))
+
+    def set_gclip(self, gclip):
+        """Knet Adam(gclip=...) per parameter tensor for every later update; 0 = off (the reference)."""
+        check(self.lib.lrcn_set_gclip(self._h, float(gclip)))
+
+    def grad_norms(self):
+        """L2 norms of the 9 gradients currently held, model order (computed on the device)."""
+        out = np.zeros(9, dtype=np.float64)
+        check(self.lib.lrcn_grad_norms(self._h, out.ctypes.data_as(_f64p)))
+        return out
 
     def token_logps(self, l, B):
         out = np.empty((l + 1, B), dtype=np.float32)

@@ -23,6 +23,7 @@ struct StepScalars {
   float one_m_beta2;
   uint32_t xchg_epoch;  // data-parallel train steps run so far + 1 (same on every rank): the value of the fused exchange's chunk flags
   uint32_t pad_;
+  double gclip;         // Knet Adam(gclip=...) per parameter tensor; 0 = off (lrcn_set_gclip)
 };
 
 // ---- programmatic dependent launch (PDL).  A kernel launched through launch_pdl may be scheduled while its predecessor in
@@ -117,11 +118,34 @@ void dz_finish(cudaStream_t s, float* dZ, float* dv, int ldv, int T, int B, int 
 // dWembT[tok[r]][:] += dE[r][:] (* dropout mask site 0)
 void scatter_add_embed(cudaStream_t s, float* dWembT, const int* tok, const float* dE, int R, int E,
                        const StepScalars* sc, bool train);
-// fused dense Adam over one flat range (Knet defaults, lrcn.jl:394,402); optionally refreshes bf16 hi/lo shadows
+// ---- per-tensor gradient clipping (Knet update!(w, g, ::Adam) -> gclip!(g, gclip)).  A range of whole parameter tensors of the
+// arena; tensor j starts at float4 index off4[j] (tensor offsets are 64-element aligned, so no float4 straddles two tensors).
+constexpr int GNORM_CHUNK4 = 4096;  // 16 Ki floats: one fp64 partial sum each, never straddling tensors
+struct TensorRange {
+  int n;                   // tensors in the range (<= 9)
+  int k[9];                // 0-based model index of each (indexes norm[] / scale[])
+  size_t off4[9];          // start, float4 units, relative to the pointer the kernel is given
+  size_t nel[9];           // elements (the tail of the last float4 beyond nel is ignored)
+  int chunk0[9];           // first partial-sum slot of each: a tensor's slots are the same whichever launch covers it
+};
+// norm[k] = sqrt(sum g^2) in fp64 and scale[k] = (gclip > 0 && norm > gclip) ? (float)(gclip / norm) : 1 for every tensor of the
+// range.  The result depends neither on the grid nor on which other tensors the launch covers.  ticket: zero on entry, reset
+// by the kernel (graph replay).
+void grad_sqnorm(cudaStream_t s, const float* g, const TensorRange& r, double* part, double* norm, float* scale, unsigned int* ticket,
+                 const StepScalars* sc, int grid_cap);
+// Adam's view of the clip: the range's tensors as end offsets (float4 units, relative to the range start) and their scales
+struct ClipMap {
+  const float* scale;      // [9], model order (written by grad_sqnorm)
+  size_t end4[9];
+  int k[9];
+  int n;
+};
+// fused dense Adam over one flat range (Knet defaults, lrcn.jl:394,402); optionally refreshes bf16 hi/lo shadows.
+// clip != null: g is multiplied by its tensor's scale before the moments (g itself is not written)
 void adam_flat(cudaStream_t s, float* w, const float* g, float* m, float* v, size_t n, const StepScalars* sc,
-               __nv_bfloat16* w_hi, __nv_bfloat16* w_lo);
+               __nv_bfloat16* w_hi, __nv_bfloat16* w_lo, const ClipMap* clip = nullptr);
 void adam_range(cudaStream_t s, float* w, const float* g, float* m, float* v, size_t n, const StepScalars* sc, __nv_bfloat16* w_hi,
-                __nv_bfloat16* w_lo, int grid);
+                __nv_bfloat16* w_lo, int grid, const ClipMap* clip = nullptr);
 void split_bf16(cudaStream_t s, const float* x, size_t n, __nv_bfloat16* hi, __nv_bfloat16* lo);
 // ---- batch staging on the device (SURVEY 8 row f-1; lrcn.jl:351-376): the epoch's token matrix and image ids are resident
 // image id -> feature-table row for a whole epoch: ids [n] (1-based wire ids), sorted_ids/rowof [n_tab]; unknown ids raise *err

@@ -758,16 +758,25 @@ void scatter_add_embed(cudaStream_t s, float* dWembT, const int* tok, const floa
 // ------------------------------------------------------------------------------------------
 // fused Adam over the flat parameter arena (Knet Adam defaults; dense over every element)
 // ------------------------------------------------------------------------------------------
-template <bool SPLIT>
+// CLIP: g is scaled by its tensor's clip factor (grad_sqnorm) first -- one fp32 multiply, exact when the factor is 1.  The clip
+// map is the LAST parameter so that the CLIP = false instantiation compiles to the kernel without it.
+template <bool SPLIT, bool CLIP>
 __global__ void __launch_bounds__(256) adam_kernel(float4* __restrict__ w, const float4* __restrict__ g, float4* __restrict__ m,
                                                    float4* __restrict__ v, size_t n4, const StepScalars* __restrict__ sc,
-                                                   __nv_bfloat16* __restrict__ w_hi, __nv_bfloat16* __restrict__ w_lo) {
+                                                   __nv_bfloat16* __restrict__ w_hi, __nv_bfloat16* __restrict__ w_lo, ClipMap cm) {
   pdl_wait();  // PDL: launched while the previous kernel drains (kernels.cuh)
   pdl_trigger();
   const float b1 = sc->beta1, b2 = sc->beta2, lr = sc->lr, eps = sc->eps, d1 = sc->adam_d1, d2 = sc->adam_d2;
   const float ob1 = sc->one_m_beta1, ob2 = sc->one_m_beta2;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
     float4 W = w[i], G = __ldg(g + i), Mv = m[i], Vv = v[i];
+    if (CLIP) {
+      int k = cm.k[0];  // the tensor holding float4 i (constant indices: the map stays in the parameter bank)
+#pragma unroll
+      for (int t = 0; t < 8; t++) if (t + 1 < cm.n && i >= cm.end4[t]) k = cm.k[t + 1];
+      const float s = __ldg(cm.scale + k);
+      G.x = __fmul_rn(G.x, s); G.y = __fmul_rn(G.y, s); G.z = __fmul_rn(G.z, s); G.w = __fmul_rn(G.w, s);
+    }
     float* wp = reinterpret_cast<float*>(&W);
     const float* gp = reinterpret_cast<const float*>(&G);
     float* mp = reinterpret_cast<float*>(&Mv);
@@ -793,22 +802,108 @@ __global__ void __launch_bounds__(256) adam_kernel(float4* __restrict__ w, const
   }
 }
 void adam_flat(cudaStream_t s, float* w, const float* g, float* m, float* v, size_t n, const StepScalars* sc,
-               __nv_bfloat16* w_hi, __nv_bfloat16* w_lo) {
+               __nv_bfloat16* w_hi, __nv_bfloat16* w_lo, const ClipMap* clip) {
   size_t n4 = n / 4;  // arena sizes are padded to multiples of 4
   int grid = 148 * 8;
-  if (w_hi) launch_pdl<2>(adam_kernel<true>, dim3(grid), dim3(256), 0, s, (float4*)w, (const float4*)g, (float4*)m, (float4*)v, n4, sc, w_hi, w_lo);
-  else launch_pdl<2>(adam_kernel<false>, dim3(grid), dim3(256), 0, s, (float4*)w, (const float4*)g, (float4*)m, (float4*)v, n4, sc, (__nv_bfloat16*)nullptr, (__nv_bfloat16*)nullptr);
+  const ClipMap cm = clip ? *clip : ClipMap{};
+#define LRCN_ADAM(SPLIT, CLIP) launch_pdl<2>(adam_kernel<SPLIT, CLIP>, dim3(grid), dim3(256), 0, s, (float4*)w, (const float4*)g, (float4*)m, \
+                                             (float4*)v, n4, sc, SPLIT ? w_hi : (__nv_bfloat16*)nullptr, SPLIT ? w_lo : (__nv_bfloat16*)nullptr, cm)
+  if (w_hi) { if (clip) LRCN_ADAM(true, true); else LRCN_ADAM(true, false); }
+  else { if (clip) LRCN_ADAM(false, true); else LRCN_ADAM(false, false); }
+#undef LRCN_ADAM
   count_launch();
 }
 
 // Adam on an arena range with a bounded grid and no PDL attribute: a bucket of the step's update, launched on a side stream under
 // the rest of the backward pass (lrcn_api.cu)
 void adam_range(cudaStream_t s, float* w, const float* g, float* m, float* v, size_t n, const StepScalars* sc, __nv_bfloat16* w_hi,
-                __nv_bfloat16* w_lo, int grid) {
+                __nv_bfloat16* w_lo, int grid, const ClipMap* clip) {
   const size_t n4 = n / 4;
   if (n4 == 0) return;
-  if (w_hi) adam_kernel<true><<<grid, 256, 0, s>>>((float4*)w, (const float4*)g, (float4*)m, (float4*)v, n4, sc, w_hi, w_lo);
-  else adam_kernel<false><<<grid, 256, 0, s>>>((float4*)w, (const float4*)g, (float4*)m, (float4*)v, n4, sc, (__nv_bfloat16*)nullptr, (__nv_bfloat16*)nullptr);
+  const ClipMap cm = clip ? *clip : ClipMap{};
+#define LRCN_ADAM(SPLIT, CLIP) adam_kernel<SPLIT, CLIP><<<grid, 256, 0, s>>>((float4*)w, (const float4*)g, (float4*)m, (float4*)v, n4, sc, \
+                                                                            SPLIT ? w_hi : (__nv_bfloat16*)nullptr, SPLIT ? w_lo : (__nv_bfloat16*)nullptr, cm)
+  if (w_hi) { if (clip) LRCN_ADAM(true, true); else LRCN_ADAM(true, false); }
+  else { if (clip) LRCN_ADAM(false, true); else LRCN_ADAM(false, false); }
+#undef LRCN_ADAM
+  count_launch();
+}
+
+// ------------------------------------------------------------------------------------------
+// per-tensor gradient norms for Knet's gclip (kernels.cuh: grad_sqnorm).  CTAs walk the range's 16 Ki-float chunks; a chunk's
+// partial sum of squares (fp64) is reduced in a fixed order by whichever CTA takes it, and the last CTA (atomic ticket) sums each
+// tensor's partials in a fixed order: the norms are bit-identical for any grid and any grouping of tensors into launches.
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ int gnorm_chunks(size_t nel) { return (int)(((nel + 3) / 4 + GNORM_CHUNK4 - 1) / GNORM_CHUNK4); }
+
+__global__ void __launch_bounds__(256) grad_sqnorm_kernel(const float4* __restrict__ g, TensorRange r, double* __restrict__ part,
+                                                          double* __restrict__ norm, float* __restrict__ scale,
+                                                          unsigned int* __restrict__ ticket, const StepScalars* __restrict__ sc, int total) {
+  __shared__ double red[8];
+  __shared__ bool last;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int c = blockIdx.x; c < total; c += gridDim.x) {
+    int j = 0, q = c;
+    while (q >= gnorm_chunks(r.nel[j])) { q -= gnorm_chunks(r.nel[j]); j++; }
+    const size_t nel = r.nel[j], n4 = (nel + 3) / 4, b = (size_t)q * GNORM_CHUNK4;
+    const size_t e = b + GNORM_CHUNK4 < n4 ? b + GNORM_CHUNK4 : n4;
+    const float4* p = g + r.off4[j];
+    // all 16 loads of a thread in flight at once; then the sum in chunk order (a float4 past the chunk's end adds +0: exact)
+    constexpr int PER = GNORM_CHUNK4 / 256;
+    float4 x[PER];
+#pragma unroll
+    for (int u = 0; u < PER; u++) {
+      const size_t i = b + threadIdx.x + 256 * u;
+      x[u] = i < e ? __ldg(p + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+      if (i < e && 4 * i + 4 > nel) {  // the tensor's last float4: ignore the padding
+        if (4 * i + 1 >= nel) x[u].y = 0.f;
+        if (4 * i + 2 >= nel) x[u].z = 0.f;
+        if (4 * i + 3 >= nel) x[u].w = 0.f;
+      }
+    }
+    double acc = 0.0;
+#pragma unroll
+    for (int u = 0; u < PER; u++) {
+      acc += (double)x[u].x * x[u].x; acc += (double)x[u].y * x[u].y; acc += (double)x[u].z * x[u].z; acc += (double)x[u].w * x[u].w;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) red[warp] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double s = 0.0;
+#pragma unroll
+      for (int k = 0; k < 8; k++) s += red[k];
+      part[r.chunk0[j] + q] = s;
+    }
+    __syncthreads();
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  for (int j = warp; j < r.n; j += 8) {  // one warp per tensor: lane-strided partials, then a fixed butterfly
+    const int nch = gnorm_chunks(r.nel[j]);
+    double s = 0.0;
+    for (int q = lane; q < nch; q += 32) s += __ldcg(part + r.chunk0[j] + q);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) {
+      const double nrm = sqrt(s), gclip = sc->gclip;
+      norm[r.k[j]] = nrm;
+      scale[r.k[j]] = gclip > 0.0 && nrm > gclip ? (float)(gclip / nrm) : 1.0f;
+    }
+  }
+  if (threadIdx.x == 0) *ticket = 0u;  // ready for the next launch (graph replay)
+}
+void grad_sqnorm(cudaStream_t s, const float* g, const TensorRange& r, double* part, double* norm, float* scale, unsigned int* ticket,
+                 const StepScalars* sc, int grid_cap) {
+  int total = 0;
+  for (int j = 0; j < r.n; j++) total += (int)(((r.nel[j] + 3) / 4 + GNORM_CHUNK4 - 1) / GNORM_CHUNK4);
+  const int grid = total < grid_cap ? total : grid_cap;
+  grad_sqnorm_kernel<<<grid, 256, 0, s>>>((const float4*)g, r, part, norm, scale, ticket, sc, total);
   count_launch();
 }
 

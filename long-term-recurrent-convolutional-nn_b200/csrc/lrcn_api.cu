@@ -165,7 +165,7 @@ static int s_destroy(lrcn_handle* h) {
   for (cudaEvent_t e : h->sc_ev) if (e) cudaEventDestroy(e);
   void* ptrs[] = {h->w, h->g, h->m, h->v, h->w_hi, h->w_lo, h->wp1_hi, h->wp1_lo, h->wp2_hi, h->wp2_lo, h->wt1_hi, h->wt1_lo, h->wt2_hi, h->wt2_lo, h->tab[0].d, h->tab[1].d, h->ws.f, h->ws.hi, h->ws.lo, h->d_tok_in,
                   h->d_tok_tgt, h->d_rows, h->d_sc, h->p2p_ctl, h->d_loss_total, h->d_epoch, h->d_epoch_side, h->stage, h->d_counters, h->d_trace, h->g_last, h->g_ctok, h->g_stok, h->g_spar, h->g_hista, h->g_histb,
-                  h->g_done, h->g_ndone, h->g_olen, h->g_rows, h->g_otok, h->l2_scratch, h->g_keep, h->g_omap, h->g_omap_s};
+                  h->g_done, h->g_ndone, h->g_olen, h->g_rows, h->g_otok, h->l2_scratch, h->g_keep, h->g_omap, h->g_omap_s, h->d_gnorm};
   for (void* p : ptrs) if (p) cudaFree(p);
   for (void* q : {(void*)h->ep_seq, (void*)h->ep_ids, (void*)h->ep_rows, (void*)h->ep_loss, (void*)h->ep_err, (void*)h->tab[0].d_ids, (void*)h->tab[0].d_rowof,
                   (void*)h->tab[1].d_ids, (void*)h->tab[1].d_rowof})
@@ -249,6 +249,14 @@ static int create_impl(const lrcn_config* cfg, lrcn_handle* h) {
   h->P = pos;
   CK(cudaMalloc(&h->w, h->P * 4)); CK(cudaMalloc(&h->g, h->P * 4)); CK(cudaMalloc(&h->m, h->P * 4)); CK(cudaMalloc(&h->v, h->P * 4));
   CK(cudaMemset(h->w, 0, h->P * 4)); CK(cudaMemset(h->g, 0, h->P * 4)); CK(cudaMemset(h->m, 0, h->P * 4)); CK(cudaMemset(h->v, 0, h->P * 4));
+  {  // gradient-norm state: norm[9] @0, scale[9] @128, tickets[8] @192, chunk partials @256
+    int chunks = 0;
+    for (int k = 0; k < 9; k++) { h->gchunk0[k] = chunks; chunks += (int)(((h->nel[k] + 3) / 4 + GNORM_CHUNK4 - 1) / GNORM_CHUNK4); }
+    char* base = nullptr;
+    CK(cudaMalloc(&base, 256 + (size_t)chunks * 8));
+    CK(cudaMemset(base, 0, 256 + (size_t)chunks * 8));
+    h->d_gnorm = (double*)base; h->d_gscale = (float*)(base + 128); h->d_gticket = (unsigned int*)(base + 192); h->d_gpart = (double*)(base + 256);
+  }
   if (h->bf16mode) {
     CK(cudaMalloc(&h->w_hi, h->P * 2)); CK(cudaMalloc(&h->w_lo, h->P * 2));
     CK(cudaMemset(h->w_hi, 0, h->P * 2)); CK(cudaMemset(h->w_lo, 0, h->P * 2));
@@ -770,8 +778,36 @@ static void enqueue_backward_seg(lrcn_handle* h, int B, int l, bool train, int s
   }
 }
 
-static void enqueue_adam(lrcn_handle* h) {
-  adam_flat(h->stream, h->w, h->g, h->m, h->v, h->P, h->d_sc, h->w_hi, h->w_lo);
+// Norms (and clip factors) of the whole tensors in the arena range [b0, e0), on stream st; returns Adam's map of the range.
+// ticket: 0..3 for the launch of gradient bucket k (they may run concurrently), 4 for whole-arena launches.
+static ClipMap enqueue_grad_norms(lrcn_handle* h, cudaStream_t st, size_t b0, size_t e0, int ticket, int grid_cap) {
+  static const int order[9] = {8, 9, 3, 4, 5, 6, 1, 2, 7};  // arena order (create_impl)
+  TensorRange r{};
+  ClipMap cm{};
+  cm.scale = h->d_gscale;
+  for (int i = 0; i < 9; i++) {
+    const int k = order[i] - 1;
+    if (h->off[k] < b0 || h->off[k] >= e0) continue;
+    r.k[r.n] = k; r.off4[r.n] = (h->off[k] - b0) / 4; r.nel[r.n] = h->nel[k]; r.chunk0[r.n] = h->gchunk0[k];
+    cm.k[cm.n] = k; cm.end4[cm.n] = (h->off[k] - b0 + (h->nel[k] + 63) / 64 * 64) / 4;
+    r.n++; cm.n++;
+  }
+  grad_sqnorm(st, h->g + b0, r, h->d_gpart, h->d_gnorm, h->d_gscale, h->d_gticket + ticket, h->d_sc, grid_cap);
+  return cm;
+}
+
+static void enqueue_adam(lrcn_handle* h, bool clip) {
+  if (!clip) { adam_flat(h->stream, h->w, h->g, h->m, h->v, h->P, h->d_sc, h->w_hi, h->w_lo); return; }
+  const ClipMap cm = enqueue_grad_norms(h, h->stream, 0, h->P, 4, 148 * 8);
+  adam_flat(h->stream, h->w, h->g, h->m, h->v, h->P, h->d_sc, h->w_hi, h->w_lo, &cm);
+}
+
+// Per-tensor clipping is single-GPU only: the data-parallel exchanges run Adam on each chunk of the reduced gradient as soon as
+// it arrives, before any tensor's norm could be known
+static int gclip_check(const lrcn_handle* h) {
+  if (h->gclip > 0.0 && h->nranks > 1)
+    return fail(LRCN_ERR_STATE, "gradient clipping (lrcn_set_gclip) is not supported with data parallelism (%d ranks)", h->nranks);
+  return LRCN_OK;
 }
 
 // run `fn` directly or as a cached CUDA graph keyed by (kind, B, l, flags)
@@ -832,6 +868,7 @@ static int push_scalars(lrcn_handle* h, int B, int l, float pdrop, uint64_t seed
   sc->lr = (float)h->cfg.lr; sc->beta1 = (float)h->cfg.beta1; sc->beta2 = (float)h->cfg.beta2; sc->eps = (float)h->cfg.eps;
   sc->one_m_beta1 = (float)(1.0 - h->cfg.beta1);
   sc->one_m_beta2 = (float)(1.0 - h->cfg.beta2);
+  sc->gclip = h->gclip;
   CK(cudaMemcpyAsync(h->d_sc, sc, sizeof(StepScalars), cudaMemcpyHostToDevice, h->stream));
   CK(cudaEventRecord(h->sc_ev[slot], h->stream));
   h->sc_busy[slot] = true;
@@ -851,7 +888,10 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
   const bool drop = train && pdrop > 0.f;
   { int rc0 = push_scalars(h, B, l, train ? pdrop : 0.f, seed, mode == 2); if (rc0) return rc0; }
   h->last_B = B; h->last_l = l;
-  const int fl = (split << 1) | (drop ? 1 : 0);
+  if (train) h->have_grad = true;
+  // the norm launches are in the step's graph only while clipping is on; gclip itself travels in the step scalars
+  const bool clip = mode == 2 && h->gclip > 0.0;
+  const int fl = (split << 1) | (drop ? 1 : 0) | (clip ? 4 : 0);
   int rc;
   h->loss_is_total = false;
   if (mode == 0) {
@@ -870,7 +910,10 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
     return run_cached(h, std::make_tuple(25, B, l, fl), [&] {
       auto adam_bucket = [&](int k, cudaStream_t st, int grid) {
         const size_t b0 = h->bucket_off[k], n = h->bucket_off[k + 1] - b0;
-        adam_range(st, h->w + b0, h->g + b0, h->m + b0, h->v + b0, n, h->d_sc, h->w_hi + b0, h->w_lo + b0, grid);
+        if (!clip) { adam_range(st, h->w + b0, h->g + b0, h->m + b0, h->v + b0, n, h->d_sc, h->w_hi + b0, h->w_lo + b0, grid); return; }
+        // a bucket holds whole tensors: their norms are complete here, on the bucket's own stream
+        const ClipMap cm = enqueue_grad_norms(h, st, b0, b0 + n, k, grid);
+        adam_range(st, h->w + b0, h->g + b0, h->m + b0, h->v + b0, n, h->d_sc, h->w_hi + b0, h->w_lo + b0, grid, &cm);
       };
       enqueue_forward(h, split, B, l, true);
       enqueue_backward_seg(h, B, l, true, 1);
@@ -895,7 +938,7 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
     return run_cached(h, std::make_tuple(mode == 2 ? 2 : 1, B, l, fl), [&] {
       enqueue_forward(h, split, B, l, true);
       for (int seg = 1; seg <= 3; seg++) enqueue_backward_seg(h, B, l, true, seg);
-      if (mode == 2) enqueue_adam(h);
+      if (mode == 2) enqueue_adam(h, clip);
     });
   }
   static const bool force_nccl = getenv("LRCN_DP_NCCL") != nullptr;
@@ -1093,7 +1136,7 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
         if (h->bf16mode) split_bf16(h->stream, h->w, h->P, h->w_hi, h->w_lo);
       } else {
         dp_p2p_allreduce(h->stream, h->peers, h->P, h->d_epoch, h->d_loss_total);
-        if (mode == 2) enqueue_adam(h);
+        if (mode == 2) enqueue_adam(h, false);
       }
     });
   }
@@ -1113,7 +1156,7 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
     rc = nccl_check(n->AllReduce(h->d_loss, h->d_loss, 1, NCCL_FLOAT64, NCCL_SUM, h->comm, h->stream), "ncclAllReduce(loss)"); if (rc) return rc;
     rc = nccl_check(n->GroupEnd(), "ncclGroupEnd"); if (rc) return rc;
     if (mode == 2) {
-      rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h); });
+      rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h, false); });
       if (rc) return rc;
     }
     return LRCN_OK;
@@ -1143,7 +1186,7 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
   CK(cudaEventRecord(h->ev_comm, h->comm_stream));
   CK(cudaStreamWaitEvent(h->stream, h->ev_comm, 0));
   if (mode == 2) {
-    rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h); });
+    rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h, false); });
     if (rc) return rc;
   }
   return LRCN_OK;
@@ -1201,7 +1244,9 @@ static int s_grad(lrcn_handle* h, int split, const int64_t* image_ids, const int
 static int s_train_step(lrcn_handle* h, int split, const int64_t* image_ids, const int64_t* tokens, int l, int B, float pdrop,
                                uint64_t seed, double* loss_out) {
   if (pdrop < 0.f || pdrop >= 1.f) return fail(LRCN_ERR_ARG, "pdrop must be in [0,1)");
-  int rc = stage_current(h, split, image_ids, tokens, l, B);
+  int rc = gclip_check(h);
+  if (rc) return rc;
+  rc = stage_current(h, split, image_ids, tokens, l, B);
   if (rc) return rc;
   rc = run_step(h, split, B, l, pdrop, seed, 2);
   if (rc) return rc;
@@ -1219,9 +1264,10 @@ static int s_adam_update(lrcn_handle* h) {
   if (h->nranks > 1 && h->adam_sharded)
     return fail(LRCN_ERR_STATE, "lrcn_adam_update after a sharded data-parallel train step: Adam state is distributed over the ranks; "
                                 "call lrcn_get_adam_state (gathers it) on every rank first, or keep using lrcn_train_step");
+  { int rc0 = gclip_check(h); if (rc0) return rc0; }
   { int rc0 = push_scalars(h, 1, 0, 0.f, 0, true); if (rc0) return rc0; }
   g_counter = &h->counter;
-  enqueue_adam(h);
+  enqueue_adam(h, h->gclip > 0.0);
   return sync_stream(h);
 }
 static int s_get_token_logps(lrcn_handle* h, float* out, int64_t n) {
@@ -1256,6 +1302,7 @@ static int s_stage_batch(lrcn_handle* h, int slot, int split, const int64_t* ima
 static int s_train_step_staged(lrcn_handle* h, int slot, float pdrop, uint64_t seed, double* loss_out) {
   if (!h || slot < 0 || slot >= 64 || !h->slots[slot].tok_in) return fail(LRCN_ERR_ARG, "slot %d not staged", slot);
   if (pdrop < 0.f || pdrop >= 1.f) return fail(LRCN_ERR_ARG, "pdrop must be in [0,1)");
+  { int rc0 = gclip_check(h); if (rc0) return rc0; }
   Slot& s = h->slots[slot];
   const size_t R = (size_t)(s.l + 1) * s.B;
   CK(cudaSetDevice(h->cfg.device));
@@ -1640,7 +1687,7 @@ static int s_time_kernel(lrcn_handle* h, const char* name, int reps, float* avg_
       CK(cudaEventRecord(h->ev0, h->stream));
       if (!strcmp(name, "adam")) {
         // algorithmic traffic: read w,g,m,v + write w,m,v = 28 B/param (+4 B/param of bf16 shadows in bf16x3 mode)
-        enqueue_adam(h);
+        enqueue_adam(h, false);
         bytes = (double)h->P * (h->bf16mode ? 32.0 : 28.0);
       } else if (!strcmp(name, "vocab_gemm")) {
         gemm(h, true, true, R, h->V, h->H2, WS(h, o.h2) + (size_t)B * h->H2, h->H2, Wp(h, 8), h->H2, WS(h, o.logits), h->ldV, false, Wp(h, 9));
@@ -1852,6 +1899,26 @@ extern "C" int lrcn_adam_update(lrcn_handle* h) {
     FOR_ALL(h, s_adam_update(m));
   }
   return s_adam_update(h);
+}
+extern "C" int lrcn_set_gclip(lrcn_handle* h, double gclip) {
+  ENTER(h);
+  if (!(gclip >= 0.0 && gclip < INFINITY)) return fail(LRCN_ERR_ARG, "gclip must be finite and >= 0 (0 = off), got %g", gclip);
+  if (gclip > 0.0 && (is_group(h) || h->nranks > 1))
+    return fail(LRCN_ERR_STATE, "gradient clipping is not supported on a handle with more than one GPU");
+  h->gclip = gclip;  // a group handle only ever holds 0, like its members
+  return LRCN_OK;
+}
+extern "C" int lrcn_grad_norms(lrcn_handle* h, double norms_out[9]) {
+  ENTER(h);
+  if (!norms_out) return fail(LRCN_ERR_ARG, "null");
+  if (is_group(h) || h->nranks > 1) return fail(LRCN_ERR_STATE, "lrcn_grad_norms is not supported on a handle with more than one GPU");
+  if (!h->have_grad) return fail(LRCN_ERR_STATE, "no gradient yet (lrcn_grad, lrcn_train_step, lrcn_train_step_staged or lrcn_train_epoch first)");
+  CK(cudaSetDevice(h->cfg.device));
+  g_counter = &h->counter;
+  enqueue_grad_norms(h, h->stream, 0, h->P, 4, 148 * 8);
+  CK(cudaPeekAtLastError());
+  CK(cudaMemcpyAsync(norms_out, h->d_gnorm, 9 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  return sync_stream(h);
 }
 extern "C" int lrcn_get_token_logps(lrcn_handle* h, float* out, int64_t n) {
   ENTER(h);
@@ -2069,6 +2136,7 @@ static int epoch_run(lrcn_handle* h, int mode, int split, const int64_t* sequenc
   }
   if (start[n_batches] > n_rows) return fail(LRCN_ERR_ARG, "lengths sum to %lld rows, sequence has %lld", (long long)start[n_batches], (long long)n_rows);
   int rc;
+  if (mode == 2) for (lrcn_handle* m : hs) { rc = gclip_check(m); if (rc) return rc; }
   for (lrcn_handle* m : hs) { rc = epoch_upload(m, split, sequence, n_rows, input_ids, n_batches, B); if (rc) return rc; }
   for (lrcn_handle* m : hs) { rc = epoch_check(m); if (rc) return rc; }  // unknown ids fail the call before any step runs (like the per-step call)
   const int64_t n_run_max = n_order > 0 ? n_order : n_batches;

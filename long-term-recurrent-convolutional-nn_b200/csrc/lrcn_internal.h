@@ -60,6 +60,13 @@ struct lrcn_handle {
   bf16 *wp1_hi = nullptr, *wp1_lo = nullptr, *wp2_hi = nullptr, *wp2_lo = nullptr;  // gate-interleaved recurrent weights (lstm_sm100.cu)
   bf16 *wt1_hi = nullptr, *wt1_lo = nullptr, *wt2_hi = nullptr, *wt2_lo = nullptr;  // transposed recurrent weights for the backward step
   int64_t adam_t = 0;
+  // per-tensor gradient clipping (lrcn_set_gclip, kernels.cuh grad_sqnorm): one allocation holding norm[9] (fp64), scale[9],
+  // the launch tickets (one per gradient bucket + one for whole-arena launches) and the chunk partial sums; gchunk0[k]: first
+  // partial slot of tensor k (model order)
+  double gclip = 0.0;
+  bool have_grad = false;   // a gradient has been computed (lrcn_grad_norms)
+  int gchunk0[9] = {};
+  double *d_gnorm = nullptr, *d_gpart = nullptr; float* d_gscale = nullptr; unsigned int* d_gticket = nullptr;
   Table tab[2];
   Arena ws;
   Workspace o;

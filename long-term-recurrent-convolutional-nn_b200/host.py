@@ -28,7 +28,7 @@ class LRCN:
     through train1 / average_loss / generate."""
 
     def __init__(self, hidden, vocab_size, embed, batchsize, max_len=28, precision=abi.PREC_BF16X3, device=0,
-                 max_gen_rows=1024, use_graphs=True):
+                 max_gen_rows=1024, use_graphs=True, gclip=0.0):
         if len(hidden) != 2:
             raise ValueError("lrcn() hard-wires two LSTM layers (lrcn.jl:540-551): --hidden needs exactly 2 sizes")
         self.hidden = [int(hidden[0]), int(hidden[1])]
@@ -37,6 +37,8 @@ class LRCN:
                                  max_batch=self.batchsize, max_len=max_len, max_gen_rows=max_gen_rows, device=device,
                                  precision=precision, use_graphs=1 if use_graphs else 0)
         self.h = abi.Handle(cfg)
+        if gclip:
+            self.h.set_gclip(gclip)  # Knet Adam(gclip=o[:gclip]); the reference ignores --gclip, so 0 keeps its training
         self._step = 0
 
     def close(self):
@@ -131,7 +133,8 @@ class LRCN:
 
     def train1(self, seq, batch_size=None, pdrop=0.0, shuffle_seed=0, split=0, progress=None, per_step=False):
         """One epoch of the hot loop lrcn.jl:351-396: shuffled batch order, skip l>28,
-        gradient + Adam per batch.  `lr`/`gclip` are ignored by the reference and so not taken.
+        gradient + Adam per batch.  Adam clips each gradient tensor to the `gclip` given to the constructor (0, the default, is
+        the reference: it ignores --gclip).
         Default: ONE library call for the epoch (batches staged on the device, no per-step host work; SURVEY 8 row f-1);
         per_step=True or a progress callback drives one lrcn_train_step per batch instead.  Both give the same losses."""
         sequence, input_ids, lengths = seq
