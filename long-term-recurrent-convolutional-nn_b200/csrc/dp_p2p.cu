@@ -1,11 +1,13 @@
 // dp_p2p.cu -- data-parallel gradient exchange over NVLink peer memory, without NCCL kernels.
 //
-// One process per GPU; every rank maps its peers' gradient arenas (CUDA IPC).  Rank r OWNS a contiguous 1/N shard of the
-// arena: it loads that shard from every rank over NVLink (fixed rank order, so the sum is deterministic and identical
-// everywhere), and stores the sum back into every rank's arena in place -- reduce-scatter and all-gather fused in one
-// kernel with owner-computes semantics (nobody else touches an owner's elements, so no staging buffers are needed).
-// Cross-GPU ordering is two flag barriers in peer memory (system-scope release / acquire):
-//   B1  every rank's backward pass is complete  ->  exchange kernel  ->  B2  every rank's stores have landed.
+// One handle per GPU; every rank maps its peers' gradient and weight arenas, control blocks and staging allocations (CUDA IPC,
+// or direct peer pointers in a single-process group).  Rank r OWNS a contiguous 1/N slice of what is exchanged and sums it over
+// all ranks in fixed rank order, so the sum is deterministic and identical everywhere.
+//   training step      one fused_exchange_kernel launch per gradient bucket: every rank pushes its gradient chunks into the
+//                      owners' staging rows, the owner sums them, runs Adam on its slice and pushes the new weights into every
+//                      rank's arena; per-chunk flags and completion counters order it (see the section above the kernel).
+//   gradient-only step flag barrier  ->  allreduce_p2p_kernel: the owner loads its shard of the arena from every rank and stores
+//                      the sum into every rank's arena in place  ->  flag barrier (every rank's stores have landed).
 // Why not NCCL here: its kernels compete for SMs with the persistent tcgen05 GEMM / LSTM kernels (which need their whole
 // grid co-resident), so a "bucketed, overlapped" allreduce ends up serialising; measured in profiles/r01_progress.md.
 #include "kernels.cuh"
@@ -36,19 +38,17 @@ __device__ __forceinline__ float4 ld_peer_f4(const float4* p) {  // peer memory 
   return v;
 }
 
-// one warp: lane q signals rank q and waits for rank q's signal.  flag_base selects one of the independent flag sets of the
-// control block (barriers issued concurrently from two streams must not share flags or epoch counters)
-__global__ void xgpu_barrier_kernel(P2PPeers peers, unsigned int* epoch_ctr, int flag_base, unsigned long long* trace) {
+// one warp: lane q signals rank q and waits for rank q's signal
+__global__ void xgpu_barrier_kernel(P2PPeers peers, unsigned int* epoch_ctr) {
   __shared__ unsigned int epoch;
-  if (trace && threadIdx.x == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); trace[0] = t; }
   if (threadIdx.x == 0) { epoch = *epoch_ctr + 1u; *epoch_ctr = epoch; }
   __syncwarp();
   const unsigned int e = epoch;
   const int q = threadIdx.x;
   __threadfence_system();
   if (q < peers.nranks) {
-    st_release_sys(&peers.ctl[q]->flags[flag_base + peers.rank], e);
-    const unsigned int* mine = &peers.ctl[peers.rank]->flags[flag_base + q];
+    st_release_sys(&peers.ctl[q]->flags[peers.rank], e);
+    const unsigned int* mine = &peers.ctl[peers.rank]->flags[q];
     const long long t0 = clock64();
     while ((int)(ld_acquire_sys(mine) - e) < 0) {
       if (dev_aborted()) break;
@@ -82,186 +82,28 @@ __global__ void __launch_bounds__(256) allreduce_p2p_kernel(P2PPeers peers, size
     }
     *loss_total = t;
   }
-  __threadfence_system();  // my stores into peer memory are performed before this kernel ends (B2 follows)
-}
-
-// reduce-scatter + Adam + all-gather in one kernel: the owner of a shard sums its gradients over all ranks, updates ITS slice of
-// m, v and w exactly like adam_kernel (same operation order: replicas stay bit-identical to the replicated update) and stores
-// the new weights into every rank's arena.  Adam costs 1/N per GPU and the NVLink volume is the same as the allreduce's.
-__global__ void __launch_bounds__(256) adam_p2p_kernel(P2PPeers peers, size_t begin4, size_t end4, float4* __restrict__ m, float4* __restrict__ v,
-                                                       const StepScalars* __restrict__ sc, double* loss_total) {
-  const int N = peers.nranks;
-  const float b1 = sc->beta1, b2 = sc->beta2, lr = sc->lr, eps = sc->eps, d1 = sc->adam_d1, d2 = sc->adam_d2;
-  const float ob1 = sc->one_m_beta1, ob2 = sc->one_m_beta2;
-  const float4* wl = reinterpret_cast<const float4*>(peers.w[peers.rank]);
-  for (size_t i = begin4 + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < end4; i += (size_t)gridDim.x * blockDim.x) {
-    float4 G = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll 8
-    for (int p = 0; p < N; p++) {
-      const float4 x = ld_peer_f4(reinterpret_cast<const float4*>(peers.g[p]) + i);
-      G.x += x.x; G.y += x.y; G.z += x.z; G.w += x.w;
-    }
-    float4 W = wl[i], Mv = m[i], Vv = v[i];
-    float* wp = reinterpret_cast<float*>(&W);
-    const float* gp = reinterpret_cast<const float*>(&G);
-    float* mp = reinterpret_cast<float*>(&Mv);
-    float* vp = reinterpret_cast<float*>(&Vv);
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const float mm = __fadd_rn(__fmul_rn(b1, mp[k]), __fmul_rn(ob1, gp[k]));
-      const float vv = __fadd_rn(__fmul_rn(b2, vp[k]), __fmul_rn(ob2, __fmul_rn(gp[k], gp[k])));
-      const float upd = __fdiv_rn(__fdiv_rn(mm, d1), __fadd_rn(__fsqrt_rn(__fdiv_rn(vv, d2)), eps));
-      wp[k] = __fsub_rn(wp[k], __fmul_rn(lr, upd));
-      mp[k] = mm; vp[k] = vv;
-    }
-    m[i] = Mv; v[i] = Vv;
-    for (int p = 0; p < N; p++) reinterpret_cast<float4*>(peers.w[p])[i] = W;
-    reinterpret_cast<float4*>(peers.g[peers.rank])[i] = G;  // the summed gradient of the owned shard stays readable (lrcn_get_grad)
-  }
-  if (blockIdx.x == 0 && threadIdx.x == 0 && loss_total) {
-    double t = 0.0;
-    for (int p = 0; p < N; p++) {
-      double x;
-      asm volatile("ld.relaxed.sys.global.f64 %0, [%1];" : "=d"(x) : "l"(&peers.ctl[p]->loss_partial) : "memory");
-      t += x;
-    }
-    *loss_total = t;
-  }
-  __threadfence_system();
+  __threadfence_system();  // my stores into peer memory are performed before this kernel ends (the second barrier follows)
 }
 
 bool dp_bind_abort(unsigned int* host_flag) { return dev_abort_bind(host_flag) == cudaSuccess; }
 
-void dp_p2p_shard(size_t n_floats, int nranks, int r, size_t* begin, size_t* end) {
+// [begin, end) of rank r's shard of an arena of n_floats, in floats
+static void dp_p2p_shard(size_t n_floats, int nranks, int r, size_t* begin, size_t* end) {
   const size_t n4 = n_floats / 4, per = (n4 + nranks - 1) / nranks;
   const size_t b = per * r < n4 ? per * r : n4;
   const size_t e = b + per < n4 ? b + per : n4;
   *begin = 4 * b; *end = 4 * e;
 }
 
-void dp_p2p_adam(cudaStream_t s, const P2PPeers& peers, size_t n_floats, unsigned int* epoch_ctr, double* loss_total, float* m, float* v,
-                 const StepScalars* sc) {
-  size_t b, e;
-  dp_p2p_shard(n_floats, peers.nranks, peers.rank, &b, &e);
-  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr, 0, nullptr);
-  adam_p2p_kernel<<<148 * 4, 256, 0, s>>>(peers, b / 4, e / 4, reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v), sc, loss_total);
-  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr, 0, nullptr);
-  if (g_counter) g_counter->n += 3;
-}
-
 void dp_p2p_allreduce(cudaStream_t s, const P2PPeers& peers, size_t n_floats, unsigned int* epoch_ctr, double* loss_total) {
   size_t b, e;  // arena sizes are multiples of 64 floats
   dp_p2p_shard(n_floats, peers.nranks, peers.rank, &b, &e);
-  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr, 0, nullptr);
+  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr);
   allreduce_p2p_kernel<<<148 * 4, 256, 0, s>>>(peers, b / 4, e / 4, loss_total);
-  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr, 0, nullptr);
+  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr);
   if (g_counter) g_counter->n += 3;
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// Copy-engine exchange (default for training).  The NVLink traffic of the gradient reduce-scatter and of the weight
-// all-gather is done by cudaMemcpyAsync nodes (DMA engines, no SMs): every rank PUSHES the slices of a gradient bucket into
-// their owners' staging buffers, a flag barrier says "my pushes have landed", the owner sums the N contributions and runs
-// Adam on its slice with the small local kernel below, and pushes the new weights back.  Because no SM is involved in the
-// transfers, the buckets that are ready early (Wout/bout after the vocab backward; W2, b2, Wf, Wcnn after layer-2 BPTT) are
-// exchanged on a side stream UNDER the persistent LSTM / GEMM kernels of the rest of the backward pass, which the SM-driven
-// exchange (and NCCL's kernels) could not do without stealing SMs from kernels that need their whole grid resident.
-// stage: [nranks][stride4] float4 staging rows on the owner (row q = contribution of rank q; the owner's own row is unused,
-// its contribution is read from g directly).  Same operation order as adam_kernel: replicas stay bit-identical.
-__global__ void __launch_bounds__(256) adam_staged_kernel(float4* __restrict__ w, float4* __restrict__ g, float4* __restrict__ m, float4* __restrict__ v,
-                                                          const float4* __restrict__ stage, size_t stride4, size_t stage_off4, size_t b4, size_t e4, int nranks,
-                                                          int rank, const StepScalars* __restrict__ sc, P2PPeers peers, double* loss_total, int push_w) {
-  const float b1 = sc->beta1, b2 = sc->beta2, lr = sc->lr, eps = sc->eps, d1 = sc->adam_d1, d2 = sc->adam_d2;
-  const float ob1 = sc->one_m_beta1, ob2 = sc->one_m_beta2;
-  for (size_t i = b4 + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < e4; i += (size_t)gridDim.x * blockDim.x) {
-    float4 G = make_float4(0.f, 0.f, 0.f, 0.f);
-    const size_t so = stage_off4 + (i - b4);
-    for (int q = 0; q < nranks; q++) {  // fixed rank order: the sum is deterministic and identical to the SM-driven exchange
-      const float4 x = q == rank ? g[i] : __ldcs(stage + (size_t)q * stride4 + so);
-      G.x += x.x; G.y += x.y; G.z += x.z; G.w += x.w;
-    }
-    float4 W = w[i], Mv = m[i], Vv = v[i];
-    float* wp = reinterpret_cast<float*>(&W);
-    const float* gp = reinterpret_cast<const float*>(&G);
-    float* mp = reinterpret_cast<float*>(&Mv);
-    float* vp = reinterpret_cast<float*>(&Vv);
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const float mm = __fadd_rn(__fmul_rn(b1, mp[k]), __fmul_rn(ob1, gp[k]));
-      const float vv = __fadd_rn(__fmul_rn(b2, vp[k]), __fmul_rn(ob2, __fmul_rn(gp[k], gp[k])));
-      const float upd = __fdiv_rn(__fdiv_rn(mm, d1), __fadd_rn(__fsqrt_rn(__fdiv_rn(vv, d2)), eps));
-      wp[k] = __fsub_rn(wp[k], __fmul_rn(lr, upd));
-      mp[k] = mm; vp[k] = vv;
-    }
-    w[i] = W; m[i] = Mv; v[i] = Vv;
-    g[i] = G;  // the summed gradient of the owned slice stays readable (lrcn_get_grad gathers the slices)
-    if (push_w) {  // all-gather by posted NVLink stores
-      for (int p = 0; p < nranks; p++)
-        if (p != rank) reinterpret_cast<float4*>(peers.w[p])[i] = W;
-    }
-  }
-  if (blockIdx.x == 0 && threadIdx.x == 0 && loss_total) {
-    double t = 0.0;
-    for (int p = 0; p < nranks; p++) {
-      double x;
-      asm volatile("ld.relaxed.sys.global.f64 %0, [%1];" : "=d"(x) : "l"(&peers.ctl[p]->loss_partial) : "memory");
-      t += x;
-    }
-    *loss_total = t;
-  }
-  if (push_w) __threadfence_system();  // my stores into peer memory are performed before this kernel ends (a flag barrier follows)
-}
-// SM-driven PUSH of gradient slices into their owners' staging rows (reduce-scatter by posted NVLink stores: a peer LOAD returns
-// after microseconds and keeps registers busy meanwhile -- tools/dp_timeline.py measured ~100 GB/s per direction for the
-// pull-based exchange -- while stores are fire-and-forget, which is why NCCL's protocols push as well)
-struct PushArgs { float4* dst[8]; const float4* src[8]; size_t n4[8]; int n; };
-__global__ void __launch_bounds__(256) push_slices_kernel(const PushArgs a) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (int q = 0; q < a.n; q++) {
-    const float4* __restrict__ src = a.src[q];
-    float4* dst = a.dst[q];
-    const size_t n4 = a.n4[q];
-    for (size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < n4; i0 += 4 * stride) {
-      float4 x[4];
-#pragma unroll
-      for (int u = 0; u < 4; u++) if (i0 + u * stride < n4) x[u] = src[i0 + u * stride];
-#pragma unroll
-      for (int u = 0; u < 4; u++) if (i0 + u * stride < n4) dst[i0 + u * stride] = x[u];
-    }
-  }
-  __threadfence_system();
-}
-void dp_push_slices(cudaStream_t s, int n, float* const* dst, const float* const* src, const size_t* n_floats, int grid_ctas) {
-  PushArgs a{};
-  a.n = 0;
-  for (int q = 0; q < n && a.n < 8; q++) {
-    if (n_floats[q] == 0) continue;
-    a.dst[a.n] = reinterpret_cast<float4*>(dst[q]); a.src[a.n] = reinterpret_cast<const float4*>(src[q]); a.n4[a.n] = n_floats[q] / 4; a.n++;
-  }
-  if (a.n == 0) return;
-  push_slices_kernel<<<grid_ctas, 256, 0, s>>>(a);
-  if (g_counter) g_counter->n++;
-}
-void dp_adam_staged(cudaStream_t s, float* w, float* g, float* m, float* v, const float* stage, size_t stride, size_t stage_off, size_t b, size_t e, const P2PPeers& peers,
-                    const StepScalars* sc, double* loss_total, bool push_w, int grid_ctas) {
-  const size_t n4 = (e - b) / 4;
-  int grid = (int)((n4 + 255) / 256);
-  if (grid_ctas > 0) { if (grid > grid_ctas) grid = grid_ctas; }
-  else if (grid > 148 * 2) grid = 148 * 2;
-  if (grid < 1) grid = 1;
-  adam_staged_kernel<<<grid, 256, 0, s>>>(reinterpret_cast<float4*>(w), reinterpret_cast<float4*>(g), reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v),
-                                          reinterpret_cast<const float4*>(stage), stride / 4, stage_off / 4, b / 4, e / 4, peers.nranks, peers.rank, sc, peers, loss_total,
-                                          push_w ? 1 : 0);
-  if (g_counter) g_counter->n++;
-}
-// SM-driven exchange of ONE arena range [b, e) owned by this rank (reduce-scatter + Adam + all-gather in one kernel, no
-// barriers: the caller brackets it with dp_xgpu_barrier).  grid_ctas bounds the SMs it may take.
-// (An unrolled variant with U float4 per thread and all N*U peer loads issued up front was measured SLOWER -- 111 vs 91 us on a
-// 7.9 MB slice: the loads in flight per SM are bounded by the register file either way, and the larger CTAs only add waves.)
-void dp_p2p_adam_range(cudaStream_t s, const P2PPeers& peers, size_t b, size_t e, float* m, float* v, const StepScalars* sc, double* loss_total, int grid_ctas) {
-  adam_p2p_kernel<<<grid_ctas, 256, 0, s>>>(peers, b / 4, e / 4, reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v), sc, loss_total);
-  if (g_counter) g_counter->n++;
-}
 // ---------------------------------------------------------------------------------------------------------------------
 // FUSED bucket exchange: reduce-scatter, sharded Adam and all-gather of one gradient bucket in ONE kernel over NVLink peer
 // memory, pipelined per 32 KiB chunk (tools/dp_timeline.py showed the multi-kernel exchange spending most of its time in launch
@@ -408,127 +250,6 @@ void dp_fused_exchange(cudaStream_t s, const P2PPeers& peers, const FusedXArgs& 
   if (g_counter) g_counter->n++;
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// LL exchange of the exposed bucket.  What is left of the fused exchange when nothing hides it is latency: a system-scope fence
-// after the gradient pushes (~10 us: it waits for the NVLink write acknowledgements), the flag hop, a system-scope release
-// after the weight pushes (~10 us) and the counter hop.  Here every 16-byte line {f0, epoch, f1, epoch} is its own flag (the
-// protocol NCCL calls LL: 8-byte halves of a vector store are written atomically), so
-//   A  every rank stores its gradient slices as LL lines into the owners' LL areas              (posted stores, no fence)
-//   B  the owner polls the N-1 lines of each of its elements, sums in rank order, runs Adam, writes its own arena and stores
-//      the new weights as LL lines into every peer's LL weight area                             (no fence)
-//   C  every rank polls the LL weight lines of the other owners' slices and writes them into its own weight arena.
-// Twice the bytes on the wire for this one bucket (8.4 of 53 MB).  MEASURED SLOWER than the fused kernel (N = 2: 70 vs 50 us for the
-// bucket, 0.932 vs 0.915 ms per step -- every thread polls its own lines and the pollers compete with the incoming stores), so
-// it is opt-in (LRCN_DP_LL=1) and kept as the record of the experiment.  All CTAs are resident
-// (grid <= SMs) and run A before B before C; B polls only what peers' A phases push, C only what their B phases push.
-__device__ __forceinline__ void st_ll(uint4* p, float a, float b, unsigned int ep) {
-  asm volatile("st.volatile.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(__float_as_uint(a)), "r"(ep), "r"(__float_as_uint(b)), "r"(ep) : "memory");
-}
-__device__ __forceinline__ bool ld_ll(const uint4* p, unsigned int ep, float& a, float& b, unsigned int& spins) {
-  while (true) {
-    uint4 x;
-    asm volatile("ld.relaxed.sys.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x.x), "=r"(x.y), "=r"(x.z), "=r"(x.w) : "l"(p) : "memory");
-    if (x.y == ep && x.w == ep) { a = __uint_as_float(x.x); b = __uint_as_float(x.z); return true; }
-    if ((++spins & 1023u) == 0u) {
-      if (dev_aborted()) return false;
-      if (spins > (1u << 27)) {  // ~ tens of seconds of polling
-        printf("lrcn dp_p2p: LL exchange timeout (rank %d, epoch %u, have %u/%u)\n", 0, ep, x.y, x.w);
-        dev_abort_set();
-        return false;
-      }
-    }
-  }
-}
-__global__ void __launch_bounds__(256) ll_exchange_kernel(const P2PPeers peers, const LLXArgs a, float4* __restrict__ m, float4* __restrict__ v,
-                                                          const StepScalars* __restrict__ sc, double* loss_total) {
-  const int N = peers.nranks, me = peers.rank;
-  const unsigned int ep = sc->xchg_epoch;
-  const size_t stride = (size_t)gridDim.x * blockDim.x, t0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const float4* gl = reinterpret_cast<const float4*>(peers.g[me]);
-  unsigned int spins = 0;
-  // ---- A: my gradient slices, as LL lines, into the owners' areas (region `me`)
-  for (int d = 1; d < N; d++) {
-    const int r = (me + d) % N;
-    const size_t n4 = a.e4[r] - a.b4[r];
-    uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<float4*>(a.stage[r]) + a.llg4) + (size_t)me * 2 * a.per4;
-    for (size_t i = t0; i < n4; i += stride) {
-      const float4 x = gl[a.b4[r] + i];
-      st_ll(dst + 2 * i, x.x, x.y, ep);
-      st_ll(dst + 2 * i + 1, x.z, x.w, ep);
-    }
-  }
-  // ---- B: my slice
-  {
-    const float b1 = sc->beta1, b2 = sc->beta2, lr = sc->lr, eps = sc->eps, d1 = sc->adam_d1, d2 = sc->adam_d2;
-    const float ob1 = sc->one_m_beta1, ob2 = sc->one_m_beta2;
-    const size_t b4 = a.b4[me], n4 = a.e4[me] - a.b4[me];
-    const uint4* mine = reinterpret_cast<const uint4*>(reinterpret_cast<const float4*>(a.stage[me]) + a.llg4);
-    float4* wl = reinterpret_cast<float4*>(peers.w[me]);
-    float4* gw = reinterpret_cast<float4*>(peers.g[me]);
-    for (size_t i = t0; i < n4; i += stride) {
-      float4 W = wl[b4 + i], Mv = m[b4 + i], Vv = v[b4 + i];
-      const float4 own = gl[b4 + i];
-      float4 Gs = make_float4(0.f, 0.f, 0.f, 0.f);
-      for (int q = 0; q < N; q++) {  // fixed rank order: deterministic, identical on every rank
-        float4 x = own;
-        if (q != me) {
-          const uint4* src = mine + (size_t)q * 2 * a.per4 + 2 * i;
-          if (!ld_ll(src, ep, x.x, x.y, spins) || !ld_ll(src + 1, ep, x.z, x.w, spins)) return;
-        }
-        Gs.x += x.x; Gs.y += x.y; Gs.z += x.z; Gs.w += x.w;
-      }
-      float* wp = reinterpret_cast<float*>(&W);
-      const float* gp = reinterpret_cast<const float*>(&Gs);
-      float* mp = reinterpret_cast<float*>(&Mv);
-      float* vp = reinterpret_cast<float*>(&Vv);
-#pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const float mm = __fadd_rn(__fmul_rn(b1, mp[k]), __fmul_rn(ob1, gp[k]));
-        const float vv = __fadd_rn(__fmul_rn(b2, vp[k]), __fmul_rn(ob2, __fmul_rn(gp[k], gp[k])));
-        const float upd = __fdiv_rn(__fdiv_rn(mm, d1), __fadd_rn(__fsqrt_rn(__fdiv_rn(vv, d2)), eps));
-        wp[k] = __fsub_rn(wp[k], __fmul_rn(lr, upd));
-        mp[k] = mm; vp[k] = vv;
-      }
-      for (int d = 1; d < N; d++) {  // the new weights, as LL lines, into every peer's area (region `me`)
-        const int p = (me + d) % N;
-        uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<float4*>(a.stage[p]) + a.llw4) + (size_t)me * 2 * a.per4;
-        st_ll(dst + 2 * i, W.x, W.y, ep);
-        st_ll(dst + 2 * i + 1, W.z, W.w, ep);
-      }
-      wl[b4 + i] = W; m[b4 + i] = Mv; v[b4 + i] = Vv;
-      gw[b4 + i] = Gs;  // the summed gradient of the owned slice stays readable (lrcn_get_grad gathers the slices)
-    }
-  }
-  // ---- C: the other owners' new weights
-  {
-    const uint4* mine = reinterpret_cast<const uint4*>(reinterpret_cast<const float4*>(a.stage[me]) + a.llw4);
-    float4* wl = reinterpret_cast<float4*>(peers.w[me]);
-    for (int d = 1; d < N; d++) {
-      const int q = (me + d) % N;
-      const size_t n4 = a.e4[q] - a.b4[q];
-      const uint4* src = mine + (size_t)q * 2 * a.per4;
-      for (size_t i = t0; i < n4; i += stride) {
-        float4 W;
-        if (!ld_ll(src + 2 * i, ep, W.x, W.y, spins) || !ld_ll(src + 2 * i + 1, ep, W.z, W.w, spins)) return;
-        wl[a.b4[q] + i] = W;
-      }
-    }
-  }
-  if (blockIdx.x == 0 && threadIdx.x == 0 && loss_total) {
-    double t = 0.0;
-    for (int p = 0; p < N; p++) {
-      double x;
-      asm volatile("ld.relaxed.sys.global.f64 %0, [%1];" : "=d"(x) : "l"(&peers.ctl[p]->loss_partial) : "memory");
-      t += x;
-    }
-    *loss_total = t;
-  }
-}
-void dp_ll_exchange(cudaStream_t s, const P2PPeers& peers, const LLXArgs& a, float* m, float* v, const StepScalars* sc, double* loss_total, int grid_ctas) {
-  ll_exchange_kernel<<<grid_ctas, 256, 0, s>>>(peers, a, reinterpret_cast<float4*>(m), reinterpret_cast<float4*>(v), sc, loss_total);
-  if (g_counter) g_counter->n++;
-}
-
 // timeline stamps of the data-parallel step (LRCN_DP_STAMPS=1, tools/dp_timeline.py): %globaltimer at a point of a stream
 __global__ void stamp_kernel(unsigned long long* out) {
   unsigned long long t;
@@ -537,9 +258,5 @@ __global__ void stamp_kernel(unsigned long long* out) {
 }
 void dp_stamp(cudaStream_t s, unsigned long long* out) { stamp_kernel<<<1, 1, 0, s>>>(out); }
 
-void dp_xgpu_barrier(cudaStream_t s, const P2PPeers& peers, unsigned int* epoch_ctr, int flagset, unsigned long long* trace) {
-  xgpu_barrier_kernel<<<1, 32, 0, s>>>(peers, epoch_ctr, 16 * flagset, trace);
-  if (g_counter) g_counter->n++;
-}
 
 }  // namespace lrcn

@@ -233,16 +233,7 @@ struct P2PCtl {              // one per rank, in a small exported allocation
 struct P2PPeers { float* g[LRCN_P2P_MAX_RANKS]; float* w[LRCN_P2P_MAX_RANKS]; P2PCtl* ctl[LRCN_P2P_MAX_RANKS]; int nranks, rank; };
 // barrier, in-place allreduce(sum) of the gradient arena (n_floats) + loss total, barrier
 void dp_p2p_allreduce(cudaStream_t s, const P2PPeers& peers, size_t n_floats, unsigned int* epoch_ctr, double* loss_total);
-// training step: barrier, then every rank sums ITS shard of the gradient over all ranks, applies Adam to that shard (m, v are
-// this rank's arrays; only the owned shard is kept current) and stores the new weights into every rank's arena, barrier
-void dp_p2p_adam(cudaStream_t s, const P2PPeers& peers, size_t n_floats, unsigned int* epoch_ctr, double* loss_total, float* m, float* v,
-                 const StepScalars* sc);
-// [begin, end) of rank r's shard, in floats
-void dp_p2p_shard(size_t n_floats, int nranks, int r, size_t* begin, size_t* end);
-// copy-engine exchange (dp_p2p.cu): flag barrier on one of 4 independent flag sets; owner-side sum of the staged
-// contributions + Adam over the arena range [b, e) (floats, multiples of 4); stage rows have `stride` floats, the range's
-// contributions start at stage_off inside a row
-void dp_xgpu_barrier(cudaStream_t s, const P2PPeers& peers, unsigned int* epoch_ctr, int flagset, unsigned long long* trace = nullptr);
+// %globaltimer stamp at a point of a stream (LRCN_DP_STAMPS=1, tools/dp_timeline.py)
 void dp_stamp(cudaStream_t s, unsigned long long* out);
 // FUSED exchange of one gradient bucket (dp_p2p.cu): push of gradient chunks -> per-chunk flags -> owner-side sum + Adam ->
 // push of the new weights -> completion counters, all in ONE kernel.  The control words live behind the staging rows.
@@ -255,20 +246,6 @@ struct FusedXArgs {
   int bucket, sub;
 };
 void dp_fused_exchange(cudaStream_t s, const P2PPeers& peers, const FusedXArgs& a, float* m, float* v, const StepScalars* sc, double* loss_total, int grid_ctas);
-// Flag-in-data ("LL") exchange of the EXPOSED bucket (dp_p2p.cu): every 16-byte line carries two floats and two copies of the
-// step's epoch, so a receiver knows a line has arrived from the line itself -- no system-scope fence, no flag round trip.
-struct LLXArgs {
-  float* stage[LRCN_P2P_MAX_RANKS];             // every rank's staging allocation
-  size_t b4[LRCN_P2P_MAX_RANKS], e4[LRCN_P2P_MAX_RANKS];  // rank r's slice of the bucket, arena index in float4 units
-  size_t per4;                                   // slice capacity (float4): a source's region of the LL areas holds 2 lines per float4
-  size_t llg4, llw4;                             // start of the LL gradient / LL weight areas inside a staging allocation (float4 units)
-};
-void dp_ll_exchange(cudaStream_t s, const P2PPeers& peers, const LLXArgs& a, float* m, float* v, const StepScalars* sc, double* loss_total, int grid_ctas);
-void dp_p2p_adam_range(cudaStream_t s, const P2PPeers& peers, size_t b, size_t e, float* m, float* v, const StepScalars* sc, double* loss_total, int grid_ctas);
-void dp_adam_staged(cudaStream_t s, float* w, float* g, float* m, float* v, const float* stage, size_t stride, size_t stage_off, size_t b, size_t e, const P2PPeers& peers,
-                    const StepScalars* sc, double* loss_total, bool push_w = false, int grid_ctas = 0);
-// n slices: dst[q] (peer memory) <- src[q] (local), n_floats[q] floats each (multiples of 4, 16-byte aligned)
-void dp_push_slices(cudaStream_t s, int n, float* const* dst, const float* const* src, const size_t* n_floats, int grid_ctas);
 // diagnostics (probe_mma.cu): clocks to issue / to complete a chain of n_mma tcgen05.mma M x N x 16 from resident smem operands
 bool probe_mma(cudaStream_t s, int M, int N, int n_mma, int commit_every, int issuers, long long* issue_clk, long long* total_clk);
 

@@ -164,7 +164,7 @@ static int s_destroy(lrcn_handle* h) {
   if (!h->peers_direct) for (void* q : h->p2p_opened) if (q) cudaIpcCloseMemHandle(q);
   for (cudaEvent_t e : h->sc_ev) if (e) cudaEventDestroy(e);
   void* ptrs[] = {h->w, h->g, h->m, h->v, h->w_hi, h->w_lo, h->wp1_hi, h->wp1_lo, h->wp2_hi, h->wp2_lo, h->wt1_hi, h->wt1_lo, h->wt2_hi, h->wt2_lo, h->tab[0].d, h->tab[1].d, h->ws.f, h->ws.hi, h->ws.lo, h->d_tok_in,
-                  h->d_tok_tgt, h->d_rows, h->d_sc, h->p2p_ctl, h->d_loss_total, h->d_epoch, h->d_epoch_side, h->stage, h->d_counters, h->d_trace, h->g_last, h->g_ctok, h->g_stok, h->g_spar, h->g_hista, h->g_histb,
+                  h->d_tok_tgt, h->d_rows, h->d_sc, h->p2p_ctl, h->d_loss_total, h->d_epoch, h->stage, h->d_counters, h->d_trace, h->g_last, h->g_ctok, h->g_stok, h->g_spar, h->g_hista, h->g_histb,
                   h->g_done, h->g_ndone, h->g_olen, h->g_rows, h->g_otok, h->l2_scratch, h->g_keep, h->g_omap, h->g_omap_s, h->d_gnorm};
   for (void* p : ptrs) if (p) cudaFree(p);
   for (void* q : {(void*)h->ep_seq, (void*)h->ep_ids, (void*)h->ep_rows, (void*)h->ep_loss, (void*)h->ep_err, (void*)h->tab[0].d_ids, (void*)h->tab[0].d_rowof,
@@ -178,8 +178,6 @@ static int s_destroy(lrcn_handle* h) {
   if (h->h_keep) cudaFreeHost(h->h_keep);
   for (int i = 0; i < lrcn_handle::NSNAP; i++) { if (h->ev_snap[i]) cudaEventDestroy(h->ev_snap[i]); if (h->ev_keep[i]) cudaEventDestroy(h->ev_keep[i]); }
   for (cudaEvent_t e : {h->ev0, h->ev1, h->ev_seg[0], h->ev_seg[1], h->ev_seg[2], h->ev_seg[3], h->ev_comm}) if (e) cudaEventDestroy(e);
-  if (h->ev_xfork) cudaEventDestroy(h->ev_xfork);
-  for (int i = 0; i < lrcn_handle::NXFER; i++) { if (h->ev_xjoin[i]) cudaEventDestroy(h->ev_xjoin[i]); if (h->xfer[i]) cudaStreamDestroy(h->xfer[i]); }
   if (h->comm_stream) cudaStreamDestroy(h->comm_stream);
   if (h->side_stream) cudaStreamDestroy(h->side_stream);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -225,11 +223,6 @@ static int create_impl(const lrcn_config* cfg, lrcn_handle* h) {
   CK(cudaEventCreate(&h->ev1));
   for (int i = 0; i < 4; i++) CK(cudaEventCreateWithFlags(&h->ev_seg[i], cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&h->ev_comm, cudaEventDisableTiming));
-  CK(cudaEventCreateWithFlags(&h->ev_xfork, cudaEventDisableTiming));
-  for (int i = 0; i < lrcn_handle::NXFER; i++) {
-    CK(cudaStreamCreateWithFlags(&h->xfer[i], cudaStreamNonBlocking));
-    CK(cudaEventCreateWithFlags(&h->ev_xjoin[i], cudaEventDisableTiming));
-  }
 
   // ---- parameter arenas, bucket order (1-based model index): [8,9 | 3,4,5,6 | 1,2,7]
   const int order[9] = {8, 9, 3, 4, 5, 6, 1, 2, 7};
@@ -306,12 +299,9 @@ static int create_impl(const lrcn_config* cfg, lrcn_handle* h) {
   CK(cudaMalloc(&h->p2p_ctl, 4096)); CK(cudaMemset(h->p2p_ctl, 0, 4096));
   h->d_loss = &h->p2p_ctl->loss_partial;
   CK(cudaMalloc(&h->d_loss_total, 8)); CK(cudaMalloc(&h->d_epoch, 4)); CK(cudaMemset(h->d_epoch, 0, 4));
-  CK(cudaMalloc(&h->d_epoch_side, 4)); CK(cudaMemset(h->d_epoch_side, 0, 4));
-  // + the control words of the fused exchange + the two LL areas of the exposed bucket [W1, b1] (dp_p2p.cu): 2 lines of 16 bytes
-  // per float4 and source rank, slices padded by up to 4 floats per rank
-  h->ll_floats = 2 * (h->bucket_off[3] - h->bucket_off[2] + 4 * LRCN_P2P_MAX_RANKS + 64);
-  CK(cudaMalloc(&h->stage, (h->P + 1024 + DP_XCTL_FLOATS + 2 * h->ll_floats) * 4));
-  CK(cudaMemset(h->stage, 0, (h->P + 1024 + DP_XCTL_FLOATS + 2 * h->ll_floats) * 4));  // N staging rows of ~P/N floats each for the copy-engine gradient exchange
+  // the fused exchange (dp_p2p.cu): N staging rows of ~P/N floats each (slices padded to multiples of 4 floats), then its control words
+  CK(cudaMalloc(&h->stage, (h->P + 1024 + DP_XCTL_FLOATS) * 4));
+  CK(cudaMemset(h->stage, 0, (h->P + 1024 + DP_XCTL_FLOATS) * 4));
   CK(cudaMallocHost(&h->h_loss, 8));
   CK(cudaMalloc(&h->d_counters, 320 * sizeof(unsigned int)));  // [0,256): 4 LSTM launches x 64 (half-)tile barriers; [256,..): softmax
   CK(cudaMemset(h->d_counters, 0, 320 * sizeof(unsigned int)));
@@ -475,9 +465,7 @@ static int s_get_param(lrcn_handle* h, int idx, float* p, int64_t rows, int64_t 
   int rc = check_shape(h, idx, p, rows, cols);
   return rc ? rc : download(h, h->w, idx, p);
 }
-// Peer-memory data parallelism (dp_p2p.cu) leaves m, v -- and after a sharded train step the summed gradient -- current only
-// in each owner's shard: collect the other shards from their owners.  All ranks must be idle (e.g. at a checkpoint barrier).
-// copy-engine exchange: every gradient bucket k (arena range [bucket_off[k], bucket_off[k+1])) is split into N slices of
+// fused exchange (dp_p2p.cu): every gradient bucket k (arena range [bucket_off[k], bucket_off[k+1])) is split into N slices of
 // per_k floats (multiples of 4); rank r owns [b, e) of it and its contributions sit at row offset pre_k of a staging row
 struct BucketShard { size_t b, e, pre, per; };
 static BucketShard bucket_shard(const lrcn_handle* h, int k, int r) {
@@ -499,22 +487,23 @@ static size_t stage_stride(const lrcn_handle* h) {
   return s.pre + s.per;
 }
 
+// A peer-memory train step leaves m, v and the summed gradient current only in each owner's slices: collect the other slices
+// from their owners.  All ranks must be idle (e.g. at a checkpoint barrier).
 static int gather_shards(lrcn_handle* h, bool adam, bool grad) {
   CK(cudaSetDevice(h->cfg.device));
   CK(cudaStreamSynchronize(h->stream));
   for (int r = 0; r < h->nranks; r++) {
     if (r == h->rank) continue;
-    for (int k = 0; k < (h->shard_by_bucket ? lrcn_handle::NBUCKET : 1); k++) {
-    size_t b, e;
-    if (h->shard_by_bucket) { const BucketShard bs = bucket_shard(h, k, r); b = bs.b; e = bs.e; }
-    else dp_p2p_shard(h->P, h->nranks, r, &b, &e);
-    if (e <= b) continue;
-    // on the handle's stream: device-to-device cudaMemcpy does not synchronise the host, and the download that follows is stream-ordered
-    if (adam) {
-      CK(cudaMemcpyAsync(h->m + b, h->peer_m[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
-      CK(cudaMemcpyAsync(h->v + b, h->peer_v[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
-    }
-    if (grad) CK(cudaMemcpyAsync(h->g + b, h->peers.g[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
+    for (int k = 0; k < lrcn_handle::NBUCKET; k++) {
+      const BucketShard bs = bucket_shard(h, k, r);
+      const size_t b = bs.b, e = bs.e;
+      if (e <= b) continue;
+      // on the handle's stream: device-to-device cudaMemcpy does not synchronise the host, and the download that follows is stream-ordered
+      if (adam) {
+        CK(cudaMemcpyAsync(h->m + b, h->peer_m[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
+        CK(cudaMemcpyAsync(h->v + b, h->peer_v[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
+      }
+      if (grad) CK(cudaMemcpyAsync(h->g + b, h->peers.g[r] + b, (e - b) * 4, cudaMemcpyDefault, h->stream));
     }
   }
   CK(cudaStreamSynchronize(h->stream));
@@ -944,247 +933,88 @@ static int run_step(lrcn_handle* h, int split, int B, int l, float pdrop, uint64
   static const bool force_nccl = getenv("LRCN_DP_NCCL") != nullptr;
   if (h->p2p_ready && !force_nccl) {
     h->loss_is_total = true;
-    static const bool replicated = getenv("LRCN_DP_REPLICATED_ADAM") != nullptr;
-    static const bool kernel_exchange = getenv("LRCN_DP_KERNEL_EXCHANGE") != nullptr;  // round-1 SM-driven exchange after the backward pass
-    static const bool ce_exchange = getenv("LRCN_DP_CE") != nullptr;  // copy-engine exchange: measured slower (many small copies), kept for reference
-    if (mode == 2 && !replicated) { h->adam_sharded = h->grad_sharded = true; h->shard_by_bucket = !kernel_exchange; }
-    else h->grad_sharded = false;
-    if (mode == 2 && !replicated && !kernel_exchange && !ce_exchange) {
-      // Bucketed SM-driven exchange overlapped with the backward pass.  The owner-computes kernel of bucket 1 (Wout, bout) runs
-      // on a side stream (a parallel branch of the step's graph) under the layer-2 BPTT kernel, that of bucket 2 (W2, b2, Wf, Wcnn)
-      // under the layer-1 BPTT kernel: the persistent LSTM kernels hold 128 of the 148 SMs with one (register-file-filling) CTA
-      // each, so the exchange CTAs land on the 20 SMs they leave free -- and because every exchange starts with a cross-GPU flag
-      // barrier (a 1-warp kernel that co-resides anywhere), the LSTM grid is resident before the exchange kernel is launched.
-      // The layer-1 segment ends with two buckets: the embedding gradient (Wemb, two thirds of the segment's bytes) is produced
-      // FIRST (dE GEMM + scatter) and travels on the side stream under the layer-1 weight-gradient GEMM (whose CTAs leave room
-      // for co-resident exchange CTAs on every SM); only bucket 3 (W1, b1) is exposed.
-      static const int wemb_ctas = getenv("LRCN_DP_WEMB_CTAS") ? atoi(getenv("LRCN_DP_WEMB_CTAS")) : 148 * 4;
-      static const bool stamps = getenv("LRCN_DP_STAMPS") != nullptr;
-      return run_cached(h, std::make_tuple(24, B, l, fl), [&] {
-        // stamps (tools/dp_timeline.py): main stream 0..7 = start, fwd done, seg1, seg2, seg31, seg32, last exchange done, joined;
-        // bucket k: 8+4k .. = enter, first barrier passed, exchange kernel done, second barrier + split done
-        auto stamp = [&](int id, cudaStream_t st) { if (stamps && h->d_trace) dp_stamp(st, h->d_trace + id); };
-        static const bool pull = getenv("LRCN_DP_PULL") != nullptr;  // round-2a exchange: the owner LOADS its shard from every peer
-        // measured at N = 2: 0.932 ms per step with the LL kernel on the exposed bucket vs 0.915 with the fused kernel (70 vs 50 us for
-        // the bucket: 38 k threads polling their lines compete with the incoming stores), so it is opt-in
-        static const bool ll = getenv("LRCN_DP_LL") != nullptr;
-        static const bool fused = !pull && getenv("LRCN_DP_PUSH") == nullptr;  // default; LRCN_DP_PUSH=1: push / barrier / Adam / barrier as four kernels
-        const size_t stride = stage_stride(h);
-        auto exchange_bucket = [&](int k, cudaStream_t st, unsigned int* epoch, int flagset, bool last) {
-          const int ctas = last ? 148 * 4 : (k == 3 ? wemb_ctas : 20 * 8);
-          if (fused && last && ll) {
-            // the exposed bucket: flag-in-data lines, no fences, no flag hops (dp_p2p.cu)
-            stamp(8 + 4 * k, st);
-            LLXArgs a{};
-            for (int r = 0; r < h->nranks; r++) {
-              const BucketShard bs = bucket_shard(h, k, r);
-              a.stage[r] = h->peer_stage[r]; a.b4[r] = bs.b / 4; a.e4[r] = bs.e / 4; a.per4 = bs.per / 4;
-            }
-            a.llg4 = (h->P + 1024 + DP_XCTL_FLOATS) / 4; a.llw4 = a.llg4 + h->ll_floats / 4;
-            dp_ll_exchange(st, h->peers, a, h->m, h->v, h->d_sc, h->d_loss_total, 148);
-            stamp(10 + 4 * k, st);
-            if (h->bf16mode) {
-              const size_t b0 = h->bucket_off[k], nn = h->bucket_off[k + 1] - b0;
-              split_bf16(st, h->w + b0, nn, h->w_hi + b0, h->w_lo + b0);
-            }
-            stamp(11 + 4 * k, st);
-            return;
-          }
-          if (fused) {
-            // ONE kernel per bucket: chunk-pipelined push -> flags -> owner sum + Adam -> weight push -> completion counters
-            stamp(8 + 4 * k, st);
-            FusedXArgs a{};
-            for (int r = 0; r < h->nranks; r++) {
-              const BucketShard bs = bucket_shard(h, k, r);
-              a.stage[r] = h->peer_stage[r]; a.b4[r] = bs.b / 4; a.e4[r] = bs.e / 4;
-              a.pre4 = bs.pre / 4;
-            }
-            a.stride4 = stride / 4; a.ctl4 = (h->P + 1024) / 4; a.bucket = k;
-            dp_fused_exchange(st, h->peers, a, h->m, h->v, h->d_sc, last ? h->d_loss_total : nullptr, last ? 148 * 4 : (k == 3 ? wemb_ctas : 20 * 4));
-            stamp(10 + 4 * k, st);
-            if (h->bf16mode) {
-              const size_t b0 = h->bucket_off[k], nn = h->bucket_off[k + 1] - b0;
-              split_bf16(st, h->w + b0, nn, h->w_hi + b0, h->w_lo + b0);
-            }
-            stamp(11 + 4 * k, st);
-            return;
-          }
-          if (!pull) {
-            // PUSH exchange: (1) every rank stores its slices of the bucket's gradient into the owners' staging rows; (2) flag
-            // barrier: all pushes have landed, and every rank is past its last use of the bucket's weights; (3) the owner sums the
-            // N contributions in rank order, runs Adam on its slice and stores the new weights into every peer's arena;
-            // (4) flag barrier: the new weights have landed everywhere; (5) local bf16 shadows.
-            stamp(8 + 4 * k, st);
-            float* dst[8]; const float* src[8]; size_t nf[8]; int n = 0;
-            for (int d = 1; d < h->nranks; d++) {
-              const int r = (h->rank + d) % h->nranks;  // staggered targets: no two ranks start on the same peer
-              const BucketShard bs = bucket_shard(h, k, r);
-              dst[n] = h->peer_stage[r] + (size_t)h->rank * stride + bs.pre; src[n] = h->g + bs.b; nf[n] = bs.e - bs.b; n++;
-            }
-            dp_push_slices(st, n, dst, src, nf, ctas);
-            dp_xgpu_barrier(st, h->peers, epoch, flagset, stamps && h->d_trace ? h->d_trace + 32 + k : nullptr);
-            stamp(9 + 4 * k, st);
-            const BucketShard me = bucket_shard(h, k, h->rank);
-            if (me.e > me.b || last)
-              dp_adam_staged(st, h->w, h->g, h->m, h->v, h->stage, stride, me.pre, me.b, me.e, h->peers, h->d_sc, last ? h->d_loss_total : nullptr, true, ctas);
-            stamp(10 + 4 * k, st);
-            dp_xgpu_barrier(st, h->peers, epoch, flagset);
-            if (h->bf16mode) {
-              const size_t b0 = h->bucket_off[k], nn = h->bucket_off[k + 1] - b0;
-              split_bf16(st, h->w + b0, nn, h->w_hi + b0, h->w_lo + b0);
-            }
-            stamp(11 + 4 * k, st);
-            return;
-          }
-          stamp(8 + 4 * k, st);
-          dp_xgpu_barrier(st, h->peers, epoch, flagset, stamps && h->d_trace ? h->d_trace + 32 + k : nullptr);  // every rank's gradients of this bucket are complete, and every rank is past its last use of the bucket's weights
-          stamp(9 + 4 * k, st);
-          const BucketShard me = bucket_shard(h, k, h->rank);
-          if (me.e > me.b || last) dp_p2p_adam_range(st, h->peers, me.b, me.e, h->m, h->v, h->d_sc, last ? h->d_loss_total : nullptr, ctas);
-          stamp(10 + 4 * k, st);
-          dp_xgpu_barrier(st, h->peers, epoch, flagset);  // every owner's new weights of this bucket have landed everywhere
-          if (h->bf16mode) {
-            const size_t b0 = h->bucket_off[k], n = h->bucket_off[k + 1] - b0;
-            split_bf16(st, h->w + b0, n, h->w_hi + b0, h->w_lo + b0);
-          }
-          stamp(11 + 4 * k, st);
-        };
-        stamp(0, h->stream);
+    if (mode == 1) {
+      // gradient only: backward pass, then ONE owner-computes allreduce kernel over NVLink peer memory between two flag
+      // barriers (dp_p2p.cu): no NCCL kernels competing for SMs with the persistent GEMM / LSTM kernels
+      h->grad_sharded = false;
+      return run_cached(h, std::make_tuple(21, B, l, fl), [&] {
         enqueue_forward(h, split, B, l, true);
-        stamp(1, h->stream);
-        enqueue_backward_seg(h, B, l, true, 1);
-        stamp(2, h->stream);
-        cudaEventRecord(h->ev_seg[0], h->stream);
-        cudaStreamWaitEvent(h->comm_stream, h->ev_seg[0], 0);
-        exchange_bucket(0, h->comm_stream, h->d_epoch_side, 1, false);
-        enqueue_backward_seg(h, B, l, true, 2);
-        stamp(3, h->stream);
-        cudaEventRecord(h->ev_seg[1], h->stream);
-        cudaStreamWaitEvent(h->comm_stream, h->ev_seg[1], 0);
-        exchange_bucket(1, h->comm_stream, h->d_epoch_side, 1, false);
-        enqueue_backward_seg(h, B, l, true, 31);
-        stamp(4, h->stream);
-        cudaEventRecord(h->ev_seg[2], h->stream);
-        cudaStreamWaitEvent(h->comm_stream, h->ev_seg[2], 0);
-        exchange_bucket(3, h->comm_stream, h->d_epoch_side, 1, false);
-        cudaEventRecord(h->ev_comm, h->comm_stream);
-        enqueue_backward_seg(h, B, l, true, 32);
-        stamp(5, h->stream);
-        exchange_bucket(2, h->stream, h->d_epoch, 0, true);
-        stamp(6, h->stream);
-        cudaStreamWaitEvent(h->stream, h->ev_comm, 0);  // join the side branch
-        stamp(7, h->stream);
-      });
-    }
-    if (mode == 2 && !replicated && !kernel_exchange) {
-      // copy-engine exchange (dp_p2p.cu): bucket 1 (Wout, bout) travels under the layer-2 BPTT, bucket 2 (W2, b2, Wf, Wcnn)
-      // under the layer-1 BPTT on a side stream (a parallel branch of the step's graph); only bucket 3 (W1, b1, Wemb) is exposed
-      return run_cached(h, std::make_tuple(23, B, l, fl), [&] {
-        const size_t stride = stage_stride(h);
-        // the N-1 copies of a phase run on parallel branches of the graph (several DMA engines), forked from / joined into `st`
-        auto parallel_copies = [&](cudaStream_t st, auto&& issue /* (rank r, stream) */) {
-          if (h->nranks <= 2) { for (int r = 0; r < h->nranks; r++) if (r != h->rank) issue(r, st); return; }
-          cudaEventRecord(h->ev_xfork, st);
-          for (int i = 0; i < lrcn_handle::NXFER; i++) cudaStreamWaitEvent(h->xfer[i], h->ev_xfork, 0);
-          int n = 0;
-          for (int d = 1; d < h->nranks; d++, n++) issue((h->rank + d) % h->nranks, h->xfer[n % lrcn_handle::NXFER]);  // staggered targets: no two ranks start on the same peer
-          for (int i = 0; i < lrcn_handle::NXFER; i++) { cudaEventRecord(h->ev_xjoin[i], h->xfer[i]); cudaStreamWaitEvent(st, h->ev_xjoin[i], 0); }
-        };
-        auto exchange_bucket = [&](int k, cudaStream_t st, unsigned int* epoch, int flagset, bool last) {
-          parallel_copies(st, [&](int r, cudaStream_t cs) {  // reduce-scatter: push my gradient slices to their owners
-            const BucketShard bs = bucket_shard(h, k, r);
-            if (bs.e > bs.b) cudaMemcpyAsync(h->peer_stage[r] + (size_t)h->rank * stride + bs.pre, h->g + bs.b, (bs.e - bs.b) * 4, cudaMemcpyDeviceToDevice, cs);
-          });
-          dp_xgpu_barrier(st, h->peers, epoch, flagset);  // every rank's pushes of this bucket have landed (and every rank is past its last use of the bucket's weights)
-          const BucketShard me = bucket_shard(h, k, h->rank);
-          if (me.e > me.b || last)
-            dp_adam_staged(st, h->w, h->g, h->m, h->v, h->stage, stride, me.pre, me.b, me.e, h->peers, h->d_sc, last ? h->d_loss_total : nullptr);
-          if (me.e > me.b)
-            parallel_copies(st, [&](int r, cudaStream_t cs) {  // all-gather: push the new weights of my slice
-              cudaMemcpyAsync(h->peers.w[r] + me.b, h->w + me.b, (me.e - me.b) * 4, cudaMemcpyDeviceToDevice, cs);
-            });
-          dp_xgpu_barrier(st, h->peers, epoch, flagset);  // every owner's new weights of this bucket have landed everywhere
-          if (h->bf16mode) {  // refresh the bf16 hi / lo shadows of the bucket (the exposed pass shrinks to the last bucket)
-            const size_t b0 = h->bucket_off[k], n = h->bucket_off[k + 1] - b0;
-            split_bf16(st, h->w + b0, n, h->w_hi + b0, h->w_lo + b0);
-          }
-        };
-        enqueue_forward(h, split, B, l, true);
-        enqueue_backward_seg(h, B, l, true, 1);
-        cudaEventRecord(h->ev_seg[0], h->stream);
-        cudaStreamWaitEvent(h->comm_stream, h->ev_seg[0], 0);
-        exchange_bucket(0, h->comm_stream, h->d_epoch_side, 1, false);
-        enqueue_backward_seg(h, B, l, true, 2);
-        cudaEventRecord(h->ev_seg[1], h->stream);
-        cudaStreamWaitEvent(h->comm_stream, h->ev_seg[1], 0);
-        exchange_bucket(1, h->comm_stream, h->d_epoch_side, 1, false);
-        cudaEventRecord(h->ev_comm, h->comm_stream);
-        enqueue_backward_seg(h, B, l, true, 3);
-        exchange_bucket(2, h->stream, h->d_epoch, 0, false);
-        exchange_bucket(3, h->stream, h->d_epoch, 0, true);
-        cudaStreamWaitEvent(h->stream, h->ev_comm, 0);  // join the side branch
-      });
-    }
-    // backward pass, then ONE owner-computes exchange kernel over NVLink peer memory between two flag barriers (dp_p2p.cu),
-    // then the replicated Adam: no NCCL kernels competing for SMs with the persistent GEMM / LSTM kernels
-    return run_cached(h, std::make_tuple(mode == 2 ? 22 : 21, B, l, fl), [&] {
-      enqueue_forward(h, split, B, l, true);
-      for (int seg = 1; seg <= 3; seg++) enqueue_backward_seg(h, B, l, true, seg);
-      if (mode == 2 && !replicated) {
-        // reduce-scatter + Adam on the owned shard + all-gather of the new weights in one kernel; then the local bf16 shadows
-        dp_p2p_adam(h->stream, h->peers, h->P, h->d_epoch, h->d_loss_total, h->m, h->v, h->d_sc);
-        if (h->bf16mode) split_bf16(h->stream, h->w, h->P, h->w_hi, h->w_lo);
-      } else {
+        for (int seg = 1; seg <= 3; seg++) enqueue_backward_seg(h, B, l, true, seg);
         dp_p2p_allreduce(h->stream, h->peers, h->P, h->d_epoch, h->d_loss_total);
-        if (mode == 2) enqueue_adam(h, false);
-      }
+      });
+    }
+    h->adam_sharded = h->grad_sharded = true;
+    // Train step: one fused exchange kernel per gradient bucket (reduce-scatter + sharded Adam + all-gather, dp_p2p.cu),
+    // overlapped with the backward pass.  Bucket 1 (Wout, bout) runs on a side stream (a parallel branch of the step's graph)
+    // under the layer-2 BPTT kernel, bucket 2 (W2, b2, Wf, Wcnn) under the layer-1 BPTT kernel: the persistent LSTM kernels hold
+    // 128 of the 148 SMs with one (register-file-filling) CTA each, so the 80 exchange CTAs land on the 20 SMs they leave free.
+    // The layer-1 segment ends with two buckets: the embedding gradient (Wemb, two thirds of the segment's bytes) is produced
+    // FIRST (dE GEMM + scatter) and travels on the side stream under the layer-1 weight-gradient GEMM (whose CTAs leave room
+    // for co-resident exchange CTAs on every SM); only bucket 3 (W1, b1) is exposed.
+    static const bool stamps = getenv("LRCN_DP_STAMPS") != nullptr;
+    return run_cached(h, std::make_tuple(24, B, l, fl), [&] {
+      // stamps (tools/dp_timeline.py): main stream 0..7 = start, fwd done, seg1, seg2, seg31, seg32, last exchange done, joined;
+      // bucket k: 8+4k = enter, 10+4k = exchange kernel done, 11+4k = bf16 split done
+      auto stamp = [&](int id, cudaStream_t st) { if (stamps && h->d_trace) dp_stamp(st, h->d_trace + id); };
+      const size_t stride = stage_stride(h);
+      // last: the exposed bucket, which also sums the loss over the ranks
+      auto exchange_bucket = [&](int k, cudaStream_t st, int ctas, bool last) {
+        stamp(8 + 4 * k, st);
+        FusedXArgs a{};
+        for (int r = 0; r < h->nranks; r++) {
+          const BucketShard bs = bucket_shard(h, k, r);
+          a.stage[r] = h->peer_stage[r]; a.b4[r] = bs.b / 4; a.e4[r] = bs.e / 4;
+          a.pre4 = bs.pre / 4;
+        }
+        a.stride4 = stride / 4; a.ctl4 = (h->P + 1024) / 4; a.bucket = k;
+        dp_fused_exchange(st, h->peers, a, h->m, h->v, h->d_sc, last ? h->d_loss_total : nullptr, ctas);
+        stamp(10 + 4 * k, st);
+        if (h->bf16mode) {
+          const size_t b0 = h->bucket_off[k], nn = h->bucket_off[k + 1] - b0;
+          split_bf16(st, h->w + b0, nn, h->w_hi + b0, h->w_lo + b0);
+        }
+        stamp(11 + 4 * k, st);
+      };
+      stamp(0, h->stream);
+      enqueue_forward(h, split, B, l, true);
+      stamp(1, h->stream);
+      enqueue_backward_seg(h, B, l, true, 1);
+      stamp(2, h->stream);
+      cudaEventRecord(h->ev_seg[0], h->stream);
+      cudaStreamWaitEvent(h->comm_stream, h->ev_seg[0], 0);
+      exchange_bucket(0, h->comm_stream, 20 * 4, false);
+      enqueue_backward_seg(h, B, l, true, 2);
+      stamp(3, h->stream);
+      cudaEventRecord(h->ev_seg[1], h->stream);
+      cudaStreamWaitEvent(h->comm_stream, h->ev_seg[1], 0);
+      exchange_bucket(1, h->comm_stream, 20 * 4, false);
+      enqueue_backward_seg(h, B, l, true, 31);
+      stamp(4, h->stream);
+      cudaEventRecord(h->ev_seg[2], h->stream);
+      cudaStreamWaitEvent(h->comm_stream, h->ev_seg[2], 0);
+      exchange_bucket(3, h->comm_stream, 148 * 4, false);
+      cudaEventRecord(h->ev_comm, h->comm_stream);
+      enqueue_backward_seg(h, B, l, true, 32);
+      stamp(5, h->stream);
+      exchange_bucket(2, h->stream, 148 * 4, true);
+      stamp(6, h->stream);
+      cudaStreamWaitEvent(h->stream, h->ev_comm, 0);  // join the side branch
+      stamp(7, h->stream);
     });
   }
   if (!h->comm) return fail(LRCN_ERR_ARG, "data-parallel group not initialised (lrcn_comm_init or lrcn_p2p_import)");
+  // NCCL: one allreduce over the whole gradient arena after the backward pass (no overlap, but no SM contention between the
+  // NCCL kernels and the persistent GEMM / LSTM kernels either)
   NcclApi* n = nccl_api();
-  static const bool bucketed = getenv("LRCN_DP_BUCKETS") != nullptr;  // measured: one allreduce after the backward pass beats 3 overlapped buckets
-  if (!bucketed) {
-    // one allreduce over the whole gradient arena after the backward pass (no overlap, but no SM contention between the NCCL
-    // kernels and the persistent GEMM / LSTM kernels either)
-    rc = run_cached(h, std::make_tuple(20, B, l, fl), [&] {
-      enqueue_forward(h, split, B, l, true);
-      for (int seg = 1; seg <= 3; seg++) enqueue_backward_seg(h, B, l, true, seg);
-    });
-    if (rc) return rc;
-    rc = nccl_check(n->GroupStart(), "ncclGroupStart"); if (rc) return rc;
-    rc = nccl_check(n->AllReduce(h->g, h->g, h->P, NCCL_FLOAT32, NCCL_SUM, h->comm, h->stream), "ncclAllReduce(grad)"); if (rc) return rc;
-    rc = nccl_check(n->AllReduce(h->d_loss, h->d_loss, 1, NCCL_FLOAT64, NCCL_SUM, h->comm, h->stream), "ncclAllReduce(loss)"); if (rc) return rc;
-    rc = nccl_check(n->GroupEnd(), "ncclGroupEnd"); if (rc) return rc;
-    if (mode == 2) {
-      rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h, false); });
-      if (rc) return rc;
-    }
-    return LRCN_OK;
-  }
-  // data-parallel: bucketed allreduce on the comm stream, overlapped with the remaining backward segments
-  rc = run_cached(h, std::make_tuple(10, B, l, fl), [&] { enqueue_forward(h, split, B, l, true); enqueue_backward_seg(h, B, l, true, 1); });
+  rc = run_cached(h, std::make_tuple(20, B, l, fl), [&] {
+    enqueue_forward(h, split, B, l, true);
+    for (int seg = 1; seg <= 3; seg++) enqueue_backward_seg(h, B, l, true, seg);
+  });
   if (rc) return rc;
-  for (int seg = 1; seg <= 3; seg++) {
-    CK(cudaEventRecord(h->ev_seg[seg - 1], h->stream));
-    CK(cudaStreamWaitEvent(h->comm_stream, h->ev_seg[seg - 1], 0));
-    float* gb = h->g + h->bucket_off[seg - 1];
-    size_t cnt = h->bucket_off[seg == 3 ? lrcn_handle::NBUCKET : seg] - h->bucket_off[seg - 1];  // the last allreduce takes (W1, b1) and Wemb
-    if (seg == 3) { rc = nccl_check(n->GroupStart(), "ncclGroupStart"); if (rc) return rc; }
-    rc = nccl_check(n->AllReduce(gb, gb, cnt, NCCL_FLOAT32, NCCL_SUM, h->comm, h->comm_stream), "ncclAllReduce(grad bucket)");
-    if (rc) return rc;
-    if (seg == 3) {
-      rc = nccl_check(n->AllReduce(h->d_loss, h->d_loss, 1, NCCL_FLOAT64, NCCL_SUM, h->comm, h->comm_stream), "ncclAllReduce(loss)");
-      if (rc) return rc;
-      rc = nccl_check(n->GroupEnd(), "ncclGroupEnd");
-      if (rc) return rc;
-    }
-    if (seg < 3) {
-      rc = run_cached(h, std::make_tuple(10 + seg, B, l, fl), [&] { enqueue_backward_seg(h, B, l, true, seg + 1); });
-      if (rc) return rc;
-    }
-  }
-  CK(cudaEventRecord(h->ev_comm, h->comm_stream));
-  CK(cudaStreamWaitEvent(h->stream, h->ev_comm, 0));
+  rc = nccl_check(n->GroupStart(), "ncclGroupStart"); if (rc) return rc;
+  rc = nccl_check(n->AllReduce(h->g, h->g, h->P, NCCL_FLOAT32, NCCL_SUM, h->comm, h->stream), "ncclAllReduce(grad)"); if (rc) return rc;
+  rc = nccl_check(n->AllReduce(h->d_loss, h->d_loss, 1, NCCL_FLOAT64, NCCL_SUM, h->comm, h->stream), "ncclAllReduce(loss)"); if (rc) return rc;
+  rc = nccl_check(n->GroupEnd(), "ncclGroupEnd"); if (rc) return rc;
   if (mode == 2) {
     rc = run_cached(h, std::make_tuple(14, 0, 0, 0), [&] { enqueue_adam(h, false); });
     if (rc) return rc;
@@ -1626,7 +1456,7 @@ static int s_p2p_import(lrcn_handle* h, const char* blobs, int rank, int nranks)
   h->peers = pe;
   h->rank = rank; h->nranks = nranks;
   h->dp_epoch = 0;  // the fused exchange's flags / counters count the group's data-parallel steps: start them together
-  CK(cudaMemset(h->stage + h->P + 1024, 0, (DP_XCTL_FLOATS + 2 * h->ll_floats) * 4));
+  CK(cudaMemset(h->stage + h->P + 1024, 0, DP_XCTL_FLOATS * 4));
   h->p2p_ready = true;
   return LRCN_OK;
 }

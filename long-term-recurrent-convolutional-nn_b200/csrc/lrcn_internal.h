@@ -103,16 +103,11 @@ struct lrcn_handle {
   float* peer_m[LRCN_P2P_MAX_RANKS] = {};
   float* peer_v[LRCN_P2P_MAX_RANKS] = {};
   bool adam_sharded = false;          // m, v are current only in each owner's shard (gathered on lrcn_get_adam_state)
-  // copy-engine exchange (dp_p2p.cu): staging rows for the gradient slices the peers push to this rank, and the peers' rows
+  // fused exchange (dp_p2p.cu): staging rows for the gradient chunks the peers push to this rank, followed by the control
+  // words (chunk flags, completion counters); and the peers' staging allocations
   float* stage = nullptr;
   float* peer_stage[LRCN_P2P_MAX_RANKS] = {};
-  size_t ll_floats = 0;               // floats of each of the two LL areas (gradient lines, weight lines) behind the control words of `stage`
   unsigned int dp_epoch = 0;          // data-parallel train steps run since the peer group was formed (the fused exchange's flag value)
-  bool shard_by_bucket = false;       // how the last sharded step split the arena: per gradient bucket (copy engines) or as a whole
-  unsigned int* d_epoch_side = nullptr;  // epoch counter of the side-stream barriers
-  static constexpr int NXFER = 4;        // parallel copy branches (so that several DMA engines work on the N-1 slices of a phase)
-  cudaStream_t xfer[NXFER] = {};
-  cudaEvent_t ev_xfork = nullptr, ev_xjoin[NXFER] = {};
   unsigned int* d_counters = nullptr;  // per-m-tile grid-barrier counters of the persistent LSTM kernels
   unsigned long long* d_trace = nullptr;  // LRCN_SEQ_TRACE=1: per-step timeline of the layer-2 forward sequence kernel
   Slot slots[64];

@@ -39,10 +39,8 @@ t = raw.astype(np.int64)
 names = {0: "step start", 1: "forward done", 2: "seg1 (vocab bwd) done", 3: "seg2 (layer-2 bwd) done", 4: "seg31 (L1 BPTT + dWemb) done", 5: "seg32 (dW1) done",
          6: "last exchange done", 7: "joined"}
 for k, nm in enumerate(["bucket0 Wout", "bucket1 W2..", "bucket2 W1 (main)", "bucket3 Wemb"]):
-    for j, ph in enumerate(["enter", "barrier1 passed", "exchange kernel done", "barrier2+split done"]):
+    for j, ph in ((0, "enter"), (2, "exchange kernel done"), (3, "bf16 split done")):
         names[8 + 4 * k + j] = f"{nm}: {ph}"
-for k in range(4):
-    names[32 + k] = f"bucket{k}: first barrier KERNEL STARTED"
 if rank == 0:
     for i in sorted(names, key=lambda i: t[i]):
         if t[i]:
