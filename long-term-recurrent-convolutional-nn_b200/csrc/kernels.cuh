@@ -162,29 +162,31 @@ struct ZeroSegs { float* p[16]; size_t n[16]; int count = 0; void add(void* ptr,
 void zero_multi(cudaStream_t s, const ZeroSegs& z);
 
 // ---------------------------------------------------------------- beam search
-// per row: prob = exp(logp(a)); top-K by (prob desc, index asc); cand_* are [R][K]
+// per row: prob = exp(logp(a)); top-K by (prob desc, index asc); cand_* are [R][K].  Needs 1 <= K <= TOPK_MAXK (11):
+// lrcn_beam_search and the test hooks reject larger beam widths before any launch.
 void beam_row_topk(cudaStream_t s, const float* logits, int ld, int R, int V, int K, const float* parent_prob,
                    int* cand_tok, float* cand_score, float* cand_lp);
+// the same on given probabilities (test hook only)
 void beam_row_topk_probs(cudaStream_t s, const float* probs, int ld, int R, int V, int K, const float* parent_prob,
                          int* cand_tok, float* cand_score, float* cand_lp);
-// per image: pick K of the K*K (K at the first step) candidates by (score desc, list position asc)
+// per image: pick K of the K*K (K at the first step) candidates by (score desc, list position asc).  Only the test hook calls
+// it; in a decode step beam_advance makes the same picks with the same device code.
 void beam_select(cudaStream_t s, const int* cand_tok, const float* cand_score, const float* cand_lp, int n_img, int K,
                  int first_step, int* sel_tok, int* sel_parent, float* sel_score, float* sel_lp);
 struct BeamAdvanceArgs {
   int n_img, K, H1, H2, maxlen, step, nword;
   int ld1, ld2;  // row pitch of h1_out / h2_out (they are the h-columns of the [x|h] GEMM operand buffers)
-  const int* sel_tok; const int* sel_parent; const float* sel_score; const float* sel_lp;
   const float *h1_in, *c1_in, *h2_in, *c2_in; float *h1_out, *c1_out, *h2_out, *c2_out;
   const int* hist_in; int* hist_out; const float* lp_in; float* lp_out;
   __nv_bfloat16 *h1_hi, *h1_lo, *h2_hi, *h2_lo;  // optional bf16 split of the gathered h states (null in fp32 mode)
   float* prob; int* last_tok; int* done; int* n_done;
   long long* out_tokens; int* out_len; float* out_prob; float* out_lp;
   const int* out_map;  // compacted image index -> image index of the caller's chunk (outputs are written there); null = identity
-  // fused = 1: the row's CTA also does the image's stable selection over the K*K candidates (beam_select_kernel's job) and the
-  // k = 0 row marks the image done (beam_mark_done_kernel's job): one launch per step instead of three
-  int fused;
+  // the row's CTA picks its candidate by the image's stable selection over the K*K candidates (K at the first step), and the
+  // k = 0 row marks the image done: one launch per decode step does all its bookkeeping
   const int* cand_tok; const float* cand_score; const float* cand_lp;
-  // fused: the row also gathers the embedding of its new token -- the next step's x operand (gather_embed_kernel's job, lrcn.jl:650)
+  // the row also gathers the embedding of its new token -- the next step's x operand (gather_embed_kernel's job, lrcn.jl:650);
+  // skipped when wemb is null
   const float* wemb; float* e_out; __nv_bfloat16 *e_hi, *e_lo; int E, lde;
 };
 void beam_advance(cudaStream_t s, const BeamAdvanceArgs& a);

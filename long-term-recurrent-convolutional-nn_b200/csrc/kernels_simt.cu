@@ -1023,36 +1023,7 @@ void fill_l2_scratch(cudaStream_t s, float* buf, size_t n, float val) {
 // ------------------------------------------------------------------------------------------
 // beam search (lrcn.jl:644-678): fp32 probabilities exp(logp), ties -> lower index
 // ------------------------------------------------------------------------------------------
-struct BestPair { float v; int i; };
-__device__ __forceinline__ BestPair better(BestPair a, BestPair b) {
-  return (b.v > a.v || (b.v == a.v && b.i < a.i)) ? b : a;
-}
-__device__ __forceinline__ BestPair block_argmax(BestPair p, BestPair* red) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    BestPair q;
-    q.v = __shfl_xor_sync(0xffffffffu, p.v, o);
-    q.i = __shfl_xor_sync(0xffffffffu, p.i, o);
-    p = better(p, q);
-  }
-  int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = blockDim.x >> 5;
-  __syncthreads();
-  if (l == 0) red[w] = p;
-  __syncthreads();
-  BestPair q;
-  q.v = -2.f; q.i = 0x7fffffff;
-  if (l < nw) q = red[l];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    BestPair t;
-    t.v = __shfl_xor_sync(0xffffffffu, q.v, o);
-    t.i = __shfl_xor_sync(0xffffffffu, q.i, o);
-    q = better(q, t);
-  }
-  return q;
-}
-
-constexpr int TOPK_MAX = 11;
+constexpr int TOPK_MAXK = 11;  // largest beam width: lrcn_beam_search and the test hooks reject K > 11 before any launch
 constexpr int TOPK_CAP = 256;  // candidate list capacity of the threshold-select path
 struct TopPair { float v; int i; };
 __device__ __forceinline__ TopPair top_better(TopPair a, TopPair b) { return (b.v > a.v || (b.v == a.v && b.i < a.i)) ? b : a; }
@@ -1081,117 +1052,20 @@ __device__ __forceinline__ TopPair block_top(TopPair p, TopPair* red) {
 
 // per row: probabilities ynorm = exp(logp(ypred,2)) (fp32, lrcn.jl:652-654) and the K largest by (prob desc, index asc)
 // (lrcn.jl:655-656: sortperm(rev=true) breaks ties by index).  Threshold select:
-//   1. the row is staged once in shared memory; max and normaliser by block reductions (the normaliser uses __expf: its ~1e-7
-//      relative error shifts every probability of the row alike, so no ordering changes);
+//   1. the row is staged once in shared memory (40 KB at V = 10000, so 4 CTAs share an SM); max and normaliser come from ONE
+//      block reduction of per-thread (max, sum exp) pairs (the normaliser uses __expf: its ~1e-7 relative error shifts every
+//      probability of the row alike, so no ordering changes);
 //   2. tau = K-th largest of the per-thread maxima is a lower bound of the K-th largest element, so every top-K element is >= tau;
+//      it comes from per-warp top-K lists of the thread maxima, so a row costs 4 block barriers;
 //   3. the (few) elements >= tau are appended to a candidate list; one warp evaluates their precise probabilities and picks the
 //      K best by (prob desc, index asc).  Ties at tau are all candidates, so selection on given probabilities is exact.
 //   A row with more than TOPK_CAP candidates (e.g. all-equal logits) falls back to K exact block-argmax rounds.
 template <bool FROM_LOGITS>
-__global__ void __launch_bounds__(512) beam_row_topk_kernel(const float* __restrict__ in, int ld, int R, int V, int K,
-                                                            const float* __restrict__ parent_prob, int* __restrict__ cand_tok,
-                                                            float* __restrict__ cand_score, float* __restrict__ cand_lp) {
-  extern __shared__ __align__(16) float row[];  // V values (logits, or the given probabilities)
-  __shared__ float red[32];
-  __shared__ TopPair pred[32];
-  __shared__ float cv[TOPK_CAP];
-  __shared__ int ci[TOPK_CAP];
-  __shared__ int ccount;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int r = blockIdx.x; r < R; r += gridDim.x) {  // persistent over rows
-    const float* a = in + (size_t)r * ld;
-    __syncthreads();  // previous row's shared state is no longer read
-    if (threadIdx.x == 0) ccount = 0;
-    float tmax = -INFINITY;
-    const int V4 = ((reinterpret_cast<uintptr_t>(a) & 15) == 0) ? (V >> 2) : 0;
-    for (int q = threadIdx.x; q < V4; q += blockDim.x) {
-      const float4 x = *reinterpret_cast<const float4*>(a + 4 * q);
-      *reinterpret_cast<float4*>(row + 4 * q) = x;
-      tmax = fmaxf(fmaxf(tmax, fmaxf(x.x, x.y)), fmaxf(x.z, x.w));
-    }
-    for (int j = 4 * V4 + threadIdx.x; j < V; j += blockDim.x) { const float x = a[j]; row[j] = x; tmax = fmaxf(tmax, x); }
-    float lse = 0.f, mx = 0.f;
-    if (FROM_LOGITS) {
-      mx = block_max(tmax, red);
-      float sum = 0.f;
-      for (int j = threadIdx.x; j < V; j += blockDim.x) sum += __expf(row[j] - mx);
-      sum = block_sum(sum, red);
-      lse = logf(sum);
-    }
-    // tau: K-th largest of the thread maxima (each thread covered a disjoint set of elements)
-    float mine = tmax, tau = 0.f;
-    for (int k = 0; k < K; k++) {
-      TopPair p; p.v = mine; p.i = threadIdx.x;
-      p = block_top(p, pred);
-      tau = p.v;
-      if (p.i == (int)threadIdx.x) mine = -INFINITY;
-    }
-    __syncthreads();
-    for (int j = threadIdx.x; j < V; j += blockDim.x) {
-      const float x = row[j];
-      if (x >= tau) {
-        const int pos = atomicAdd(&ccount, 1);
-        if (pos < TOPK_CAP) { cv[pos] = x; ci[pos] = j; }
-      }
-    }
-    __syncthreads();
-    const int nc = ccount;
-    const float pp = parent_prob[r];
-    if (nc <= TOPK_CAP) {
-      if (warp == 0) {
-        constexpr int PER = TOPK_CAP / 32;
-        float pv[PER]; int pi[PER];
-#pragma unroll
-        for (int q = 0; q < PER; q++) {
-          const int c = lane + 32 * q;
-          pv[q] = -INFINITY; pi[q] = 0x7fffffff;
-          if (c < nc) { const float x = cv[c]; pv[q] = FROM_LOGITS ? expf((x - mx) - lse) : x; pi[q] = ci[c]; }
-        }
-        for (int k = 0; k < K; k++) {
-          TopPair best; best.v = -INFINITY; best.i = 0x7fffffff;
-#pragma unroll
-          for (int q = 0; q < PER; q++) { TopPair c; c.v = pv[q]; c.i = pi[q]; best = top_better(best, c); }
-          best = warp_top(best);
-#pragma unroll
-          for (int q = 0; q < PER; q++) if (pi[q] == best.i) { pv[q] = -INFINITY; pi[q] = 0x7fffffff; }  // indices are unique
-          if (lane == 0) {
-            cand_tok[(size_t)r * K + k] = best.i;
-            cand_score[(size_t)r * K + k] = __fmul_rn(best.v, pp);  // pmaxes = ynorm[xmaxes]*current_probability (lrcn.jl:657)
-            cand_lp[(size_t)r * K + k] = FROM_LOGITS ? ((row[best.i] - mx) - lse) : logf(best.v);
-          }
-        }
-      }
-    } else {
-      // exact fallback: K rounds of block argmax over the whole row on the probabilities themselves
-      if (FROM_LOGITS) {
-        __syncthreads();
-        for (int j = threadIdx.x; j < V; j += blockDim.x) row[j] = expf((row[j] - mx) - lse);
-      }
-      for (int k = 0; k < K; k++) {
-        __syncthreads();
-        TopPair p; p.v = -INFINITY; p.i = 0x7fffffff;
-        for (int j = threadIdx.x; j < V; j += blockDim.x) { TopPair c; c.v = row[j]; c.i = j; p = top_better(p, c); }
-        p = block_top(p, pred);
-        if (threadIdx.x == 0) {
-          cand_tok[(size_t)r * K + k] = p.i;
-          cand_score[(size_t)r * K + k] = __fmul_rn(p.v, pp);
-          cand_lp[(size_t)r * K + k] = logf(p.v);
-          row[p.i] = -1.f;  // exclude from later rounds
-        }
-      }
-    }
-  }
-}
-// Second-generation threshold select.  Like beam_row_topk_kernel the row is staged once in shared memory (40 KB at V = 10000,
-// so 4 CTAs share an SM), but max and normaliser come from ONE block reduction of per-thread (max, sum exp) pairs and tau from
-// per-warp top-K lists of the thread maxima: 4 block barriers per row instead of ~12.  Same results on given probabilities.
-constexpr int TOPK_MAXK = 11;
-template <bool FROM_LOGITS, int THREADS>
-__global__ void __launch_bounds__(THREADS) beam_row_topk2_kernel(const float* __restrict__ in, int ld, int R, int V, int K,
+__global__ void __launch_bounds__(256) beam_row_topk2_kernel(const float* __restrict__ in, int ld, int R, int V, int K,
                                                              const float* __restrict__ parent_prob, int* __restrict__ cand_tok,
                                                              float* __restrict__ cand_score, float* __restrict__ cand_lp) {
   extern __shared__ __align__(16) float row[];
-  constexpr int NW = THREADS / 32;
+  constexpr int THREADS = 256, NW = THREADS / 32;
   __shared__ float2 wred[NW];
   __shared__ float wtop[NW][TOPK_MAXK + 1];
   __shared__ float cv[TOPK_CAP];
@@ -1343,7 +1217,7 @@ __global__ void __launch_bounds__(THREADS) beam_row_topk2_kernel(const float* __
     }
   }
 }
-// Third generation: the row lives in REGISTERS (NV4 float4 per thread, every load of the row in flight at once), shared memory
+// topk2's threshold select with the row in REGISTERS (NV4 float4 per thread, every load of the row in flight at once), shared memory
 // holds only the candidate list; the row is dumped to shared memory only for the exact fallback.  The shared-memory staging of
 // topk2 serialised a global round trip, three shared-memory passes and four block barriers per row with 4-5 CTAs per SM (0.30 of
 // HBM at V = 10000); here the passes run on registers.  Same arithmetic in the same order per element => same results.
@@ -1505,7 +1379,7 @@ __global__ void __launch_bounds__(256, 3) beam_row_topk3_kernel(const float* __r
     }
   }
 }
-// Fourth generation: ONE WARP PER ROW, one streaming pass, no shared memory and no block barrier.  topk2 / topk3 process a row per
+// ONE WARP PER ROW, one streaming pass, no shared memory and no block barrier.  topk2 / topk3 process a row per
 // CTA in phases separated by four block barriers with a serial last phase in warp 0: ~8 us of latency per row and 3 rows in
 // flight per SM = 0.33 of the HBM peak (ncu launch list: 56 us for 3072 x 10000 logits).  Here every lane streams its float4
 // columns (16 loads in flight per lane, 32 independent rows per SM), keeps an online (max, sum exp) pair and its own top-KM list
@@ -1599,68 +1473,68 @@ __global__ void __launch_bounds__(256) beam_row_topk4_kernel(const float* __rest
     }
   }
 }
+// One warp per row needs many rows to fill the machine (a lone warp streams a 40 KB row in ~20 us); below that the CTA-per-row
+// kernels are faster (measured: COCO-shaped decode, i.e. compacted batches, 157 k captions/s with topk4 everywhere vs 163 k).
+constexpr int TOPK4_MIN_ROWS = 2048;
 template <bool FROM_LOGITS>
-static void beam_topk4_launch(cudaStream_t s, const float* in, int ld, int R, int V, int K, const float* parent_prob, int* cand_tok, float* cand_score,
-                              float* cand_lp) {
-  const int want = (R + 7) / 8;
-  const int cap = 148 * 4;  // 48-64 registers per thread: four 256-thread CTAs per SM
-  const int grid = want < cap ? want : cap;
-  if (K <= 1) beam_row_topk4_kernel<FROM_LOGITS, 1, 8><<<grid, 256, 0, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-  else if (K <= 3) beam_row_topk4_kernel<FROM_LOGITS, 3, 8><<<grid, 256, 0, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-  else if (K <= 5) beam_row_topk4_kernel<FROM_LOGITS, 5, 8><<<grid, 256, 0, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-  else beam_row_topk4_kernel<FROM_LOGITS, TOPK_MAXK, 4><<<grid, 256, 0, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-  count_launch();
-}
-static void beam_topk_launch(cudaStream_t s, bool from_logits, const float* in, int ld, int R, int V, int K,
-                             const float* parent_prob, int* cand_tok, float* cand_score, float* cand_lp) {
+static void beam_topk2_launch(cudaStream_t s, const float* in, int ld, int R, int V, int K, const float* parent_prob, int* cand_tok,
+                              float* cand_score, float* cand_lp) {
   const size_t smem = ((size_t)V + 4) * sizeof(float);
-  const int grid = R < 148 * 4 ? R : 148 * 4;
-  static const bool v1 = getenv("LRCN_TOPK_V1") != nullptr;
-  static const bool no_v4 = getenv("LRCN_TOPK_V3") != nullptr || getenv("LRCN_TOPK_V2") != nullptr;
-  // one warp per row needs many rows to fill the machine (a lone warp streams a 40 KB row in ~20 us); below that the CTA-per-row
-  // kernels are faster (measured: COCO-shaped decode, i.e. compacted batches, 157 k captions/s with topk4 everywhere vs 163 k)
-  static const int v4_rows = getenv("LRCN_TOPK_V4_ROWS") ? atoi(getenv("LRCN_TOPK_V4_ROWS")) : 2048;
-  if (!v1 && !no_v4 && R >= v4_rows && K <= TOPK_MAXK && V % 4 == 0 && ld % 4 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && V >= 128) {
-    if (from_logits) beam_topk4_launch<true>(s, in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    else beam_topk4_launch<false>(s, in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    return;
-  }
-  static const bool no_v3 = getenv("LRCN_TOPK_V2") != nullptr;
-  constexpr int NV4 = 11;  // V <= 11264 (COCO: 10000 / 10636)
-  if (!v1 && !no_v3 && K <= TOPK_MAXK && V % 4 == 0 && ld % 4 == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0 && V > 4096 && V <= 4 * 256 * NV4) {
-    const int g3 = R < 148 * 3 ? R : 148 * 3;  // 3 CTAs per SM (registers)
-    if (from_logits) beam_row_topk3_kernel<true, NV4><<<g3, 256, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    else beam_row_topk3_kernel<false, NV4><<<g3, 256, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    count_launch();
-    return;
-  }
-  if (!v1 && K <= TOPK_MAXK) {
-    static const int th = getenv("LRCN_TOPK_THREADS") ? atoi(getenv("LRCN_TOPK_THREADS")) : 256;
-    const int g2 = R < 148 * 8 ? R : 148 * 8;
-    if (th == 512) {
-      if (from_logits) beam_row_topk2_kernel<true, 512><<<grid, 512, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-      else beam_row_topk2_kernel<false, 512><<<grid, 512, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    } else {
-      if (from_logits) beam_row_topk2_kernel<true, 256><<<g2, 256, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-      else beam_row_topk2_kernel<false, 256><<<g2, 256, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-    }
-    count_launch();
-    return;
-  }
-  if (from_logits) beam_row_topk_kernel<true><<<grid, 512, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
-  else beam_row_topk_kernel<false><<<grid, 512, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+  const int grid = R < 148 * 8 ? R : 148 * 8;
+  beam_row_topk2_kernel<FROM_LOGITS><<<grid, 256, smem, s>>>(in, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
   count_launch();
 }
 void beam_row_topk(cudaStream_t s, const float* logits, int ld, int R, int V, int K, const float* parent_prob, int* cand_tok,
                    float* cand_score, float* cand_lp) {
-  beam_topk_launch(s, true, logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+  const bool vec4 = V % 4 == 0 && ld % 4 == 0 && (reinterpret_cast<uintptr_t>(logits) & 15) == 0;  // float4 rows: topk3 / topk4
+  if (vec4 && R >= TOPK4_MIN_ROWS && V >= 128) {
+    const int want = (R + 7) / 8;
+    const int cap = 148 * 4;  // 48-64 registers per thread: four 256-thread CTAs per SM
+    const int grid = want < cap ? want : cap;
+    if (K <= 1) beam_row_topk4_kernel<true, 1, 8><<<grid, 256, 0, s>>>(logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+    else if (K <= 3) beam_row_topk4_kernel<true, 3, 8><<<grid, 256, 0, s>>>(logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+    else if (K <= 5) beam_row_topk4_kernel<true, 5, 8><<<grid, 256, 0, s>>>(logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+    else beam_row_topk4_kernel<true, TOPK_MAXK, 4><<<grid, 256, 0, s>>>(logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+    count_launch();
+    return;
+  }
+  constexpr int NV4 = 11;  // V <= 11264 (COCO: 10000 / 10636)
+  if (vec4 && V > 4096 && V <= 4 * 256 * NV4) {
+    const size_t smem = ((size_t)V + 4) * sizeof(float);
+    const int grid = R < 148 * 3 ? R : 148 * 3;  // 3 CTAs per SM (registers)
+    beam_row_topk3_kernel<true, NV4><<<grid, 256, smem, s>>>(logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+    count_launch();
+    return;
+  }
+  beam_topk2_launch<true>(s, logits, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
 }
 void beam_row_topk_probs(cudaStream_t s, const float* probs, int ld, int R, int V, int K, const float* parent_prob,
                          int* cand_tok, float* cand_score, float* cand_lp) {
-  beam_topk_launch(s, false, probs, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
+  beam_topk2_launch<false>(s, probs, ld, R, V, K, parent_prob, cand_tok, cand_score, cand_lp);
 }
 
-// one thread per image: stable descending selection over the candidate list (beam-major, rank-minor)
+// The image's stable selection (lrcn.jl:667-668) over the ncand scores of its candidate list (beam-major, rank-minor): k+1
+// rounds of "best unused candidate"; returns the last one, i.e. the (k+1)-th best.  Strict '>' keeps the earlier list position
+// on ties.
+struct BeamPick { int c; float v; };
+__device__ __forceinline__ BeamPick beam_pick(const float* sc, int ncand, int k) {
+  unsigned long long used_lo = 0, used_hi = 0;  // K*K <= 128 candidates
+  int best = -1;
+  float bv = 0.f;
+  for (int kk = 0; kk <= k; kk++) {
+    best = -1; bv = 0.f;
+    for (int c = 0; c < ncand; c++) {
+      const bool used = c < 64 ? ((used_lo >> c) & 1ull) : ((used_hi >> (c - 64)) & 1ull);
+      if (used) continue;
+      const float v = sc[c];
+      if (best < 0 || v > bv) { best = c; bv = v; }
+    }
+    if (best < 64) used_lo |= 1ull << best; else used_hi |= 1ull << (best - 64);
+  }
+  return {best, bv};
+}
+
+// one thread per image: all K picks of beam_pick (beam_advance_kernel makes the same picks in the decode step)
 __global__ void beam_select_kernel(const int* __restrict__ cand_tok, const float* __restrict__ cand_score,
                                    const float* __restrict__ cand_lp, int n_img, int K, int first_step, int* __restrict__ sel_tok,
                                    int* __restrict__ sel_parent, float* __restrict__ sel_score, float* __restrict__ sel_lp) {
@@ -1668,22 +1542,13 @@ __global__ void beam_select_kernel(const int* __restrict__ cand_tok, const float
   if (img >= n_img) return;
   int ncand = first_step ? K : K * K;
   const float* sc = cand_score + (size_t)img * K * K;
-  unsigned long long used_lo = 0, used_hi = 0;  // K*K <= 128 candidates
   for (int k = 0; k < K; k++) {
-    int best = -1;
-    float bv = 0.f;
-    for (int c = 0; c < ncand; c++) {
-      bool used = c < 64 ? ((used_lo >> c) & 1ull) : ((used_hi >> (c - 64)) & 1ull);
-      if (used) continue;
-      float v = sc[c];
-      if (best < 0 || v > bv) { best = c; bv = v; }  // strict > keeps the earlier list position on ties
-    }
-    if (best < 64) used_lo |= 1ull << best; else used_hi |= 1ull << (best - 64);
+    const BeamPick p = beam_pick(sc, ncand, k);
     size_t o = (size_t)img * K + k;
-    sel_tok[o] = cand_tok[(size_t)img * K * K + best];
-    sel_parent[o] = best / K;  // ceil((best+1)/K) - 1  (lrcn.jl:675)
-    sel_score[o] = bv;
-    sel_lp[o] = cand_lp[(size_t)img * K * K + best];
+    sel_tok[o] = cand_tok[(size_t)img * K * K + p.c];
+    sel_parent[o] = p.c / K;  // ceil((best+1)/K) - 1  (lrcn.jl:675)
+    sel_score[o] = p.v;
+    sel_lp[o] = cand_lp[(size_t)img * K * K + p.c];
   }
 }
 void beam_select(cudaStream_t s, const int* cand_tok, const float* cand_score, const float* cand_lp, int n_img, int K,
@@ -1693,40 +1558,21 @@ void beam_select(cudaStream_t s, const int* cand_tok, const float* cand_score, c
   count_launch();
 }
 
-// one CTA per (image, beam) row: reorder/gather the advanced states of the parents, extend histories,
-// detect termination (best hypothesis ends in eos, or step > nword: lrcn.jl:670) and emit results.
+// one CTA per (image, beam) row: select the row's candidate, reorder/gather the advanced states of the parents, extend
+// histories, gather the next step's input embedding, detect termination (best hypothesis ends in eos, or step > nword:
+// lrcn.jl:670), emit results and mark the image done.
 __global__ void __launch_bounds__(128) beam_advance_kernel(BeamAdvanceArgs a) {
   int r = blockIdx.x;
   int img = r / a.K, k = r - img * a.K;
-  if (a.done[img]) return;  // (fused: the k = 0 row of this launch may set the flag meanwhile -- either outcome is fine, the image is frozen from here on)
+  if (a.done[img]) return;  // (the k = 0 row of this launch may set the flag meanwhile -- either outcome is fine, the image is frozen from here on)
   __shared__ int s_tok, s_par;
   __shared__ float s_score, s_lp;
-  if (a.fused) {
-    // the image's selection, as beam_select_kernel does it: k+1 rounds of "best unused candidate", strict '>' keeps the earlier
-    // list position (beam-major, rank-minor) on ties; this row takes the (k+1)-th
-    if (threadIdx.x == 0) {
-      const int ncand = a.step == 1 ? a.K : a.K * a.K;
-      const float* sc = a.cand_score + (size_t)img * a.K * a.K;
-      unsigned long long used_lo = 0, used_hi = 0;  // K*K <= 128 candidates
-      int best = -1;
-      float bv = 0.f;
-      for (int kk = 0; kk <= k; kk++) {
-        best = -1; bv = 0.f;
-        for (int c = 0; c < ncand; c++) {
-          const bool used = c < 64 ? ((used_lo >> c) & 1ull) : ((used_hi >> (c - 64)) & 1ull);
-          if (used) continue;
-          const float v = sc[c];
-          if (best < 0 || v > bv) { best = c; bv = v; }
-        }
-        if (best < 64) used_lo |= 1ull << best; else used_hi |= 1ull << (best - 64);
-      }
-      s_tok = a.cand_tok[(size_t)img * a.K * a.K + best];
-      s_par = best / a.K;  // ceil((best+1)/K) - 1  (lrcn.jl:675)
-      s_score = bv;
-      s_lp = a.cand_lp[(size_t)img * a.K * a.K + best];
-    }
-  } else if (threadIdx.x == 0) {
-    s_tok = a.sel_tok[r]; s_par = a.sel_parent[r]; s_score = a.sel_score[r]; s_lp = a.sel_lp[r];
+  if (threadIdx.x == 0) {  // this row takes the image's (k+1)-th pick
+    const BeamPick p = beam_pick(a.cand_score + (size_t)img * a.K * a.K, a.step == 1 ? a.K : a.K * a.K, k);
+    s_tok = a.cand_tok[(size_t)img * a.K * a.K + p.c];
+    s_par = p.c / a.K;  // ceil((best+1)/K) - 1  (lrcn.jl:675)
+    s_score = p.v;
+    s_lp = a.cand_lp[(size_t)img * a.K * a.K + p.c];
   }
   __syncthreads();
   int parent = img * a.K + s_par;
@@ -1766,7 +1612,7 @@ __global__ void __launch_bounds__(128) beam_advance_kernel(BeamAdvanceArgs a) {
     a.lp_out[(size_t)r * a.maxlen + j] = a.lp_in[(size_t)parent * a.maxlen + j];
   }
   int tok = s_tok;
-  if (a.fused && a.wemb) {  // the next step's input embedding Wemb[tok,:] (+ its bf16 split)
+  if (a.wemb) {  // the next step's input embedding Wemb[tok,:] (+ its bf16 split)
     const float* src = a.wemb + (size_t)tok * a.E;
     if (vec) {
       for (int q = threadIdx.x; q < (a.E >> 2); q += blockDim.x) {
@@ -1800,20 +1646,10 @@ __global__ void __launch_bounds__(128) beam_advance_kernel(BeamAdvanceArgs a) {
       if (threadIdx.x == 0) {
         a.out_len[oimg] = total;
         a.out_prob[oimg] = s_score;
-        if (a.fused) { a.done[img] = 1; atomicAdd(a.n_done, 1); }
+        a.done[img] = 1;
+        atomicAdd(a.n_done, 1);
       }
     }
-  }
-}
-// second tiny kernel marks images done AFTER all K rows of the step were advanced (avoids a race on done[])
-__global__ void beam_mark_done_kernel(const int* __restrict__ sel_tok, int n_img, int K, int step, int nword, int* __restrict__ done,
-                                      int* __restrict__ n_done) {
-  int img = blockIdx.x * blockDim.x + threadIdx.x;
-  if (img >= n_img || done[img]) return;
-  int tok = sel_tok[(size_t)img * K];
-  if (tok == 0 || step > nword) {
-    done[img] = 1;
-    atomicAdd(n_done, 1);
   }
 }
 __global__ void __launch_bounds__(128) beam_compact_gather_kernel(BeamCompactArgs a) {
@@ -1897,9 +1733,6 @@ void beam_compact(cudaStream_t s, const BeamCompactArgs& a) {
 void beam_advance(cudaStream_t s, const BeamAdvanceArgs& a) {
   beam_advance_kernel<<<a.n_img * a.K, 128, 0, s>>>(a);
   count_launch();
-  if (a.fused) return;
-  beam_mark_done_kernel<<<(a.n_img + 127) / 128, 128, 0, s>>>(a.sel_tok, a.n_img, a.K, a.step, a.nword, a.done, a.n_done);
-  count_launch();
 }
 
 // called once per process from lrcn_create (never inside a stream capture)
@@ -1909,12 +1742,8 @@ void init_simt_kernels() {
   cudaFuncSetAttribute(softmax_ce_fused_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
   cudaFuncSetAttribute(softmax_ce_fused_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024);
   cudaFuncSetAttribute(softmax_ce_fused_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024);
-  cudaFuncSetAttribute(beam_row_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(beam_row_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(beam_row_topk2_kernel<true, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(beam_row_topk2_kernel<false, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(beam_row_topk2_kernel<true, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  cudaFuncSetAttribute(beam_row_topk2_kernel<false, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaFuncSetAttribute(beam_row_topk2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  cudaFuncSetAttribute(beam_row_topk2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 }
 
 }  // namespace lrcn

@@ -164,7 +164,7 @@ static int s_destroy(lrcn_handle* h) {
   if (!h->peers_direct) for (void* q : h->p2p_opened) if (q) cudaIpcCloseMemHandle(q);
   for (cudaEvent_t e : h->sc_ev) if (e) cudaEventDestroy(e);
   void* ptrs[] = {h->w, h->g, h->m, h->v, h->w_hi, h->w_lo, h->wp1_hi, h->wp1_lo, h->wp2_hi, h->wp2_lo, h->wt1_hi, h->wt1_lo, h->wt2_hi, h->wt2_lo, h->tab[0].d, h->tab[1].d, h->ws.f, h->ws.hi, h->ws.lo, h->d_tok_in,
-                  h->d_tok_tgt, h->d_rows, h->d_sc, h->p2p_ctl, h->d_loss_total, h->d_epoch, h->stage, h->d_counters, h->d_trace, h->g_last, h->g_ctok, h->g_stok, h->g_spar, h->g_hista, h->g_histb,
+                  h->d_tok_tgt, h->d_rows, h->d_sc, h->p2p_ctl, h->d_loss_total, h->d_epoch, h->stage, h->d_counters, h->d_trace, h->g_last, h->g_ctok, h->g_stok, h->g_hista, h->g_histb,
                   h->g_done, h->g_ndone, h->g_olen, h->g_rows, h->g_otok, h->l2_scratch, h->g_keep, h->g_omap, h->g_omap_s, h->d_gnorm};
   for (void* p : ptrs) if (p) cudaFree(p);
   for (void* q : {(void*)h->ep_seq, (void*)h->ep_ids, (void*)h->ep_rows, (void*)h->ep_loss, (void*)h->ep_err, (void*)h->tab[0].d_ids, (void*)h->tab[0].d_rowof,
@@ -281,7 +281,7 @@ static int create_impl(const lrcn_config* cfg, lrcn_handle* h) {
   o.gh1a = a.take(G * H1); o.gc1a = a.take(G * H1); o.gh1b = a.take(G * H1); o.gc1b = a.take(G * H1);
   o.gz = a.take(G * 2 * C); o.gg2 = a.take(G * 4 * H2);
   o.gh2a = a.take(G * H2); o.gc2a = a.take(G * H2); o.gh2b = a.take(G * H2); o.gc2b = a.take(G * H2);
-  o.glogits = a.take(G * ldV); o.gprob = a.take(G); o.gcs = a.take(G * 16); o.gclp = a.take(G * 16); o.gss = a.take(G); o.gslp = a.take(G);
+  o.glogits = a.take(G * ldV); o.gprob = a.take(G); o.gcs = a.take(G * 16); o.gclp = a.take(G * 16); o.gss = a.take(G);  // gss, g_stok: beam-compaction scratch (prob_s, last_s)
   o.glpa = a.take(G * ML); o.glpb = a.take(G * ML); o.goprob = a.take(G); o.golp = a.take(G * ML);
   o.gxh1 = a.take(G * (E + H1)); o.gxh2 = a.take(G * (2 * C + H2));  // [x|h] operands of the wide (many-row) generation path
   a.cap = a.used;
@@ -306,7 +306,7 @@ static int create_impl(const lrcn_config* cfg, lrcn_handle* h) {
   CK(cudaMalloc(&h->d_counters, 320 * sizeof(unsigned int)));  // [0,256): 4 LSTM launches x 64 (half-)tile barriers; [256,..): softmax
   CK(cudaMemset(h->d_counters, 0, 320 * sizeof(unsigned int)));
   if (getenv("LRCN_SEQ_TRACE") || getenv("LRCN_DP_STAMPS")) { CK(cudaMalloc(&h->d_trace, 64 * 32 * 8)); CK(cudaMemset(h->d_trace, 0, 64 * 32 * 8)); }
-  CK(cudaMalloc(&h->g_last, G * 4)); CK(cudaMalloc(&h->g_ctok, G * 16 * 4)); CK(cudaMalloc(&h->g_stok, G * 4)); CK(cudaMalloc(&h->g_spar, G * 4));
+  CK(cudaMalloc(&h->g_last, G * 4)); CK(cudaMalloc(&h->g_ctok, G * 16 * 4)); CK(cudaMalloc(&h->g_stok, G * 4));
   CK(cudaMalloc(&h->g_hista, G * ML * 4)); CK(cudaMalloc(&h->g_histb, G * ML * 4)); CK(cudaMalloc(&h->g_done, G * 4));
   CK(cudaMalloc(&h->g_ndone, 4)); CK(cudaMalloc(&h->g_olen, G * 4)); CK(cudaMalloc(&h->g_rows, G * 4)); CK(cudaMalloc(&h->g_otok, G * ML * 8));
   CK(cudaMallocHost(&h->h_ndone, (size_t)lrcn_handle::NSNAP * (G + 1) * 4));
@@ -1170,7 +1170,7 @@ static void beam_lstm_step(lrcn_handle* h, int layer, int step, int R, float* g,
 // reference's hcat(input,hidden)*weight, lrcn.jl:529) so there is no accumulate pass over the gates.
 static bool beam_wide(const lrcn_handle* h, int R) { return h->bf16mode && R > 512; }
 
-// need_embed: gather the step's input embeddings here (first step, after a compaction, unfused mode); otherwise the previous
+// need_embed: gather the step's input embeddings here (first step, after a compaction); otherwise the previous
 // step's advance kernel has already written them
 static void enqueue_beam_step(lrcn_handle* h, int n_img, int K, int step, int nword, int maxlen, bool flip, float* out_lp, bool wide, const int* out_map,
                               bool need_embed) {
@@ -1209,24 +1209,21 @@ static void enqueue_beam_step(lrcn_handle* h, int n_img, int K, int step, int nw
   }
   gemm(h, true, true, R, V, H2, h2b, H2, Wp(h, 8), H2, logits, ldV, false, Wp(h, 9));
   beam_row_topk(s, logits, ldV, R, V, K, WS(h, o.gprob), h->g_ctok, WS(h, o.gcs), WS(h, o.gclp));             // lrcn.jl:652-661
-  static const bool unfused = getenv("LRCN_BEAM_UNFUSED") != nullptr;  // selection, advance and done-marking as three launches
-  if (unfused) beam_select(s, h->g_ctok, WS(h, o.gcs), WS(h, o.gclp), n_img, K, step == 1, h->g_stok, h->g_spar, WS(h, o.gss), WS(h, o.gslp));  // :667-668
   BeamAdvanceArgs a;
-  a.fused = unfused ? 0 : 1; a.cand_tok = h->g_ctok; a.cand_score = WS(h, o.gcs); a.cand_lp = WS(h, o.gclp);
+  a.cand_tok = h->g_ctok; a.cand_score = WS(h, o.gcs); a.cand_lp = WS(h, o.gclp);
   {
     float* ebuf = wide ? WS(h, o.gxh1) : e;
-    a.wemb = unfused ? nullptr : Wp(h, 7); a.e_out = ebuf; a.e_hi = SH(h, ebuf).hi; a.e_lo = SH(h, ebuf).lo; a.E = E; a.lde = wide ? E + H1 : E;
+    a.wemb = Wp(h, 7); a.e_out = ebuf; a.e_hi = SH(h, ebuf).hi; a.e_lo = SH(h, ebuf).lo; a.E = E; a.lde = wide ? E + H1 : E;
   }
   a.n_img = n_img; a.K = K; a.H1 = H1; a.H2 = H2; a.maxlen = maxlen; a.step = step; a.nword = nword;
   a.ld1 = ld1; a.ld2 = ld2;
-  a.sel_tok = h->g_stok; a.sel_parent = h->g_spar; a.sel_score = WS(h, o.gss); a.sel_lp = WS(h, o.gslp);
   a.h1_in = h1b; a.c1_in = c1b; a.h2_in = h2b; a.c2_in = c2b; a.h1_out = h1a; a.c1_out = c1a; a.h2_out = h2a; a.c2_out = c2a;
   a.hist_in = flip ? h->g_histb : h->g_hista; a.hist_out = flip ? h->g_hista : h->g_histb;
   a.lp_in = flip ? WS(h, o.glpb) : WS(h, o.glpa); a.lp_out = flip ? WS(h, o.glpa) : WS(h, o.glpb);
   a.h1_hi = SH(h, h1a).hi; a.h1_lo = SH(h, h1a).lo; a.h2_hi = SH(h, h2a).hi; a.h2_lo = SH(h, h2a).lo;
   a.prob = WS(h, o.gprob); a.last_tok = h->g_last; a.done = h->g_done; a.n_done = h->g_ndone;
   a.out_tokens = h->g_otok; a.out_len = h->g_olen; a.out_prob = WS(h, o.goprob); a.out_lp = out_lp; a.out_map = out_map;
-  beam_advance(s, a);  // reorder/gather parent states (+ their bf16 split for the next recurrent GEMMs)                 lrcn.jl:670-677
+  beam_advance(s, a);  // select (:667-668), reorder/gather parent states (+ their bf16 split for the next recurrent GEMMs)                 lrcn.jl:670-677
 }
 
 __global__ void beam_init_kernel(int R, int maxlen, float* prob, int* last, int* hist, float* lp, int* done, int* n_done, int n_img, int* out_map) {
@@ -1287,9 +1284,8 @@ static int s_beam_search(lrcn_handle* h, int split, const int64_t* image_ids, in
       bool flip = false;
       const bool wide = beam_wide(h, R);  // fixed for the chunk: the two paths keep the states in different buffers
       int n_act = ni;                     // images still in flight (compacted to the front)
-      static const bool no_compact = getenv("LRCN_BEAM_NO_COMPACT") != nullptr;
-      static const int den = getenv("LRCN_BEAM_COMPACT_DEN") ? atoi(getenv("LRCN_BEAM_COMPACT_DEN")) : 8;
-      static const int lag = getenv("LRCN_BEAM_LAG") ? atoi(getenv("LRCN_BEAM_LAG")) : 1;  // 1..NSNAP-1 (measured: 1 = 162k, 2 = 157k, 3 = 152k captions/s: later decisions cost more than the queued step gains)
+      constexpr int den = 8;  // compact when 1/den of the images in flight have ended
+      constexpr int lag = 1;  // decide from the snapshot `lag` steps back, 1..NSNAP-1 (measured: 1 = 162k, 2 = 157k, 3 = 152k captions/s: later decisions cost more than the queued step gains)
       // Asynchronous polling.  After EVERY step the done flags are copied into a ring of pinned snapshots (+ an event); the host
       // reads the snapshot of step s-1 right after it has enqueued step s, so the GPU always has a whole step queued while the
       // host waits, decides and enqueues -- the pipeline never drains (round 2a polled every 4 steps with a full
@@ -1304,7 +1300,6 @@ static int s_beam_search(lrcn_handle* h, int split, const int64_t* image_ids, in
       int snap_gen[lrcn_handle::NSNAP], snap_n[lrcn_handle::NSNAP], gen = 0, n_compactions = 0;
       for (int q = 0; q < lrcn_handle::NSNAP; q++) snap_gen[q] = -1;
       bool all_done = false;
-      static const bool beam_unfused = getenv("LRCN_BEAM_UNFUSED") != nullptr;
       bool need_embed = true;
       static const bool beam_debug = getenv("LRCN_BEAM_DEBUG") != nullptr;
       double wait_us = 0.0;
@@ -1313,7 +1308,7 @@ static int s_beam_search(lrcn_handle* h, int split, const int64_t* image_ids, in
       for (int step = 1; step <= nword + 1 && !all_done; step++) {
         steps_run = step;
         enqueue_beam_step(h, n_act, K, step, nword, maxlen, flip, logp_out ? WS(h, o.golp) : nullptr, wide, h->g_omap, need_embed);
-        need_embed = beam_unfused;
+        need_embed = false;
         flip = !flip;
         const int q = step % lrcn_handle::NSNAP;
         int* snap = h->h_ndone + (size_t)q * G1;
@@ -1333,7 +1328,7 @@ static int s_beam_search(lrcn_handle* h, int split, const int64_t* image_ids, in
         if (beam_debug) wait_us += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - tw0).count();
         const int* ps = h->h_ndone + (size_t)p * G1;
         if (ps[0] >= ni) { all_done = true; break; }      // (the step already enqueued runs on frozen images: a no-op)
-        if (snap_gen[p] != gen || no_compact || step >= nword + 1) continue;  // indices of an older numbering
+        if (snap_gen[p] != gen || step >= nword + 1) continue;  // indices of an older numbering
         int n_keep = 0;
         for (int i = 0; i < n_act; i++) n_keep += ps[1 + i] ? 0 : 1;
         if (n_keep == 0 || (n_act - n_keep) * den < n_act) continue;

@@ -42,7 +42,7 @@ struct Slot { int l = 0, B = 0, split = 0; int *tok_in = nullptr, *tok_tgt = nul
 struct Workspace {  // element offsets into the workspace arena
   size_t X, v, dv, Eall, dE, acts1, h1, c1, Z, dZ, acts2, h2, c2, logits, rowlp, dh2, dh1, dhrec1, dc1, dhrec2, dc2, colpart;
   // generation
-  size_t gX, gv, ge, gg1, gh1a, gc1a, gh1b, gc1b, gz, gg2, gh2a, gc2a, gh2b, gc2b, glogits, gprob, gcs, gclp, gss, gslp, glpa, glpb, goprob, golp, gxh1, gxh2;
+  size_t gX, gv, ge, gg1, gh1a, gc1a, gh1b, gc1b, gz, gg2, gh2a, gc2a, gh2b, gc2b, glogits, gprob, gcs, gclp, gss, glpa, glpb, goprob, golp, gxh1, gxh2;
 };
 struct lrcn_handle {
   lrcn_config cfg;
@@ -121,7 +121,7 @@ struct lrcn_handle {
   // DP
   ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
   // generation int buffers
-  int *g_last = nullptr, *g_ctok = nullptr, *g_stok = nullptr, *g_spar = nullptr, *g_hista = nullptr, *g_histb = nullptr, *g_done = nullptr,
+  int *g_last = nullptr, *g_ctok = nullptr, *g_stok = nullptr, *g_hista = nullptr, *g_histb = nullptr, *g_done = nullptr,
       *g_ndone = nullptr, *g_olen = nullptr, *g_rows = nullptr;
   long long* g_otok = nullptr;
   static constexpr int NSNAP = 4;   // ring of pinned snapshots of the done flags / survivor lists (asynchronous beam-search polling)

@@ -2,29 +2,29 @@
 logits row must fit 200 KiB of shared memory) and 1 <= K <= 11 (lrcn_beam_search).  Which kernel runs depends on V, K and
 the row count R; this file puts a case on both sides of every bound, against fp64 references (plain numpy or the oracle).
 
-Top-K selection for beam search, beam_topk_launch (csrc/kernels_simt.cu:1519-1558).  Rows are padded to ldV = roundup(V, 8),
-so they are always 16-byte aligned.
+Top-K selection for beam search, beam_row_topk (csrc/kernels_simt.cu).  Rows are padded to ldV = roundup(V, 8), so they are
+always 16-byte aligned.
 
   kernel                              taken when                                         covered here by
-  beam_row_topk4_kernel (warp/row),   R >= 2048, V % 4 == 0, V >= 128                    R = 2048 at V = 128, 4096, 11264, 51192;
+  beam_row_topk4_kernel (warp/row),   R >= TOPK4_MIN_ROWS = 2048, V % 4 == 0, V >= 128   R = 2048 at V = 128, 4096, 11264, 51192;
     KM = 1 / 3 / 5 / 11 for                                                              K = 1..6, 10, 11 (full and partly filled
     K = 1 / 2-3 / 4-5 / 6-11                                                             lists); the 1024-image decode's first steps
   beam_row_topk3_kernel (row in       R < 2048, V % 4 == 0, 4096 < V <= 11264            V = 11264 (static + dynamic shared memory just
     registers, grid = min(R, 444))                                                       under 48 KB); R = 2047 (persistent row loop);
                                                                                          decodes at V = 10000, 660 rows in flight
-  beam_row_topk2_kernel<256> (row in  everything else: V <= 4096, V % 4 != 0 (7731),     V = 127, 4096, 4100, 7731, 11268, 51192
+  beam_row_topk2_kernel (row in       everything else: V <= 4096, V % 4 != 0 (7731),     V = 127, 4096, 4100, 7731, 11268, 51192
     shared memory, grid = min(R,      V > 11264 up to the 200 KiB row (51192), and       (200 KiB dynamic shared memory); R = 2047 and
     1184))                            R >= 2048 with V % 4 != 0 or V < 128               2048 (persistent row loop, shared row reused)
   exact fallback in each kernel       more than 256 candidates >= tau                    all-equal rows, 300 copies of the maximum
 
-Softmax cross-entropy in training, softmax_ce_fused (kernels_simt.cu:595-610), nv4 = ceil(ldV / 2048):
+Softmax cross-entropy in training, softmax_ce_fused (kernels_simt.cu), nv4 = ceil(ldV / 2048):
   <2> nv4 <= 2 (V <= 4096), <4> nv4 <= 4 (V <= 8192), <6> nv4 <= 6 (V <= 12288), <8> nv4 <= 8 (V <= 16384); above that the
   bf16x3 mode runs softmax_ce_kernel plus a separate colsum for the output-bias gradient, as the fp32 mode always does.
   Covered: V = 4096 / 4097 / 8192 / 8193 / 12288 / 12289 / 16384 / 16385 / 51192 at R = 320 rows, so every fused variant runs
   its persistent row loop with the next-row prefetch (grid = min(R, 296), or min(R, 148) for <6> / <8>).
 
-Beam bookkeeping, beam_advance_kernel (kernels_simt.cu:1603): the per-image selection over K*K candidates keeps two 64-bit
-"used" masks; the second is reached from K = 9 (K*K > 64).  Covered by decodes at K = 10 and 11.
+Beam bookkeeping, beam_advance_kernel (kernels_simt.cu): the per-image selection over K*K candidates (beam_pick) keeps two
+64-bit "used" masks; the second is reached from K = 9 (K*K > 64).  Covered by decodes at K = 10 and 11.
 
 Generation at coco_2f dimensions (E = H = 1000, C = 500, V = 10636): per-step LSTM gen kernels up to 512 rows, the wide
 [x|h] operand path (ld2 = 2C + H2 = 2000) above.
